@@ -1,14 +1,16 @@
 #!/usr/bin/env python
 """Benchmark of the DrQ-v2 agent update (BASELINE.json metric: updates/sec at batch 256).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one DrQV2Agent.update (critic + actor + soft target update) on a fresh
 batch of the walker_walk shape (B=256, 9x84x84 uint8 stacks, A=6, F=50, H=1024, n-step 3).
 
 ours      : `value` = updates/s with the replay ring resident in HBM (sample + n-step
-            gather + update captured in one CUDA graph, timed with CUDA events; the K-step block is
-            repeated --blocks times, `value` is the median block, min / max are reported beside it);
+            gather + update captured in one CUDA graph, timed with CUDA events; the K timed steps are
+            split into --blocks blocks, `value` is the median block, min / max are reported beside it);
+            --dump-outputs DIR writes the parameters and metrics of the last timed step (seeded inputs:
+            the same arguments give the same inputs, so two builds can be compared output for output);
             `e2e` = the same update through the public API fed from HOST batches
             (pinned memory -> H2D inside the timed region, metrics read back D2H).
             Before anything is timed, one update at this configuration is checked against the oracle
@@ -18,7 +20,7 @@ ours      : `value` = updates/s with the replay ring resident in HBM (sample + n
             Sub-records `ensemble_8_per_gpu` (BASELINE configs[3]) and `dp_humanoid_b4096` (configs[4]) carry
             the two multi-GPU configurations with their own one-GPU points.
 reference : the reference's own update on the host cores (unmodified sources from baseline/_ref, else the
-            oracle port), bounded sample.
+            oracle port), --steps timed updates (default 40).
 Multi-GPU : one process per GPU (torchrun); the headline is independent agents (ensemble members) with no
             collective, value = sum over ranks / max-over-ranks time, scaling "weak".
 """
@@ -130,34 +132,39 @@ def ring_iter(key, A, episodes, B, dev, seed):
     return iter(make_replay_loader(key, episodes * 501, B, 0, False, 3, 0.99))
 
 
-def timed_blocks(step_fn, steps, blocks, world, dev):
-    """`blocks` back-to-back blocks of exactly `steps` updates, each bracketed by barrier + synchronize and timed
-    with CUDA events on the launching stream; per block the max over ranks.  Returns the ms of every block."""
-    out = []
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _ in range(blocks):
-        torch.cuda.synchronize()
-        if world > 1:
-            torch.distributed.barrier()
-        torch.cuda.synchronize()
-        e0.record()
+def block_sizes(steps, blocks):
+    """`steps` updates split into at most `blocks` back-to-back blocks of near-equal size (none empty)."""
+    n = max(1, min(blocks, steps))
+    return [steps // n + (i < steps % n) for i in range(n)]
+
+
+def timed_blocks(step_fn, sizes, world, dev):
+    """Blocks of exactly sizes[i] updates, enqueued back to back after one barrier + synchronize and timed with CUDA
+    events on the launching stream at every block boundary: nothing pauses between blocks, so only the first carries
+    the pipeline fill, however the steps are split.  Per block the max over ranks.  Returns the ms of every block."""
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(sizes) + 1)]
+    torch.cuda.synchronize()
+    if world > 1:
+        torch.distributed.barrier()
+    torch.cuda.synchronize()
+    ev[0].record()
+    for e, steps in zip(ev[1:], sizes):
         for _ in range(steps):
             step_fn()
-        e1.record()
-        torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1)
-        if world > 1:
-            t = torch.tensor([ms], device=dev)
-            torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-            ms = t.item()
-        out.append(ms)
+        e.record()
+    torch.cuda.synchronize()
+    out = [a.elapsed_time(b) for a, b in zip(ev, ev[1:])]
+    if world > 1:
+        t = torch.tensor(out, device=dev)
+        torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
+        out = t.tolist()
     return out
 
 
-def block_stats(ms_blocks, steps, units):
-    per = sorted(m / steps for m in ms_blocks)
+def block_stats(ms_blocks, sizes, units):
+    per = sorted(m / n for m, n in zip(ms_blocks, sizes))
     med = statistics.median(per)
-    return med, {"blocks": len(per), "steps_per_block": steps, "ms_per_step_median": med, "ms_per_step_min": per[0],
+    return med, {"blocks": len(per), "steps_per_block": sizes, "ms_per_step_median": med, "ms_per_step_min": per[0],
                  "ms_per_step_max": per[-1], "value_median": units * 1e3 / med, "value_best": units * 1e3 / per[0],
                  "value_worst": units * 1e3 / per[-1]}
 
@@ -563,9 +570,9 @@ def sub_ensemble(args, rank, world, dev, K=8):
     solo_ms = None
     if world > 1:                                    # one-GPU point: rank 0 runs while the others wait
         if rank == 0:
-            solo_ms = statistics.median(m / steps for m in timed_blocks(one, steps, 3, 1, dev))
+            solo_ms = statistics.median(m / steps for m in timed_blocks(one, [steps] * 3, 1, dev))
         torch.distributed.barrier()
-    med, stats = block_stats(timed_blocks(one, steps, 3, world, dev), steps, world * K)
+    med, stats = block_stats(timed_blocks(one, [steps] * 3, world, dev), [steps] * 3, world * K)
     if solo_ms is None:
         solo_ms = med
     del ens, its
@@ -593,7 +600,7 @@ def sub_dp(args, rank, world, dev):
             st[0] += 2
         for _ in range(3):
             solo()
-        one_gpu = statistics.median(m / steps for m in timed_blocks(solo, steps, 3, 1, dev))
+        one_gpu = statistics.median(m / steps for m in timed_blocks(solo, [steps] * 3, 1, dev))
         del agent, it
         torch.cuda.empty_cache()
     rec["one_gpu_b4096"] = None if one_gpu is None else {"ms_per_step": one_gpu, "value": 1e3 / one_gpu}
@@ -612,7 +619,7 @@ def sub_dp(args, rank, world, dev):
         st[0] += 2
     for _ in range(4):
         one()
-    med, stats = block_stats(timed_blocks(one, steps, 3, world, dev), steps, 1)
+    med, stats = block_stats(timed_blocks(one, [steps] * 3, world, dev), [steps] * 3, 1)
     a = agent._arena
     identical = D.replicas_identical([a.params, a.target, a.exp_avg, a.exp_avg_sq])
     # the same shard update without communication, and the collectives alone (eager, same tensors)
@@ -625,7 +632,7 @@ def sub_dp(args, rank, world, dev):
         st[0] += 2
     for _ in range(4):
         nocomm()
-    nc = statistics.median(m / steps for m in timed_blocks(nocomm, steps, 3, world, dev))
+    nc = statistics.median(m / steps for m in timed_blocks(nocomm, [steps] * 3, world, dev))
     ranges = {"critic": a._grads_full[a.seg["critic"][0]:a.seg["critic"][0] + a.seg["critic"][2]],
               "actor+metrics": a._grads_full[a.seg["actor"][0]:a.total + 8],
               "encoder": a._grads_full[a.seg["encoder"][0]:a.seg["encoder"][0] + a.seg["encoder"][2]]}
@@ -634,7 +641,7 @@ def sub_dp(args, rank, world, dev):
         t = t.clone()
         for _ in range(5):
             D.average_(t)
-        ms = statistics.median(timed_blocks(lambda: D.average_(t), 20, 3, world, dev)) / 20
+        ms = statistics.median(timed_blocks(lambda: D.average_(t), [20] * 3, world, dev)) / 20
         ar[name] = {"mbytes": t.numel() * 4 / 1e6, "us": ms * 1e3}
     rec.update({"value": 1e3 / med, "unit": "global-batch updates/s", "ms_per_step": med, "repeat": stats,
                 "shard_batch": Bs, "ms_per_step_same_shard_no_communication": nc, "ratio_vs_no_communication": med / nc,
@@ -678,6 +685,31 @@ def sub_act(args):
                 ragent.act(obs, 5000, False)
         rec["reference_on_gpu_batch_1_ms_per_call"] = (time.perf_counter() - t) / 100 * 1e3
     return rec
+
+
+# ----------------------------------------------------------------------------- outputs of the timed path
+DUMP_BYTES = 60 << 20     # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, agent, B):
+    """Writes what the last timed update computed, as a caller of DrQV2Agent.update receives it: every parameter of
+    the four networks (`<net>.<name>.npy`) and the 8 metrics (`metrics.npy`, in METRIC_KEYS order), float32.  Arrays
+    stay whole while everything fits DUMP_BYTES; past that the largest are cut to a fixed seeded sample of their
+    flattened elements (the same positions for the same size on every run), smallest arrays first."""
+    from drqv2_b200.drqv2 import METRIC_KEYS
+    m = agent.read_metrics(agent.workspace(B))
+    arrays = {"metrics": np.array([m[k] for k in METRIC_KEYS], dtype=np.float32)}
+    for net in ("encoder", "actor", "critic", "critic_target"):
+        for name, p in getattr(agent, net).named_parameters():
+            arrays[f"{net}.{name}"] = p.detach().float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    left, n = DUMP_BYTES // 4, len(arrays)
+    for name, a in sorted(arrays.items(), key=lambda kv: kv[1].size):
+        keep = left // n
+        if a.size > keep:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        left, n = left - a.size, n - 1
 
 
 # ----------------------------------------------------------------------------- main arm
@@ -761,8 +793,11 @@ def run_ours(args, rank, world):
     if rank == 0:                     # one nvidia-smi poller per job: NVML queries perturb the GPUs they touch, and in
         sampler.start()               # data-parallel mode a stall on any rank stalls every rank twice per update
     units = 1 if dp else world * K    # dp: global-batch updates/s; ensemble: sum over agents
-    ms_per_step, repeat = block_stats(timed_blocks(one_device_step, args.steps, args.blocks, world, dev), args.steps, units)
+    sizes = block_sizes(args.steps, args.blocks)
+    ms_per_step, repeat = block_stats(timed_blocks(one_device_step, sizes, world, dev), sizes, units)
     value = units * 1e3 / ms_per_step
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, agent, B)
 
     # ---- e2e: public API fed from host batches (pinned), metrics read back.  prefetch: the agent pulls the next
     # host batch one update ahead and overlaps its H2D copy with the running update (a DrQV2Agent option)
@@ -792,7 +827,7 @@ def run_ours(args, rank, world):
         step[0] += 2
     for _ in range(4):
         one_host_step()
-    e2e_ms, e2e_repeat = block_stats(timed_blocks(one_host_step, args.steps, args.blocks, world, dev), args.steps, units)
+    e2e_ms, e2e_repeat = block_stats(timed_blocks(one_host_step, sizes, world, dev), sizes, units)
     clocks = sampler.stop()
     e2e_value = units * 1e3 / e2e_ms
     h2d = K * (sum(t.numel() * t.element_size() for t in host_batches[0]) + 4 * 32)
@@ -844,12 +879,12 @@ def run_ours(args, rank, world):
                                       f"rows), CUDA-graphed, {'bf16 tensor-core mode (fp32 master weights, fp32 accumulation)' if args.mode == 'bf16' else 'fp32 parity mode'}" + (f"; global batch {args.batch} data-parallel over {world} GPUs (NCCL gradient all-reduce in the graph)" if dp else (f"; {world * K} independent agents (ensemble), {K} per GPU on their own streams, no collective" if world * K > 1 else "")),
                           "l2": "inputs larger than L2: each step gathers a fresh 32.5 MB batch from a "
                                 f"{args.episodes * 501 * 21168 / 1e6:.0f} MB ring and streams ~700 MB of activations",
-                          "timed_blocks": f"{args.blocks} blocks of {args.steps} steps; value / ms_per_step = the median block",
+                          "timed_blocks": f"{args.steps} steps in {len(sizes)} blocks; value / ms_per_step = the median block",
                           "mode": args.mode, "agents_per_gpu": K},
                "repeat": repeat,
                "e2e": {"value": e2e_value, "unit": "updates/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                        "repeat": e2e_repeat},
-               "gpu_launches": launches_per_update * args.steps * args.blocks * K, "launches_per_update": launches_per_update,
+               "gpu_launches": launches_per_update * args.steps * K, "launches_per_update": launches_per_update,
                "clocks": clocks, "roofline": roof, "cpu_baseline": cpu, "gpu_reference": gref}
         out.update(parity)
         out.update(extra)
@@ -935,7 +970,7 @@ def cpu_baseline(args, steps=5, warm=1):
 def run_reference(args, rank, world):
     if rank != 0:
         return None
-    steps = max(1, min(args.steps, 40))
+    steps = args.steps
     warm = max(1, min(args.warmup, 3))
     cpu = cpu_baseline(args, steps=steps, warm=warm)
     B, A, Fd, H = args.batch, args.action_dim, args.feature_dim, args.hidden_dim
@@ -952,9 +987,11 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed updates (default 1000; --impl reference: 40, its CPU update takes ~0.25 s)")
     ap.add_argument("--warmup", type=int, default=10)
-    ap.add_argument("--blocks", type=int, default=5, help="the K-step timed block is repeated this many times; value = median block")
+    ap.add_argument("--blocks", type=int, default=5,
+                    help="the --steps timed updates are split into this many blocks; value = median block")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256)
     ap.add_argument("--action-dim", type=int, default=6)
@@ -972,7 +1009,16 @@ def main():
     ap.add_argument("--no-kernels", action="store_true", help="skip the per-launch roofline timings")
     ap.add_argument("--no-subrecords", action="store_true", help="skip ensemble_8_per_gpu / dp_humanoid_b4096")
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip the reference-on-GPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the parameters and metrics the last timed update computed "
+                         "(rank 0, ensemble member 0) as DIR/<name>.npy, float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 40 if args.impl == "reference" else 1000
+    if args.steps < 1 or args.blocks < 1:
+        ap.error("--steps and --blocks must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":

@@ -567,44 +567,67 @@ def test_replay_snapshot_files_and_resume(dev, tmp_path):
     assert torch.equal(ring2.reward[:n], ring1.reward[:n]) and torch.equal(ring2.discount[:n], ring1.discount[:n])
 
 
-def test_reference_snapshot_interop(dev):
-    """SURVEY §8f-3: a reference agent's state (what train.py:192-204 pickles) moves into this agent and back."""
-    import bench
+def _reference_standin(A, Fd, H, lr, p, m=None, v=None, step=0):
+    """What a reference DrQV2Agent carries from one update to the next (drqv2.py:137-153): the four networks
+    (reference-shaped modules, the names / shapes of drqv2.py:55-59,74-81,100-111) holding parameters `p`, and
+    the three torch.optim.Adam optimisers holding moments `m`, `v` after `step` steps (none when m is None)."""
+    from types import SimpleNamespace
+
+    from drqv2_b200 import Actor, Critic, Encoder
+    ref = SimpleNamespace(encoder=Encoder((9, 84, 84)), actor=Actor(O.REPR_DIM, (A,), Fd, H),
+                          critic=Critic(O.REPR_DIM, (A,), Fd, H), critic_target=Critic(O.REPR_DIM, (A,), Fd, H))
+    for net in ("encoder", "actor", "critic", "critic_target"):
+        getattr(ref, net).load_state_dict(p[net])
+    for net in ("encoder", "actor", "critic"):
+        opt = torch.optim.Adam(getattr(ref, net).parameters(), lr=lr)
+        if m is not None:
+            for k, q in getattr(ref, net).named_parameters():
+                opt.state[q] = dict(step=torch.tensor(float(step)), exp_avg=m[net][k].clone(),
+                                    exp_avg_sq=v[net][k].clone())
+        setattr(ref, f"{net}_opt", opt)
+    return ref
+
+
+def test_reference_snapshot_interop(dev, golden_dir):
+    """SURVEY §8f-3: a reference agent's state (what train.py:192-204 pickles) moves into this agent and back.
+    The reference agent is the unmodified reference after the two updates recorded in update_golden.json
+    (case walker_small, B=8, H=1024, its own grid_sample aug): the oracle replays those updates, the rebuilt
+    parameters are checked against the reference's recorded ones, and act() from the taken-over state is
+    compared with the action the reference itself returned."""
     from drqv2_b200 import DrQV2Agent
-    ref = bench._load_reference()
-    if ref is None:
-        pytest.skip("baseline/_ref (unmodified reference sources) not present")
-    A, Fd, H = 6, 50, 64
-    torch.manual_seed(3)
-    ragent = ref.DrQV2Agent((9, 84, 84), (A,), "cuda", 1e-4, Fd, H, 0.01, 2000, 2, SCHED, 0.3, False)
-    b = O.synthetic_batch(4, A, seed=2)
-    batch = tuple(b[k].cuda() for k in ("obs", "action", "reward", "discount", "next_obs"))
-    for i in range(2):                                         # two reference updates: Adam state, step = 2
-        ragent.update(iter([batch]), 2 * i)
-    mine = DrQV2Agent((9, 84, 84), (A,), "cuda", 1e-4, Fd, H, 0.01, 2000, 2, SCHED, 0.3, False, seed=1, mode="fp32")
+    g = json.loads((golden_dir / "update_golden.json").read_text())[0]
+    c, rec = g["case"], g["variants"]["ref"]
+    A, Fd, H, lr = c["A"], c["F"], c["H"], c["lr"]
+    oracle = O.OracleAgent(O.synthetic_params(9, A, Fd, H, seed=c["pseed"]), lr, 0.01, SCHED, 0.3, aug="grid")
+    for s in range(c["steps"]):
+        b = O.synthetic_batch(c["B"], A, seed=c["bseed"] + s)
+        oracle.update(b["obs"], b["action"], b["reward"], b["discount"], b["next_obs"], 2 * s, b["shift_obs"],
+                      b["shift_next"], b["eps_critic"], b["eps_actor"])
+    for net, ps in rec["steps"][-1]["params"].items():      # the tolerances of tests/test_oracle_golden.py
+        for k, summ in ps.items():
+            t = oracle.p[net][k].double().flatten()
+            assert np.max(np.abs(t[summ["probe_idx"]].numpy() - summ["probe"])) <= 2.5 * lr * c["steps"], (net, k)
+            assert abs(float(t.norm()) - summ["l2"]) <= 1e-4 * summ["l2"] + 1e-6, (net, k)
+    ragent = _reference_standin(A, Fd, H, lr, oracle.p, oracle.m, oracle.v, c["steps"])
+    mine = DrQV2Agent((9, 84, 84), (A,), "cuda", lr, Fd, H, 0.01, 2000, 2, SCHED, 0.3, False, seed=1, mode="fp32")
     mine.load_reference_agent(ragent)
-    assert mine._opt_step == 2
+    assert mine._opt_step == c["steps"]
     for net in ("encoder", "actor", "critic", "critic_target"):
         for (n1, p1), p2 in zip(getattr(mine, net).named_parameters(), getattr(ragent, net).parameters()):
-            assert torch.equal(p1, p2), (net, n1)
+            assert torch.equal(p1.cpu(), p2), (net, n1)
     for net in ("encoder", "actor", "critic"):
         opt = getattr(ragent, f"{net}_opt")
         sd = getattr(mine, f"{net}_opt").state_dict()
         ref_m = torch.cat([opt.state[p]["exp_avg"].reshape(-1) for p in getattr(ragent, net).parameters()])
-        assert torch.equal(sd["exp_avg"][:ref_m.numel()], ref_m)
-    # same deterministic action from both
-    obs = b["obs"][0].numpy()
-    tf32 = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False            # the reference's convs default to TF32 on GPU (SURVEY §8a R4)
-    try:
-        with torch.no_grad():
-            want = ragent.act(obs, 5000, True)
-    finally:
-        torch.backends.cudnn.allow_tf32 = tf32
-    got = mine.act(obs, 5000, True)
-    assert np.abs(got - want).max() < 2e-5
+        assert torch.equal(sd["exp_avg"][:ref_m.numel()].cpu(), ref_m)
+    # the deterministic action the reference returned from this state (act_eval: the oracle's own state is within
+    # 2e-5 of it, tests/test_oracle_golden.py), and the oracle's action from the very state taken over
+    obs1 = O.synthetic_batch(1, A, seed=99)["obs"][0].numpy()
+    got = mine.act(obs1, 5000, True)
+    assert np.abs(got - oracle.act(obs1, 5000, True)[0].numpy()).max() < 2e-5
+    assert np.abs(got - np.array(rec["act_eval"])).max() < 4e-5
     # and back: a fresh reference agent continues from the exported state
-    r2 = ref.DrQV2Agent((9, 84, 84), (A,), "cuda", 1e-4, Fd, H, 0.01, 2000, 2, SCHED, 0.3, False)
+    r2 = _reference_standin(A, Fd, H, lr, O.synthetic_params(9, A, Fd, H, seed=1))
     st = mine.export_reference_state()
     for net in ("encoder", "actor", "critic", "critic_target"):
         getattr(r2, net).load_state_dict(st[net])
@@ -612,9 +635,17 @@ def test_reference_snapshot_interop(dev):
         getattr(r2, f"{net}_opt").load_state_dict(st[f"{net}_opt"])
         o1, o2 = getattr(ragent, f"{net}_opt"), getattr(r2, f"{net}_opt")
         for p1, p2 in zip(getattr(ragent, net).parameters(), getattr(r2, net).parameters()):
+            assert torch.equal(p1, p2)
             assert torch.equal(o1.state[p1]["exp_avg_sq"], o2.state[p2]["exp_avg_sq"])
-            assert float(o2.state[p2]["step"]) == 2.0
-    r2.update(iter([batch]), 4)                                # and the reference trains on from it
+            assert float(o2.state[p2]["step"]) == c["steps"]
+    # and the reference's optimisers train on from it: one more Adam step with the same gradients keeps the two equal
+    for net in ("encoder", "actor", "critic"):
+        for (k, p1), p2 in zip(getattr(ragent, net).named_parameters(), getattr(r2, net).parameters()):
+            p1.grad, p2.grad = oracle.grads[net][k].clone(), oracle.grads[net][k].clone()
+        getattr(ragent, f"{net}_opt").step()
+        getattr(r2, f"{net}_opt").step()
+        for p1, p2 in zip(getattr(ragent, net).parameters(), getattr(r2, net).parameters()):
+            assert torch.equal(p1, p2), net
 
 
 def test_agent_pickle_roundtrip(dev):
