@@ -123,7 +123,7 @@ OPT_PLAIN, OPT_LINEAR, OPT_TRUNK, OPT_CONV, OPT_CONV1 = 0, 1, 2, 3, 4
 
 class WgReduceJob(C.Structure):
     _fields_ = [("partial", C.c_void_p), ("dw", C.c_void_p), ("db", C.c_void_p), ("n_images", C.c_int32),
-                ("hout", C.c_int32), ("cin", C.c_int32), ("ctas", C.c_int32)]
+                ("hout", C.c_int32), ("cin", C.c_int32), ("reserved", C.c_int32)]
 
 
 class ColsumJob(C.Structure):
@@ -213,13 +213,13 @@ class Bf16State:
                 PackJob(PACK_LINEAR, A, H, 0, pa("policy.4.weight"), None, self.p4.ptr(), None)]
 
     # ---- optimiser step + operand refresh in one launch (drq_adam_pack_step)
-    def _segments(self, mod, offs, base, ema, packed, only=None):
+    def _segments(self, mod, offs, base, ema, packed):
         """One segment per tensor of `mod` in arena order; tensors without a bf16 copy merge into PLAIN runs.
-        packed: pname -> (kind, rows, cols, out, out2); only: predicate on the parameter name (a part of the module)."""
+        packed: pname -> (kind, rows, cols, out, out2)."""
         segs = []
         skip = None
         for pname, prm in mod.named_parameters():
-            if pname == skip or (only is not None and not only(pname)):
+            if pname == skip:
                 continue
             off, n = offs[pname] - base, prm.numel()
             if pname in packed:
@@ -255,13 +255,6 @@ class Bf16State:
         segs_c = self._segments(ag.critic, a.offsets["critic"], 0, 0, self._critic_like_packed(self.CRITIC, 0))
         self.plan_encoder = (OptSeg * len(segs_e))(*segs_e)
         self.plan_critic_only = (OptSeg * len(segs_c))(*segs_c)
-        # the critic's step in two launches: the trunk (all the actor pass' first GEMM reads) and the Q heads
-        is_trunk = lambda n: n.startswith("trunk.")
-        pk_c = self._critic_like_packed(self.CRITIC, 0)
-        self.plan_critic_parts = []
-        for pred in (is_trunk, lambda n: not is_trunk(n)):
-            sg = self._segments(ag.critic, a.offsets["critic"], 0, 0, pk_c, only=pred)
-            self.plan_critic_parts.append((OptSeg * len(sg))(*sg))
         segs = segs_e + segs_c
         self.plan_critic = (OptSeg * len(segs))(*segs)
         act = {"trunk.0.weight": (OPT_TRUNK, Fd, REPR_DIM, self.trunk_ptr(self.ACTOR), None),
@@ -271,11 +264,6 @@ class Bf16State:
         segs_a = self._segments(ag.actor, a.offsets["actor"], 0, 0, act)
         segs_t = self._segments(ag.critic, a.offsets["critic"], a.seg["critic"][0], 1, self._critic_like_packed(self.TARGET, 2))
         self.plan_actor_only = (OptSeg * len(segs_a))(*segs_a)
-        # the actor's step in two launches: the policy MLP (its gradients are complete first) and the trunk
-        self.plan_actor_parts = []
-        for pred in (lambda n: not is_trunk(n), is_trunk):
-            sg = self._segments(ag.actor, a.offsets["actor"], 0, 0, act, only=pred)
-            self.plan_actor_parts.append((OptSeg * len(sg))(*sg))
         self.plan_target = (OptSeg * len(segs_t))(*segs_t)
         segs = segs_a + segs_t
         self.plan_actor = (OptSeg * len(segs))(*segs)
@@ -300,14 +288,6 @@ class Bf16State:
     def step_critic(self):
         """critic_opt.step() (drqv2.py:201) and the critic's bf16 operand copies."""
         self._step(self.plan_critic_only, "critic")
-
-    def step_critic_part(self, i):
-        """critic_opt.step() on the trunk (i = 0) or on the Q heads (i = 1)"""
-        self._step(self.plan_critic_parts[i], "critic")
-
-    def step_actor_part(self, i):
-        """actor_opt.step() on the policy MLP (i = 0) or on the trunk (i = 1)"""
-        self._step(self.plan_actor_parts[i], "actor")
 
     def step_encoder(self):
         """encoder_opt.step() (drqv2.py:202) and the encoder's bf16 operand copies."""
@@ -449,13 +429,6 @@ def actor_mlp_fwd(agent, hA, p1, p2, mu_pre, M, samples=(), clip=0.0):
          bias=pa("policy.0.bias"))
     gemm(p1.ptr(), p1.units, w2.ptr(), w2.units, GEMM_KK, p2.ptr(), p2.units, M, H, H, TEPI_RELU_BF16,
          bias=pa("policy.2.bias"))
-    if not agent.fused_policy_head:     # DRQV2_B200_POLICY_HEAD=0: the tensor-core tile + one sampling launch per row range
-        w4 = st.p4
-        gemm(p2.ptr(), p2.units, w4.ptr(), w4.units, GEMM_KK, mu_pre, A, M, A, H, TEPI_F32, bias=pa("policy.4.bias"))
-        for j in samples:
-            call("drq_actor_sample", mu_pre + F32 * j.row0 * A, j.eps, agent._sc("stddev"), float(clip), j.action_out, j.ld_a,
-                 j.mu_out, j.metrics, j.a_bf16, j.units_a, j.feat_off, j.rows, A, _stream())
-        return
     jobs = (PolicySample * max(1, len(samples)))(*samples)
     call("drq_policy_head_fwd_bf16", p2.ptr(), p2.units, pa("policy.4.weight"), pa("policy.4.bias"), mu_pre, M, H, A,
          jobs, len(samples), agent._sc("stddev"), float(clip), agent._policy_ticket.data_ptr(), _stream())
@@ -593,25 +566,13 @@ def critic_pass(agent, ws, bw, encoder_grad=True):
             call("drq_conv3x3_dgrad_bf16", d[layer], st.conv_wd[layer - 1].data_ptr(), acts[layer - 1], 2 * B,
                  d[layer - 1], B, hout, s2)
         src = getattr(ws, "ring_src", None)
-        # conv1's weight gradient leaves no room for any other block on its SMs: its own (smaller) SM limit when it runs
-        # beside the actor pass, and the number of partials that makes handed to the reduction
-        lim1 = agent.conv1_wgrad_sms if agent._encoder_side_stream() is not None else 0
-        g1 = 0
-        if lim1:
-            prev = _lib.lib().drq_device_sm_count()
-            call("drq_set_sm_limit", lim1)
-            g1 = min(14 * B, lim1)
-        try:
-            if src is not None:
-                call("drq_conv1_wgrad_bf16_ring", C.byref(src), B, ws.shift.data_ptr(), d[0], bw.wg_ws[0].data_ptr(), None, None,
-                     B, agent.aug.pad, s2)
-            else:
-                call("drq_conv1_wgrad_bf16", ws.obs.data_ptr(), ws.shift.data_ptr(), d[0], bw.wg_ws[0].data_ptr(), None, None,
-                     B, agent.obs_shape[0], agent.aug.pad, s2)
-        finally:
-            if lim1:
-                call("drq_set_sm_limit", prev)
-        jobs.append(WgReduceJob(bw.wg_ws[0].data_ptr(), ge("convnet.0.weight"), ge("convnet.0.bias"), B, 0, agent.obs_shape[0], g1))
+        if src is not None:
+            call("drq_conv1_wgrad_bf16_ring", C.byref(src), B, ws.shift.data_ptr(), d[0], bw.wg_ws[0].data_ptr(), None, None,
+                 B, agent.aug.pad, s2)
+        else:
+            call("drq_conv1_wgrad_bf16", ws.obs.data_ptr(), ws.shift.data_ptr(), d[0], bw.wg_ws[0].data_ptr(), None, None,
+                 B, agent.obs_shape[0], agent.aug.pad, s2)
+        jobs.append(WgReduceJob(bw.wg_ws[0].data_ptr(), ge("convnet.0.weight"), ge("convnet.0.bias"), B, 0, agent.obs_shape[0], 0))
         arr = (WgReduceJob * len(jobs))(*jobs)
         call("drq_conv_wgrad_reduce_multi", arr, len(jobs), s2)   # all four layers' partials -> dW, db in one launch
 
@@ -646,16 +607,7 @@ def critic_pass(agent, ws, bw, encoder_grad=True):
     if early:
         beside.join()
     agent._sync_grads("critic")                     # data-parallel: beside the encoder backward (no-op otherwise)
-    if agent.split_critic_step and not agent.data_parallel:
-        # the trunk first - the actor pass' trunk GEMM and LayerNorm then run beside the Q heads' step
-        st.step_critic_part(0)
-        aux = agent._aux_stream()
-        aux.wait_stream(main)
-        with torch.cuda.stream(aux):
-            st.step_critic_part(1)
-        agent._critic_rest = aux
-    else:
-        st.step_critic()
+    st.step_critic()
 
 
 def actor_pass(agent, ws, bw, soft_update=True, standalone=False):
@@ -695,16 +647,10 @@ def _actor_pass(agent, ws, bw, soft_update=True, standalone=False):
         actor_mlp_fwd(agent, bw.hA, bw.p1, bw.p2, bw.mu_pre.data_ptr(), B, clip=agent.stddev_clip, samples=[
             PolicySample(0, B, ws.eps_a.data_ptr(), ws.xA.data_ptr() + F32 * Fd, Fd + A, ws.mu.data_ptr(),
                          ws.metrics.data_ptr() + F32 * 6, xA.ptr(), xA.units, Fd, 0)])
-    rest = agent._critic_rest                       # stream of the Q heads' half of critic_opt.step(), if it was split
-    agent._critic_rest = None
     if beside.side is not None and soft_update:
         # the soft target update depends on the stepped critic only (drqv2.py:259-260 runs it after update_actor, on the
         # same critic parameters) and nothing in this pass reads the target: beside the whole pass
-        ema = agent._ema_stream() or beside.side    # nothing waits for it before the end of the update: lowest priority
-        ema.wait_stream(torch.cuda.current_stream())
-        if rest is not None:
-            ema.wait_stream(rest)
-        with torch.cuda.stream(ema):
+        with beside:
             st.step_target()
     # (the sample a = clamp(mu + clip(eps * std)) of drqv2.py:210-211 was drawn with the actor's forward - the policy head's
     # launch in the critic pass, or just above in the stage API)
@@ -715,8 +661,6 @@ def _actor_pass(agent, ws, bw, soft_update=True, standalone=False):
          splitk=S, strides=_strides(split=B * FP))
     ln_tanh_multi([LnJob(part, FP, B * FP, S, pc("trunk.0.bias"), pc("trunk.1.weight"), pc("trunk.1.bias"),
                          ws.xA.data_ptr(), Fd + A, None, None, xA.ptr(), xA.units, 0)], B, Fd)
-    if rest is not None:
-        torch.cuda.current_stream().wait_stream(rest)       # the Q heads are stepped
     twin_q_fwd(agent, bw, xA, 1, B)
     q = bw.q4.data_ptr()
     c1, c2, dc1, dc2 = bw.c1, bw.c2, bw.dc1, bw.dc2
@@ -743,40 +687,23 @@ def _actor_pass(agent, ws, bw, soft_update=True, standalone=False):
     with beside:
         gemm(dp2.ptr(), U, p1.ptr(), U, GEMM_MNMN, ga("policy.2.weight"), H, H, H, B, TEPI_F32, bn=128)
     gemm(dp2.ptr(), U, a2.ptr(), a2.units, GEMM_KMN, dp1.ptr(), U, B, H, H, TEPI_MASK_BF16, mask=p1.ptr(), units_mask=U)
-    split = agent.split_actor_step and beside.side is not None and not agent.data_parallel and soft_update
-    mlp_bias_jobs = [ColsumJob(ws.dmu_pre.data_ptr(), A, ga("policy.4.bias"), B, A, 0, 0),
-                     ColsumJob(dp2.ptr(), U, ga("policy.2.bias"), B, H, 1, 0), ColsumJob(dp1.ptr(), U, ga("policy.0.bias"), B, H, 1, 0)]
-    trunk_bias_jobs = [ColsumJob(ws.dz.data_ptr(), Fd, ga("trunk.0.bias"), B, Fd, 0, 0),
-                       ColsumJob(ws.dz.data_ptr() + F32 * B * Fd, Fd, ga("trunk.1.weight"), B, Fd, 0, 0, ws.xhatA.data_ptr()),
-                       ColsumJob(ws.dz.data_ptr() + F32 * B * Fd, Fd, ga("trunk.1.bias"), B, Fd, 0, 0)]
     with beside:
         gemm(dp1.ptr(), U, hA.ptr(), hA.units, GEMM_MNMN, ga("policy.0.weight"), Fd, H, Fd, B, TEPI_F32)
     gemm(dp1.ptr(), U, a0.ptr(), a0.units, GEMM_KMN, ws.dhA.data_ptr(), Fd, B, Fd, H, TEPI_F32)
-    aux = None
-    if split:
-        # the policy MLP's gradients are complete and the last reader of its bf16 weights (the GEMM above) is enqueued:
-        # its half of actor_opt.step() runs beside the trunk's backward
-        aux = agent._aux_stream()
-        aux.wait_stream(torch.cuda.current_stream())
-        aux.wait_stream(beside.side)
-        with torch.cuda.stream(aux):
-            colsum_multi(mlp_bias_jobs)
-            st.step_actor_part(0)
     call("drq_ln_tanh_bwd", ws.dhA.data_ptr(), Fd, ws.hA.data_ptr(), Fd, ws.xhatA.data_ptr(), ws.rstdA.data_ptr(),
          pa("trunk.1.weight"), ws.dz.data_ptr(), None, None, bw.dz.ptr(), bw.dz.units,
          B, Fd, 1, 0, s)
     with beside:
         gemm(bw.dz.ptr(), bw.dz.units, feat.ptr(), feat.units, GEMM_MNMN, ga("trunk.0.weight"), REPR_DIM, Fd, REPR_DIM, B,
              TEPI_TRUNK_WGRAD, bn=128)
-    colsum_multi(trunk_bias_jobs if split else mlp_bias_jobs + trunk_bias_jobs)
+    colsum_multi([ColsumJob(ws.dmu_pre.data_ptr(), A, ga("policy.4.bias"), B, A, 0, 0),
+                  ColsumJob(dp2.ptr(), U, ga("policy.2.bias"), B, H, 1, 0), ColsumJob(dp1.ptr(), U, ga("policy.0.bias"), B, H, 1, 0),
+                  ColsumJob(ws.dz.data_ptr(), Fd, ga("trunk.0.bias"), B, Fd, 0, 0),
+                  ColsumJob(ws.dz.data_ptr() + F32 * B * Fd, Fd, ga("trunk.1.weight"), B, Fd, 0, 0, ws.xhatA.data_ptr()),
+                  ColsumJob(ws.dz.data_ptr() + F32 * B * Fd, Fd, ga("trunk.1.bias"), B, Fd, 0, 0)])
     beside.join()                                   # the actor's weight gradients are complete
-    if beside.side is not None and soft_update and agent._ema_stream() is not None:
-        torch.cuda.current_stream().wait_stream(agent._ema_stream())
     agent._sync_grads("actor", metrics=True)
-    if split:
-        st.step_actor_part(1)
-        torch.cuda.current_stream().wait_stream(aux)
-    elif beside.side is not None or not soft_update:
+    if beside.side is not None or not soft_update:
         st.step_actor()                             # the target's soft update already ran beside this pass (or is not wanted)
     else:
         st.step_actor_target()

@@ -47,16 +47,13 @@ SIGNATURES = {
     "drq_conv1_fwd_bf16": [P, P, P, P, I, I, I, P],
     "drq_conv1_wgrad_bf16": [P, P, P, P, P, P, I, I, I, P],
     "drq_gemm_bf16": [P, I, P, I, I, P, L, I, P, P, I, I, I, I, I, I, I, I, P, I, I, P],
-    "drq_set_pdl": [I],
     "drq_set_sm_limit": [I],
     "drq_set_gemm_small": [I],
     "drq_set_conv4x1": [I],
     "drq_set_conv1_planes": [I],
     "drq_debug_gemm_stamps": [P],
-    "drq_debug_opt_min_blocks": [I],
     "drq_debug_conv_stamps": [P],
     "drq_debug_trap_note": [P],
-    "drq_debug_force_timeout": [P],
     "drq_debug_conv4x1_stamps": [P],
     "drq_debug_conv1_stamps": [P],
     "drq_pack_multi": [P, I, P],
@@ -70,7 +67,7 @@ SIGNATURES = {
     "drq_ln_tanh_fwd": [P, I, L, P, P, P, P, L, P, P, P, L, I, I, F, P],
     "drq_ln_tanh_fwd_multi": [P, I, I, I, F, P],
     "drq_ln_tanh_bwd": [P, L, P, L, P, P, P, P, P, P, P, L, I, I, I, L, P],
-    "drq_actor_sample": [P, P, P, F, P, L, P, P, P, L, I, I, I, P],
+    "drq_actor_sample": [P, P, P, F, P, L, P, P, I, I, P],
     "drq_policy_head_fwd_bf16": [P, L, P, P, P, I, I, I, P, I, P, F, P, P],
     "drq_actor_sample_bwd": [P, L, P, P, P, L, I, I, I, L, P],
     "drq_q_head_fwd_bf16": [P, L, L, P, P, P, I, I, I, L, I, L, P],
@@ -78,7 +75,6 @@ SIGNATURES = {
     "drq_critic_loss": [P, P, P, P, P, P, P, P, P, P, I, P],
     "drq_actor_loss": [P, P, P, P, P, I, P],
     "drq_copy2d_f32": [P, L, P, L, I, I, P],
-    "drq_set_l2_persist": [P, L],
     "drq_adam_step": [P, P, P, P, L, P, P],
     "drq_soft_update": [P, P, L, F, F, P],
     "drq_adam_ema_step": [P, P, P, P, L, P, P, P, L, F, F, P],
@@ -126,12 +122,8 @@ def lib():
         for name, (res, args) in SPECIAL.items():
             fn = getattr(h, name)
             fn.argtypes, fn.restype = args, res
-        if h.drq_abi_version() != 1:
+        if h.drq_abi_version() != 2:
             raise ImportError("libdrqv2_b200.so ABI version mismatch")
-        # programmatic dependent launch between the library's kernels (opt-in with DRQV2_B200_PDL=1: measured neutral without early trigger, -25 % with it)
-        h.drq_set_pdl(int(os.environ.get("DRQV2_B200_PDL", "0")))
-        if os.environ.get("DRQV2_B200_OPT_MINB"):       # tuning: register target of the fused optimiser kernel
-            h.drq_debug_opt_min_blocks(int(os.environ["DRQV2_B200_OPT_MINB"]))
         if os.environ.get("DRQV2_B200_CONV4X1"):        # A/B: 0 = one-pixel-per-row conv kernels, 1 = default, 2 = four-pixel-column kernels always
             h.drq_set_conv4x1(int(os.environ["DRQV2_B200_CONV4X1"]))
         if os.environ.get("DRQV2_B200_CONV1_PLANES"):   # A/B: 0 = im2col conv1 forward, 1 = parity-plane forward (default)

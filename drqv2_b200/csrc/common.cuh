@@ -23,38 +23,10 @@ inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s
 // the callers that include <cuda.h> (conv4x1_tc.cu, conv1_tc.cu)
 void* tensor_map_encoder();
 
-// Programmatic dependent launch (drq_set_pdl): every kernel waits for its predecessors (griddepcontrol.wait =
-// all prior grids complete and flushed) before it touches global memory, so its launch latency, barrier / TMEM
-// set-up and first instruction fetches may overlap the tail of the running kernel.  The long tensor-core
-// kernels release their dependents (pdl_release) once their producer warp has issued its last load - the
-// remaining tail is MMA drain and epilogue; everything else releases implicitly at exit.  Releasing at kernel
-// entry (pdl_trigger, -DDRQ_PDL_ENTRY_TRIGGER) parks the next kernel's CTAs on the SMs for the whole run of a
-// multi-wave kernel and was measured 25 % slower.  Without the launch attribute the instructions are no-ops.
-extern int g_pdl;        // 0 off, 1 every launch, 2 only the launches that ask for it (g_pdl_once)
-extern int g_pdl_once;   // set by a launcher right before launch_k: this launch may start before its predecessor has drained
 // SMs the persistent kernels size their grids for (drq_set_sm_limit): all of them, or fewer when a concurrent
 // collective's CTAs need SMs of their own (a persistent kernel never yields an SM once its CTAs are resident).
 extern int g_sm_limit;
 inline int sm_budget() { return g_sm_limit; }
-__device__ __forceinline__ void pdl_trigger() {
-#ifdef DRQ_PDL_ENTRY_TRIGGER
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void pdl_release() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-template <typename... P, typename... A>
-inline void launch_k(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, A&&... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = (g_pdl == 1 || (g_pdl == 2 && g_pdl_once)) ? 1 : 0;
-    g_pdl_once = 0;
-    cudaLaunchKernelEx(&cfg, kernel, static_cast<P>(args)...);
-}
 
 constexpr int kImg = DRQ_IMG;
 constexpr int kPW = DRQ_PW;

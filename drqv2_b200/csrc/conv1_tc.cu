@@ -213,7 +213,6 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
     constexpr int TILES_PER_IMG = (kPW * kPW + kC1Tile - 1) / kC1Tile;   // 14
     const int total_tiles = a.n_images * TILES_PER_IMG;
 
-    pdl_trigger();
     if (threadIdx.x == 0) {
         for (int i = 0; i < kC1Stages; ++i) { mbar_init(full + i, kC1Builders / 2); mbar_init(empty + i, 1); mbar_init(dfull + i, 1); }
         for (int i = 0; i < kC1Acc; ++i) { mbar_init(tfull + i, 1); mbar_init(tempty + i, 4); }
@@ -225,7 +224,6 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
         tmem_alloc(tmem_slot, 128);
         tmem_relinquish();
     }
-    pdl_wait();                 // CTA-local set-up above overlaps the previous kernel's tail
     if (!WGRAD) {
         const uint4* src = reinterpret_cast<const uint4*>(a.w);
         uint4* dst = reinterpret_cast<uint4*>(w_s);
@@ -408,7 +406,6 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
                 }
             }
         }
-        pdl_release();                          // last rows are on their way: the next kernel may set itself up
     } else {
         // ------------------------------------------------ epilogue warps 17..20 -> lane quarters 1,2,3,0
         const int q = warp & 3;
@@ -465,8 +462,6 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
 
 __global__ void __launch_bounds__(256)
 pack_conv1_w_kernel(const float* __restrict__ w, const float* __restrict__ bias, __nv_bfloat16* __restrict__ out, int cin) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float part[32][9];
     pack_conv1_w_block(w, bias, out, cin, threadIdx.x, part);
 }
@@ -475,8 +470,6 @@ pack_conv1_w_kernel(const float* __restrict__ w, const float* __restrict__ bias,
 // partials [32][96].  Block = 32 outputs x 8 slices of the G partials, combined in fixed order.
 __global__ void __launch_bounds__(256)
 conv1_wgrad_reduce_kernel(const float* __restrict__ partial, int G, int cin, float* __restrict__ dw, float* __restrict__ db) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float red[8][33], redb[8][33];
     conv1_reduce_block(partial, G, cin, dw, db, blockIdx.x, red, redb);
 }
@@ -568,7 +561,6 @@ __global__ void __launch_bounds__(kP1Threads, 1) conv1_planes_kernel(const __gri
     const int cin = CIN ? CIN : a.cin;
     const int total_tiles = a.n_images * kP1TilesPerImg;
 
-    pdl_trigger();
     if (threadIdx.x == 0) {
         for (int i = 0; i < kP1Stages; ++i) { mbar_init(full + i, kP1Group); mbar_init(empty + i, 1); }
         for (int i = 0; i < kP1Acc; ++i) { mbar_init(tfull + i, 1); mbar_init(tempty + i, 4); }
@@ -581,7 +573,6 @@ __global__ void __launch_bounds__(kP1Threads, 1) conv1_planes_kernel(const __gri
     }
     // plane stages start as zeros: the never written fourth row of the odd-row planes must read as finite values
     for (int i = threadIdx.x; i < kP1Stages * kP1StageBytes / 16; i += kP1Threads) reinterpret_cast<uint4*>(st_s)[i] = make_uint4(0, 0, 0, 0);
-    pdl_wait();                 // CTA-local set-up above overlaps the previous kernel's tail
     {
         // B operands from the packed im2col weights [k / 8][co][k % 8], k = 9 * c + tap: [tap][c / 8][co][c % 8].  The packed
         // block is staged in the (not yet used) raw-row buffer with 16-byte loads and re-ordered from there: 2-byte gathers
@@ -796,7 +787,6 @@ __global__ void __launch_bounds__(kP1Threads, 1) conv1_planes_kernel(const __gri
             }
             if (a.stamps && blockIdx.x == 0 && lane == 0) { a.stamps[9] = p_wait; a.stamps[10] = clock64() - p_begin; }
         }
-        pdl_release();
     } else {
         // ------------------------------------------------ epilogue warps 16..23: lane quarter warp % 4, two warps per quarter on
         // alternate tiles (one warp per quarter needs ~1000 cycles per tile between the TMEM load, 80 arithmetic
@@ -868,7 +858,7 @@ int64_t drq_conv1_w_packed_elems(void) { return kC1Units * 32 * 8 + 64; }
 
 int drq_pack_conv1_w_bf16(const float* w, const float* bias, uint16_t* out, int cin, void* stream) {
     DRQ_REQUIRE(w && bias && out && cin > 0 && cin * 9 + 1 <= kC1K, "pack_conv1_w: bad args (cin <= 10)");
-    launch_k(pack_conv1_w_kernel, 1, 256, 0, as_stream(stream), w, bias, reinterpret_cast<__nv_bfloat16*>(out), cin);
+    pack_conv1_w_kernel<<<1, 256, 0, as_stream(stream)>>>(w, bias, reinterpret_cast<__nv_bfloat16*>(out), cin);
     return check_launch("pack_conv1_w_kernel");
 }
 
@@ -952,14 +942,14 @@ static int conv1_fwd_launch(Conv1TcArgs& a, const int32_t* shift, const uint16_t
         if (int rc = ensure_smem((const void*)conv1_planes_kernel<0>, kConv1PlanesSmem, "conv1_fwd_bf16")) return rc;
         const int ptiles = N * kP1TilesPerImg;
         const int G = ptiles < sm_budget() ? ptiles : sm_budget();
-        if (cin == 9) launch_k(conv1_planes_kernel<9>, G, kP1Threads, kConv1PlanesSmem, stream, map, a);
-        else launch_k(conv1_planes_kernel<0>, G, kP1Threads, kConv1PlanesSmem, stream, map, a);
+        if (cin == 9) conv1_planes_kernel<9><<<G, kP1Threads, kConv1PlanesSmem, stream>>>(map, a);
+        else conv1_planes_kernel<0><<<G, kP1Threads, kConv1PlanesSmem, stream>>>(map, a);
         return check_launch("conv1_planes_kernel");
     }
     const int tiles = N * 14;
     const int G = tiles < sm_budget() ? tiles : sm_budget();
-    if (cin == 9) launch_k(conv1_tc_kernel<false, 9>, G, kC1Threads, kConv1FwdSmem, stream, a);
-    else launch_k(conv1_tc_kernel<false, 0>, G, kC1Threads, kConv1FwdSmem, stream, a);
+    if (cin == 9) conv1_tc_kernel<false, 9><<<G, kC1Threads, kConv1FwdSmem, stream>>>(a);
+    else conv1_tc_kernel<false, 0><<<G, kC1Threads, kConv1FwdSmem, stream>>>(a);
     return check_launch("conv1_tc_kernel<fwd>");
 }
 
@@ -986,11 +976,11 @@ static int conv1_wgrad_launch(Conv1TcArgs& a, const int32_t* shift, const uint16
     a.partial = partial;
     a.n_images = N;
     const int G = conv1_wgrad_ctas(N);
-    if (cin == 9) launch_k(conv1_tc_kernel<true, 9>, G, kC1Threads, kConv1WgSmem, stream, a);
-    else launch_k(conv1_tc_kernel<true, 0>, G, kC1Threads, kConv1WgSmem, stream, a);
+    if (cin == 9) conv1_tc_kernel<true, 9><<<G, kC1Threads, kConv1WgSmem, stream>>>(a);
+    else conv1_tc_kernel<true, 0><<<G, kC1Threads, kConv1WgSmem, stream>>>(a);
     if (int rc = check_launch("conv1_tc_kernel<wgrad>")) return rc;
     if (!dw) return DRQ_OK;                                   // partials only: reduced later by drq_conv_wgrad_reduce_multi
-    launch_k(conv1_wgrad_reduce_kernel, kC1ReduceBlocks, 256, 0, stream, partial, G, cin, dw, db);
+    conv1_wgrad_reduce_kernel<<<kC1ReduceBlocks, 256, 0, stream>>>(partial, G, cin, dw, db);
     return check_launch("conv1_wgrad_reduce_kernel");
 }
 

@@ -123,7 +123,6 @@ __global__ void __maxnreg__(128) conv4x1_tc_kernel(const __grid_constant__ CUten
     float* bias_s = reinterpret_cast<float*>(tmem_slot + 4);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    pdl_trigger();
     if (threadIdx.x == 0) {
         for (int i = 0; i < kStages; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
         for (int i = 0; i < kAcc; ++i) { mbar_init(tfull + i, 1); mbar_init(tempty + i, 8); }
@@ -133,10 +132,6 @@ __global__ void __maxnreg__(128) conv4x1_tc_kernel(const __grid_constant__ CUten
         tmem_alloc(tmem_slot, kAcc * 128);
         tmem_relinquish();
     }
-    // Programmatic dependent launch (the forward chain conv1 -> conv2 -> conv3 -> conv4): everything up to here and the
-    // weight expansion below touch nothing the previous kernel writes (parameters are from the previous update), so a CTA
-    // that gets its SM while other SMs still run the previous kernel's last tiles sets itself up meanwhile; the activation
-    // loads, the mask loads and the output stores wait for the previous grid (pdl_wait in every role).
     if (!DGRAD && threadIdx.x < 32) bias_s[threadIdx.x] = a.bias[threadIdx.x];
     tc_fence_before();
     __syncthreads();
@@ -145,7 +140,6 @@ __global__ void __maxnreg__(128) conv4x1_tc_kernel(const __grid_constant__ CUten
 
     if (warp == 1) {
         // ------------------------------------------------ TMA producer: one box per tile
-        pdl_wait();
         if (lane == 0) {
             int stage = 0; uint32_t phase = 0;
             long long st_empty = 0;
@@ -163,13 +157,11 @@ __global__ void __maxnreg__(128) conv4x1_tc_kernel(const __grid_constant__ CUten
             if (a.stamps && blockIdx.x == 0) { a.stamps[0] = st_empty; a.stamps[3] = clock64() - st_begin; }
         }
         __syncwarp();
-        pdl_release();
     } else {
         // ------------------------------------------------ everyone else first expands the weights
         expand_weights<DGRAD>(a.w, w_s, warp == 0 ? lane : threadIdx.x - 32);
         fence_proxy_async();
         asm volatile("bar.sync 1, %0;" ::"n"(kExpanders) : "memory");
-        pdl_wait();
         if (warp == 0) {
             // -------------------------------------------- UMMA issuer
             // A: K-major, 16-byte K units (channel blocks) 4 regions apart; B: K-major, K units 32 * cnt rows apart
@@ -391,14 +383,13 @@ int conv4x1_launch(bool dgrad, const __nv_bfloat16* in, long long cs_in, const _
         return DRQ_ERR_INVALID;
     }
     const int grid = a.total_tiles < sm_budget() ? a.total_tiles : sm_budget();
-    if (!dgrad) g_pdl_once = 1;       // drq_set_pdl(2): the forward chain's launches overlap their set-up with the predecessor's tail
     if (dgrad) {
         if (int rc = ensure_smem((const void*)conv4x1_tc_kernel<true>, kSmem, "conv4x1_dgrad")) return rc;
-        launch_k(conv4x1_tc_kernel<true>, grid, kThreads, kSmem, stream, map, a);
+        conv4x1_tc_kernel<true><<<grid, kThreads, kSmem, stream>>>(map, a);
         return check_launch("conv4x1_tc_kernel<dgrad>");
     }
     if (int rc = ensure_smem((const void*)conv4x1_tc_kernel<false>, kSmem, "conv4x1_fwd")) return rc;
-    launch_k(conv4x1_tc_kernel<false>, grid, kThreads, kSmem, stream, map, a);
+    conv4x1_tc_kernel<false><<<grid, kThreads, kSmem, stream>>>(map, a);
     return check_launch("conv4x1_tc_kernel<fwd>");
 }
 

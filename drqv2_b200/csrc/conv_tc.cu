@@ -88,7 +88,6 @@ __global__ void __launch_bounds__(kThreadsTC, 2) conv3x3_tc_kernel(ConvTcArgs a)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int total_tiles = a.n_images * a.ntiles;
-    pdl_trigger();
     if (threadIdx.x == 0) {
         for (int i = 0; i < kStagesTC; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
         for (int i = 0; i < kAccStages; ++i) { mbar_init(tfull + i, 1); mbar_init(tempty + i, 4); }
@@ -98,7 +97,6 @@ __global__ void __launch_bounds__(kThreadsTC, 2) conv3x3_tc_kernel(ConvTcArgs a)
         tmem_alloc(tmem_slot, kAccStages * 32);
         tmem_relinquish();
     }
-    pdl_wait();                 // CTA-local set-up above overlaps the previous kernel's tail
     if (!DGRAD && threadIdx.x < 32) bias_s[threadIdx.x] = a.bias[threadIdx.x];
 
     // packed weights -> smem (same byte layout)
@@ -132,7 +130,6 @@ __global__ void __launch_bounds__(kThreadsTC, 2) conv3x3_tc_kernel(ConvTcArgs a)
                     bulk_g2s(dst + lane * kStageRows * 16, a.in + (lane * a.cs_in + row0) * 8, kWinRows * 16, full + stage);
                 if (++stage == kStagesTC) { stage = 0; phase ^= 1; }
             }
-            pdl_release();                      // last window is on its way: the next kernel may set itself up
             CV_STAMPS(if (a.stamps && blockIdx.x == 0 && lane == 0) { a.stamps[0] = w_empty; a.stamps[1] = CV_T() - t_begin; })
         }
     } else if (warp == 1) {
@@ -283,8 +280,6 @@ __global__ void __launch_bounds__(kThreadsTC, 2) conv3x3_tc_kernel(ConvTcArgs a)
 
 __global__ void pack_conv_w_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ w_fwd,
                                    __nv_bfloat16* __restrict__ w_dgrad) {
-    pdl_trigger();
-    pdl_wait();
     pack_conv_w_elem(w, w_fwd, w_dgrad, blockIdx.x * blockDim.x + threadIdx.x);
 }
 
@@ -328,7 +323,6 @@ __global__ void __launch_bounds__(kThreadsTC, 1) conv3x3_wgrad_tc_kernel(WgradTc
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int total_tiles = a.n_images * a.ntiles;
     const int cta = blockIdx.x, ncta = gridDim.x;
-    pdl_trigger();
     for (int i = threadIdx.x; i < kWgStages * (kWgPlane / 4); i += kThreadsTC) {
         const int st = i / (kWgPlane / 4), w = i - st * (kWgPlane / 4);
         reinterpret_cast<uint32_t*>(st_s + st * kWgStageBytes + 12 * kWgPlane)[w] = 0x3F803F80u;    // bf16 1.0 x2
@@ -346,7 +340,6 @@ __global__ void __launch_bounds__(kThreadsTC, 1) conv3x3_wgrad_tc_kernel(WgradTc
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    pdl_wait();
     const uint32_t tmem_base = *tmem_slot;
 
     if (warp == 0) {
@@ -365,7 +358,6 @@ __global__ void __launch_bounds__(kThreadsTC, 1) conv3x3_wgrad_tc_kernel(WgradTc
                 bulk_g2s(dst + kWgABytes + (lane - 12) * kWgDRows * 16, a.d + ((lane - 12) * a.cs_d + row0) * 8, kWgDRows * 16, full + stage);
             if (++stage == kWgStages) { stage = 0; phase ^= 1; }
         }
-        pdl_release();
     } else if (warp == 1) {
         constexpr uint32_t idesc = make_idesc_bf16(128, 32, true, true);
         int stage = 0; uint32_t phase = 0;
@@ -421,8 +413,6 @@ __global__ void __launch_bounds__(kThreadsTC, 1) conv3x3_wgrad_tc_kernel(WgradTc
 
 __global__ void __launch_bounds__(256) wgrad_tc_reduce_kernel(const float* __restrict__ partial, int G, float* __restrict__ dw,
                                                               float* __restrict__ db) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float red[8][33];
     wgrad3x3_reduce_block(partial, G, dw, db, blockIdx.x, red);
 }
@@ -448,18 +438,6 @@ extern "C" {
 
 int drq_debug_conv_stamps(int64_t* buf) { g_conv_stamps = reinterpret_cast<long long*>(buf); return DRQ_OK; }
 
-// self-test of drq_debug_trap_note: one thread waits on a barrier nobody arrives on (bounded: ~2^20 polls), then traps
-__global__ void debug_force_timeout_kernel() {
-    __shared__ uint64_t bar;
-    mbar_init(&bar, 1);
-    fence_barrier_init();
-    mbar_wait(&bar, 0);
-}
-int drq_debug_force_timeout(void* stream) {
-    launch_k(debug_force_timeout_kernel, 1, 1, 0, as_stream(stream));
-    return check_launch("debug_force_timeout_kernel");
-}
-
 int drq_set_conv4x1(int mode) {
     const int prev = g_conv4x1;
     if (mode >= 0 && mode <= 4) g_conv4x1 = mode;
@@ -470,7 +448,7 @@ int64_t drq_wb_elems(int n_images) { return 4ll * ((long long)n_images * kPLB + 
 
 int drq_pack_conv_w_bf16(const float* w, uint16_t* w_fwd, uint16_t* w_dgrad, void* stream) {
     DRQ_REQUIRE(w && w_fwd && w_dgrad, "pack_conv_w: null pointer");
-    launch_k(pack_conv_w_kernel, (9216 + 255) / 256, 256, 0, as_stream(stream), 
+    pack_conv_w_kernel<<<(9216 + 255) / 256, 256, 0, as_stream(stream)>>>(
         w, reinterpret_cast<__nv_bfloat16*>(w_fwd), reinterpret_cast<__nv_bfloat16*>(w_dgrad));
     return check_launch("pack_conv_w_kernel");
 }
@@ -500,7 +478,7 @@ int drq_conv3x3_fwd_bf16(const uint16_t* in, const uint16_t* w_fwd, const float*
     if (use_conv4x1(N, false))
         return conv4x1_launch(false, a.in, a.cs_in, a.w, bias, nullptr, 0, a.out, a.cs_out, N, hout, nhwc_out, feat_rpad, a.feat_half,
                               feat_half_row, as_stream(stream));
-    launch_k(conv3x3_tc_kernel<false>, conv_tc_grid(N * a.ntiles, 2), kThreadsTC, kConvTcSmem, as_stream(stream), a);
+    conv3x3_tc_kernel<false><<<conv_tc_grid(N * a.ntiles, 2), kThreadsTC, kConvTcSmem, as_stream(stream)>>>(a);
     return check_launch("conv3x3_tc_kernel<fwd>");
 }
 
@@ -526,7 +504,7 @@ int drq_conv3x3_dgrad_bf16(const uint16_t* dout, const uint16_t* w_dgrad, const 
     a.stamps = g_conv_stamps;
     if (use_conv4x1(N, true))
         return conv4x1_launch(true, a.in, a.cs_in, a.w, nullptr, a.mask, a.cs_mask, a.out, a.cs_out, N, hout, 0, 0, 0, 0, as_stream(stream));
-    launch_k(conv3x3_tc_kernel<true>, conv_tc_grid(N * a.ntiles, 2), kThreadsTC, kConvTcSmem, as_stream(stream), a);
+    conv3x3_tc_kernel<true><<<conv_tc_grid(N * a.ntiles, 2), kThreadsTC, kConvTcSmem, as_stream(stream)>>>(a);
     return check_launch("conv3x3_tc_kernel<dgrad>");
 }
 
@@ -546,10 +524,10 @@ int drq_conv3x3_wgrad_bf16(const uint16_t* in, int n_in, const uint16_t* dpre, f
     a.n_images = N;
     a.ntiles = (hout * kPW + kTM - 1) / kTM;
     const int G = conv_wgrad_ctas(N, hout);                   // tile walkers, one per SM
-    launch_k(conv3x3_wgrad_tc_kernel, G, kThreadsTC, kWgradTcSmem, as_stream(stream), a);
+    conv3x3_wgrad_tc_kernel<<<G, kThreadsTC, kWgradTcSmem, as_stream(stream)>>>(a);
     if (int rc = check_launch("conv3x3_wgrad_tc_kernel")) return rc;
     if (!dw) return DRQ_OK;                                   // partials only: reduced later by drq_conv_wgrad_reduce_multi
-    launch_k(wgrad_tc_reduce_kernel, kWgReduceBlocks, 256, 0, as_stream(stream), partial, G, dw, db);
+    wgrad_tc_reduce_kernel<<<kWgReduceBlocks, 256, 0, as_stream(stream)>>>(partial, G, dw, db);
     return check_launch("wgrad_tc_reduce_kernel");
 }
 

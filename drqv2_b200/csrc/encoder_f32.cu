@@ -25,8 +25,6 @@ __global__ void __launch_bounds__(128)
 conv3x3_wide_kernel(const float* __restrict__ in, const float* __restrict__ w,
                     const float* __restrict__ bias, const float* __restrict__ act_mask,
                     float* __restrict__ out, int n_pos, int w_valid, int compact_out) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ __align__(16) float smem[];
     float* in_s = smem;                 // [32][kWin]
     float* w_s = smem + kCh * kWin;     // [9][32 s][32 d]
@@ -112,8 +110,6 @@ conv3x3_wide_kernel(const float* __restrict__ in, const float* __restrict__ w,
 __global__ void __launch_bounds__(128)
 conv3x3_wgrad_kernel(const float* __restrict__ in, const float* __restrict__ dpre,
                      float* __restrict__ partial, int N, int n_pos, int ntiles) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ __align__(16) float smem[];
     constexpr int kDS = kTP + 4;   // padded row: conflict-free LDS.128 over 8 lanes
     float* d_s = smem;             // [32][kDS]
@@ -192,8 +188,6 @@ conv3x3_wgrad_kernel(const float* __restrict__ in, const float* __restrict__ dpr
 // dw[i] = sum_g partial[g][i] (i < nw), db[i - nw] likewise; fixed order.
 __global__ void wgrad_reduce_kernel(const float* __restrict__ partial, int G, int nw, int nb,
                                     float* __restrict__ dw, float* __restrict__ db) {
-    pdl_trigger();
-    pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const int row = nw + nb;
     if (i >= row) return;
@@ -224,8 +218,6 @@ __global__ void __launch_bounds__(288)
 conv1_fwd_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shift,
                  const float* __restrict__ w, const float* __restrict__ bias,
                  float* __restrict__ out, int cin, int pad) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ __align__(16) float smem[];
     float* x_s = smem;                              // [cin][15][84]
     float* w_s = smem + cin * kC1InRows * kImg;     // [cin*9][32]
@@ -276,8 +268,6 @@ __global__ void __launch_bounds__(256)
 conv1_wgrad_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shift,
                    const float* __restrict__ dpre, float* __restrict__ partial, int N, int cin,
                    int pad) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ __align__(16) float smem[];
     constexpr int kDS = kC1Rows * kPW + 1;   // 288
     float* x_s = smem;                              // [cin][15][84]
@@ -360,7 +350,7 @@ int drq_conv1_fwd_f32(const uint8_t* obs, const int32_t* shift, const float* w, 
     if (N == 0) return DRQ_OK;
     const size_t smem = (size_t)(cin * kC1InRows * kImg + cin * 9 * kCh) * sizeof(float);
     if (int rc = set_smem(conv1_fwd_kernel, smem, "conv1_fwd")) return rc;
-    launch_k(conv1_fwd_kernel, dim3(kC1Tiles, N), 288, smem, as_stream(stream), obs, shift, w, b, out, cin, pad);
+    conv1_fwd_kernel<<<dim3(kC1Tiles, N), 288, smem, as_stream(stream)>>>(obs, shift, w, b, out, cin, pad);
     return check_launch("conv1_fwd_kernel");
 }
 
@@ -372,10 +362,10 @@ int drq_conv1_wgrad_f32(const uint8_t* obs, const int32_t* shift, const float* d
     if (int rc = set_smem(conv1_wgrad_kernel, smem, "conv1_wgrad")) return rc;
     const int items = N * kC1Tiles;
     const int G = items < kWgradBlocks ? items : kWgradBlocks;
-    launch_k(conv1_wgrad_kernel, G, 256, smem, as_stream(stream), obs, shift, dpre, partial, N, cin, pad);
+    conv1_wgrad_kernel<<<G, 256, smem, as_stream(stream)>>>(obs, shift, dpre, partial, N, cin, pad);
     if (int rc = check_launch("conv1_wgrad_kernel")) return rc;
     const int nw = kCh * cin * 9;
-    launch_k(wgrad_reduce_kernel, (nw + kCh + 127) / 128, 128, 0, as_stream(stream), partial, G, nw, kCh, dw, db);
+    wgrad_reduce_kernel<<<(nw + kCh + 127) / 128, 128, 0, as_stream(stream)>>>(partial, G, nw, kCh, dw, db);
     return check_launch("wgrad_reduce_kernel");
 }
 
@@ -387,7 +377,7 @@ int drq_conv3x3_fwd_f32(const float* in, const float* w, const float* b, float* 
     const size_t smem = (size_t)(kCh * kWin + 9 * kCh * kCh) * sizeof(float);
     if (int rc = set_smem(conv3x3_wide_kernel<false>, smem, "conv3x3_fwd")) return rc;
     const int n_pos = hout * kPW;
-    launch_k(conv3x3_wide_kernel<false>, dim3((n_pos + kTP - 1) / kTP, N), 128, smem, as_stream(stream), 
+    conv3x3_wide_kernel<false><<<dim3((n_pos + kTP - 1) / kTP, N), 128, smem, as_stream(stream)>>>(
         in, w, b, nullptr, out, n_pos, hout, compact_out);
     return check_launch("conv3x3_fwd_kernel");
 }
@@ -401,7 +391,7 @@ int drq_conv3x3_dgrad_f32(const float* dout, const float* w, const float* act_in
     if (int rc = set_smem(conv3x3_wide_kernel<true>, smem, "conv3x3_dgrad")) return rc;
     const int hin = hout + 2;
     const int n_pos = hin * kPW;
-    launch_k(conv3x3_wide_kernel<true>, dim3((n_pos + kTP - 1) / kTP, N), 128, smem, as_stream(stream), 
+    conv3x3_wide_kernel<true><<<dim3((n_pos + kTP - 1) / kTP, N), 128, smem, as_stream(stream)>>>(
         dout, w, nullptr, act_in, din, n_pos, hin, 0);
     return check_launch("conv3x3_dgrad_kernel");
 }
@@ -416,10 +406,10 @@ int drq_conv3x3_wgrad_f32(const float* in, const float* dpre, float* partial, fl
     const int ntiles = (n_pos + kTP - 1) / kTP;
     const int items = N * ntiles;
     const int G = items < kWgradBlocks ? items : kWgradBlocks;
-    launch_k(conv3x3_wgrad_kernel, G, 128, smem, as_stream(stream), in, dpre, partial, N, n_pos, ntiles);
+    conv3x3_wgrad_kernel<<<G, 128, smem, as_stream(stream)>>>(in, dpre, partial, N, n_pos, ntiles);
     if (int rc = check_launch("conv3x3_wgrad_kernel")) return rc;
     const int nw = kCh * kCh * 9;
-    launch_k(wgrad_reduce_kernel, (nw + kCh + 127) / 128, 128, 0, as_stream(stream), partial, G, nw, kCh, dw, db);
+    wgrad_reduce_kernel<<<(nw + kCh + 127) / 128, 128, 0, as_stream(stream)>>>(partial, G, nw, kCh, dw, db);
     return check_launch("wgrad_reduce_kernel");
 }
 

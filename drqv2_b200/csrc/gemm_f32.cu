@@ -28,8 +28,6 @@ __device__ __forceinline__ long long compact_to_wide(int k) {
 }
 
 __global__ void __launch_bounds__(256) gemm_f32_kernel(GemmArgs g) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ __align__(16) float As[BK][BM + kPad];
     __shared__ __align__(16) float Bs[BK][BN + kPad];
     const int tid = threadIdx.x;
@@ -129,8 +127,6 @@ __global__ void __launch_bounds__(256) gemm_f32_kernel(GemmArgs g) {
 __global__ void __launch_bounds__(256)
 colsum_kernel(const float* __restrict__ X, long long ld, float* __restrict__ out, int M, int N,
               long long bs_x, long long bs_out) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float red[8][33];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int n = blockIdx.x * 32 + tx;
@@ -181,14 +177,14 @@ int drq_gemm_f32(const float* A, int64_t sa_m, int64_t sa_k, const float* B, int
         DRQ_REQUIRE((long long)chunk * (splitk - 1) < K, "gemm: splitk %d leaves empty chunks for K=%d", splitk, K);
     }
     dim3 grid((N + BN - 1) / BN, (M + BM - 1) / BM, splitk > 1 ? splitk : batch);
-    launch_k(gemm_f32_kernel, grid, 256, 0, as_stream(stream), g);
+    gemm_f32_kernel<<<grid, 256, 0, as_stream(stream)>>>(g);
     return check_launch("gemm_f32_kernel");
 }
 
 int drq_colsum_f32(const float* X, int64_t ld, float* out, int M, int N, int batch, int64_t bs_x,
                    int64_t bs_out, void* stream) {
     DRQ_REQUIRE(X && out && M > 0 && N > 0 && batch > 0, "colsum: bad args");
-    launch_k(colsum_kernel, dim3((N + 31) / 32, batch), 256, 0, as_stream(stream), X, ld, out, M, N, bs_x, bs_out);
+    colsum_kernel<<<dim3((N + 31) / 32, batch), 256, 0, as_stream(stream)>>>(X, ld, out, M, N, bs_x, bs_out);
     return check_launch("colsum_kernel");
 }
 

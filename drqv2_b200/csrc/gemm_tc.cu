@@ -130,7 +130,6 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const GemmTcArgs
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + ACC);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    pdl_trigger();
     if (tid == 0) GT_STAMP(0);
     const int nt = (g.N + BN - 1) / BN, mt = (g.M + GT_BM - 1) / GT_BM;
     const int total_tiles = g.grid3d ? 1 : nt * mt * g.nz;
@@ -155,7 +154,6 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const GemmTcArgs
         asm volatile("bar.sync 2, 192;" ::: "memory");
         tc_fence_after();
     }
-    pdl_wait();                 // everything above is CTA-local; global memory is first touched below
     const uint32_t tmem_base = warp == 0 ? 0u : *tmem_slot;
     if (tid == 0) GT_STAMP(1);
 
@@ -211,7 +209,6 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const GemmTcArgs
                 }
             }
         }
-        pdl_release();                          // last tiles are on their way: the next kernel may set itself up
         if (lane == 0) GT_STAMP(3);
     } else if (warp == 1) {
         // ------------------------------------------------ UMMA issuer
@@ -423,21 +420,17 @@ static int launch_gemm_tc(GemmTcArgs& g, int batch, cudaStream_t s) {
     const int tiles = nt * mt * g.nz;
     const int sms = drq_device_sm_count();
     g.grid3d = tiles <= sms ? 1 : 0;
-    launch_k(gemm_tc_kernel<MODE, BN, EPI, SMALL>, g.grid3d ? dim3(nt, mt, g.nz) : dim3(sms), GT_THREADS, Cfg::SMEM, s, g);
+    gemm_tc_kernel<MODE, BN, EPI, SMALL><<<g.grid3d ? dim3(nt, mt, g.nz) : dim3(sms), GT_THREADS, Cfg::SMEM, s>>>(g);
     return check_launch("gemm_tc_kernel");
 }
 
 __global__ void __launch_bounds__(256)
 pack_linear_tb_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ out, int rows, int cols, int units) {
-    pdl_trigger();
-    pdl_wait();
     pack_linear_tb_block(w, out, rows, cols, units, blockIdx.x, blockIdx.y, threadIdx.x);
 }
 
 __global__ void __launch_bounds__(256)
 pack_trunk_tb_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ out, int rows) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float tile[32][33];
     pack_trunk_tb_block(w, out, rows, blockIdx.x, blockIdx.y, threadIdx.x, tile);
 }
@@ -446,8 +439,6 @@ pack_trunk_tb_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ ou
 // order (stage API: update_critic / update_actor on externally supplied features)
 __global__ void __launch_bounds__(256)
 pack_features_tb_kernel(const float* __restrict__ f, __nv_bfloat16* __restrict__ out, int rows) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float tile[32][33];
     pack_trunk_tb_block<DRQ_TB_ACT>(f, out, rows, blockIdx.x, blockIdx.y, threadIdx.x, tile);
 }
@@ -536,7 +527,7 @@ int drq_pack_linear_tb(const float* w, uint16_t* out, int rows, int cols, void* 
     DRQ_REQUIRE(w && out && rows > 0 && cols > 0, "pack_linear_tb: bad args");
     const int units = (cols + 15) / 16 * 2;
     const int rpad = (rows + RW - 1) / RW * RW;
-    launch_k(pack_linear_tb_kernel, dim3((rpad + 255) / 256, units), 256, 0, as_stream(stream), 
+    pack_linear_tb_kernel<<<dim3((rpad + 255) / 256, units), 256, 0, as_stream(stream)>>>(
         w, reinterpret_cast<__nv_bfloat16*>(out), rows, cols, units);
     return check_launch("pack_linear_tb_kernel");
 }
@@ -544,7 +535,7 @@ int drq_pack_linear_tb(const float* w, uint16_t* out, int rows, int cols, void* 
 int drq_pack_trunk_tb(const float* w, uint16_t* out, int rows, void* stream) {
     DRQ_REQUIRE(w && out && rows > 0, "pack_trunk_tb: bad args");
     const int rpad = (rows + RW - 1) / RW * RW;
-    launch_k(pack_trunk_tb_kernel, dim3((1225 + 31) / 32, rpad), 256, 0, as_stream(stream), 
+    pack_trunk_tb_kernel<<<dim3((1225 + 31) / 32, rpad), 256, 0, as_stream(stream)>>>(
         w, reinterpret_cast<__nv_bfloat16*>(out), rows);
     return check_launch("pack_trunk_tb_kernel");
 }
@@ -553,7 +544,7 @@ int drq_pack_features_tb(const float* feat, uint16_t* out, int rows, void* strea
     DRQ_REQUIRE(feat && out && rows > 0, "pack_features_tb: bad args");
     DRQ_REQUIRE(((uintptr_t)out % 16) == 0, "pack_features_tb: output must be 16-byte aligned");
     const int rpad = (rows + RA - 1) / RA * RA;
-    launch_k(pack_features_tb_kernel, dim3((1225 + 31) / 32, rpad), 256, 0, as_stream(stream),
+    pack_features_tb_kernel<<<dim3((1225 + 31) / 32, rpad), 256, 0, as_stream(stream)>>>(
         feat, reinterpret_cast<__nv_bfloat16*>(out), rows);
     return check_launch("pack_features_tb_kernel");
 }

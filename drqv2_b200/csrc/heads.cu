@@ -25,8 +25,6 @@ ln_tanh_fwd_kernel(const LnJobs jobs, int B, int F, float eps) {
     // One block per (row, job): the four warps sum interleaved quarters of the split-K planes (all loads of a
     // warp in flight at once), the partial rows are combined in fixed order, warp 0 normalises.
     __shared__ float part[4][32 * NF];
-    pdl_trigger();
-    pdl_wait();
     const drq_ln_job& jb = jobs.j[blockIdx.y];
     const int row = blockIdx.x;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -97,8 +95,6 @@ ln_tanh_bwd_row_kernel(const float* __restrict__ dh, long long ld_dh, const floa
                        const float* __restrict__ rstd, const float* __restrict__ gamma,
                        float* __restrict__ dz, float* __restrict__ dy_out, __nv_bfloat16* __restrict__ dz_bf,
                        long long rpad_zb, int B, int F, int n_planes, long long plane_stride) {
-    pdl_trigger();
-    pdl_wait();
     const int row = blockIdx.x * 4 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= B) return;
@@ -145,8 +141,6 @@ ln_tanh_bwd_row_kernel(const float* __restrict__ dh, long long ld_dh, const floa
 __global__ void __launch_bounds__(256)
 ln_param_grad_kernel(const float* __restrict__ dy, const float* __restrict__ xhat,
                      float* __restrict__ dgamma, float* __restrict__ dbeta, int B, int F) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float sg[256], sb[256];
     const int f = blockIdx.x;
     float g = 0.f, b = 0.f;
@@ -181,10 +175,7 @@ __device__ __forceinline__ float block_sum_256(float v, float* sh) {
 __global__ void __launch_bounds__(256)
 actor_sample_kernel(const float* __restrict__ mu_pre, const float* __restrict__ eps,
                     const float* __restrict__ std_dev, float clip, float* __restrict__ action_out,
-                    long long ld_a, float* __restrict__ mu_out, float* __restrict__ metrics,
-                    __nv_bfloat16* __restrict__ a_bf, long long rpad_ab, int feat_off, int B, int A) {
-    pdl_trigger();
-    pdl_wait();
+                    long long ld_a, float* __restrict__ mu_out, float* __restrict__ metrics, int B, int A) {
     __shared__ float sh[256];
     const float std = std_dev ? *std_dev : 0.f;
     const float lo = -1.0f + 1e-6f, hi = 1.0f - 1e-6f;  // utils.py:113 (python: -1.0 + 1e-6 -> fp32)
@@ -205,7 +196,6 @@ actor_sample_kernel(const float* __restrict__ mu_pre, const float* __restrict__ 
                 lp += -(d * d) / (2.0f * std * std) - log_std - 0.9189385332046727f;
             }
             action_out[(long long)b * ld_a + j] = a;
-            if (a_bf) a_bf[fb_index(feat_off + j, b, rpad_ab)] = __float2bfloat16_rn(a);
             if (mu_out) mu_out[(long long)b * A + j] = mu;
         }
         lp_sum += lp;
@@ -234,8 +224,6 @@ __global__ void __launch_bounds__(256)
 policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, const float* __restrict__ w4,
                        const float* __restrict__ b4, float* __restrict__ mu_pre, int M, int H, int A, const PolicyJobs jobs,
                        const float* __restrict__ std_dev, float clip, unsigned int* __restrict__ scratch) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ float w_s[];                       // [A][H]
     __shared__ float sh[256];
     __shared__ int s_last;
@@ -350,8 +338,6 @@ __global__ void actor_sample_bwd_kernel(const float* __restrict__ da, long long 
                                         const float* __restrict__ mu, float* __restrict__ dmu_pre,
                                         __nv_bfloat16* __restrict__ dmu_bf, long long rpad_mb, int B, int A,
                                         int n_planes, long long plane_stride) {
-    pdl_trigger();
-    pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= B * A) return;
     const int b = i / A, j = i - b * A;
@@ -376,8 +362,6 @@ critic_loss_kernel(const float* __restrict__ q1, const float* __restrict__ q2,
                    const float* __restrict__ reward, const float* __restrict__ discount,
                    float* __restrict__ dq1, float* __restrict__ dq2, float* __restrict__ tq_out,
                    float* __restrict__ metrics, int B) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float sh[256];
     float s_r = 0.f, s_t = 0.f, s_1 = 0.f, s_2 = 0.f, s_l1 = 0.f, s_l2 = 0.f;
     const float scale = 2.0f / (float)B;
@@ -408,8 +392,6 @@ __global__ void __launch_bounds__(256)
 actor_loss_kernel(const float* __restrict__ q1, const float* __restrict__ q2,
                   float* __restrict__ dq1, float* __restrict__ dq2, float* __restrict__ metrics,
                   int B) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float sh[256];
     float s = 0.f;
     const float g = -1.0f / (float)B;
@@ -431,8 +413,6 @@ __global__ void __launch_bounds__(256)
 q_head_fwd_kernel(const __nv_bfloat16* __restrict__ c2, long long rpad, long long bs_c2,
                   const float* __restrict__ w3, const float* __restrict__ b3, float* __restrict__ q, int B, int H,
                   long long w_stride, int heads_inner, long long w_stride_outer) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ float w_s[];
     __shared__ float part[8][33];
     const int z = blockIdx.y;
@@ -497,8 +477,6 @@ __global__ void __launch_bounds__(256)
 q_head_bwd_kernel(const float* __restrict__ dq, const QLossArgs L, const __nv_bfloat16* __restrict__ c2, long long rpad,
                   long long bs_c2, const float* __restrict__ w3, __nv_bfloat16* __restrict__ dc2,
                   float* __restrict__ dw3, float* __restrict__ db3, int B, long long w_stride) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float red[256][9];
     const int u = blockIdx.x, z = blockIdx.y;
     const float* dqz = LOSS == 0 ? dq + (long long)z * B : nullptr;
@@ -595,9 +573,9 @@ int drq_ln_tanh_fwd_multi(const drq_ln_job* jobs, int njobs, int B, int F, float
     if (B == 0) return DRQ_OK;
     const dim3 grid(B, njobs);
     cudaStream_t s = as_stream(stream);
-    if (F <= 64) launch_k(ln_tanh_fwd_kernel<2>, grid, 128, 0, s, js, B, F, eps);
-    else if (F <= 128) launch_k(ln_tanh_fwd_kernel<4>, grid, 128, 0, s, js, B, F, eps);
-    else launch_k(ln_tanh_fwd_kernel<8>, grid, 128, 0, s, js, B, F, eps);
+    if (F <= 64) ln_tanh_fwd_kernel<2><<<grid, 128, 0, s>>>(js, B, F, eps);
+    else if (F <= 128) ln_tanh_fwd_kernel<4><<<grid, 128, 0, s>>>(js, B, F, eps);
+    else ln_tanh_fwd_kernel<8><<<grid, 128, 0, s>>>(js, B, F, eps);
     return check_launch("ln_tanh_fwd_kernel");
 }
 
@@ -619,25 +597,22 @@ int drq_ln_tanh_bwd(const float* dh, int64_t ld_dh, const float* h, int64_t ld_h
     DRQ_REQUIRE(B > 0 && F > 0 && F <= 32 * kMaxFPerLane, "ln_tanh_bwd: bad dims (F<=256)");
     // dy = dh * tanh' is staged in the second half of the caller's 2*B*F buffer
     float* dy = dz + (long long)B * F;
-    launch_k(ln_tanh_bwd_row_kernel, (B + 3) / 4, 128, 0, as_stream(stream), dh, ld_dh, h, ld_h, xhat, rstd,
+    ln_tanh_bwd_row_kernel<<<(B + 3) / 4, 128, 0, as_stream(stream)>>>(dh, ld_dh, h, ld_h, xhat, rstd,
                                                                       gamma, dz, dy,
                                                                       reinterpret_cast<__nv_bfloat16*>(dz_bf16), rpad_zb, B, F,
                                                                       n_planes, plane_stride);
     if (int rc = check_launch("ln_tanh_bwd_row_kernel")) return rc;
     if (!dgamma) return DRQ_OK;
-    launch_k(ln_param_grad_kernel, F, 256, 0, as_stream(stream), dy, xhat, dgamma, dbeta, B, F);
+    ln_param_grad_kernel<<<F, 256, 0, as_stream(stream)>>>(dy, xhat, dgamma, dbeta, B, F);
     return check_launch("ln_param_grad_kernel");
 }
 
 int drq_actor_sample(const float* mu_pre, const float* eps, const float* std_dev, float clip,
-                     float* action_out, int64_t ld_a, float* mu_out, float* metrics, uint16_t* action_bf16,
-                     int64_t rpad_ab, int feat_off, int B, int A, void* stream) {
+                     float* action_out, int64_t ld_a, float* mu_out, float* metrics, int B, int A, void* stream) {
     DRQ_REQUIRE(mu_pre && action_out, "actor_sample: null pointer");
     DRQ_REQUIRE(!(eps && !std_dev), "actor_sample: eps without std");
     DRQ_REQUIRE(B > 0 && A > 0, "actor_sample: bad dims");
-    launch_k(actor_sample_kernel, 1, 256, 0, as_stream(stream), mu_pre, eps, std_dev, clip, action_out, ld_a,
-                                                          mu_out, metrics,
-                                                          reinterpret_cast<__nv_bfloat16*>(action_bf16), rpad_ab, feat_off, B, A);
+    actor_sample_kernel<<<1, 256, 0, as_stream(stream)>>>(mu_pre, eps, std_dev, clip, action_out, ld_a, mu_out, metrics, B, A);
     return check_launch("actor_sample_kernel");
 }
 
@@ -663,7 +638,7 @@ int drq_policy_head_fwd_bf16(const uint16_t* p2, int64_t units, const float* w4,
     DRQ_REQUIRE(pj.metrics_job < 0 || (M + kPolicyRows - 1) / kPolicyRows <= 4096, "policy_head_fwd: the metrics scratch holds 4096 block partials (M <= 32768)");
     const size_t smem = (size_t)A * H * sizeof(float);
     if (int rc = ensure_smem((const void*)policy_head_fwd_kernel, smem, "policy_head_fwd")) return rc;
-    launch_k(policy_head_fwd_kernel, (M + kPolicyRows - 1) / kPolicyRows, 256, smem, as_stream(stream), reinterpret_cast<const __nv_bfloat16*>(p2),
+    policy_head_fwd_kernel<<<(M + kPolicyRows - 1) / kPolicyRows, 256, smem, as_stream(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(p2),
              (long long)units, w4, b4, mu_pre, M, H, A, pj, std_dev, clip, ticket);
     return check_launch("policy_head_fwd_kernel");
 }
@@ -672,7 +647,7 @@ int drq_actor_sample_bwd(const float* daction, int64_t ld_da, const float* mu, f
                          uint16_t* dmu_bf16, int64_t rpad_mb, int B, int A, int n_planes, int64_t plane_stride,
                          void* stream) {
     DRQ_REQUIRE(daction && mu && dmu_pre && B > 0 && A > 0 && n_planes >= 1, "actor_sample_bwd: bad args");
-    launch_k(actor_sample_bwd_kernel, (B * A + 255) / 256, 256, 0, as_stream(stream), daction, ld_da, mu,
+    actor_sample_bwd_kernel<<<(B * A + 255) / 256, 256, 0, as_stream(stream)>>>(daction, ld_da, mu,
                                                                                 dmu_pre,
                                                                                 reinterpret_cast<__nv_bfloat16*>(dmu_bf16), rpad_mb, B, A,
                                                                                 n_planes, plane_stride);
@@ -684,7 +659,7 @@ int drq_critic_loss(const float* q1, const float* q2, const float* tq1, const fl
                     float* target_q_out, float* metrics, int B, void* stream) {
     DRQ_REQUIRE(q1 && q2 && tq1 && tq2 && reward && discount && dq1 && dq2, "critic_loss: null pointer");
     DRQ_REQUIRE(B > 0, "critic_loss: bad dims");
-    launch_k(critic_loss_kernel, 1, 256, 0, as_stream(stream), q1, q2, tq1, tq2, reward, discount, dq1, dq2,
+    critic_loss_kernel<<<1, 256, 0, as_stream(stream)>>>(q1, q2, tq1, tq2, reward, discount, dq1, dq2,
                                                          target_q_out, metrics, B);
     return check_launch("critic_loss_kernel");
 }
@@ -693,7 +668,7 @@ int drq_q_head_fwd_bf16(const uint16_t* c2, int64_t rpad, int64_t bs_c2, const f
                         float* q, int B, int H, int heads, int64_t w_stride, int heads_inner, int64_t w_stride_outer,
                         void* stream) {
     DRQ_REQUIRE(c2 && w3 && b3 && q && B > 0 && H > 0 && H % 8 == 0 && heads > 0 && heads_inner > 0, "q_head_fwd: bad args");
-    launch_k(q_head_fwd_kernel, dim3((B + 31) / 32, heads), 256, H * sizeof(float), as_stream(stream), 
+    q_head_fwd_kernel<<<dim3((B + 31) / 32, heads), 256, H * sizeof(float), as_stream(stream)>>>(
         reinterpret_cast<const __nv_bfloat16*>(c2), rpad, bs_c2, w3, b3, q, B, H, w_stride, heads_inner, w_stride_outer);
     return check_launch("q_head_fwd_kernel");
 }
@@ -709,10 +684,10 @@ int drq_q_head_bwd_loss_bf16(int loss, const float* q, const float* tq, const fl
     const auto c2p = reinterpret_cast<const __nv_bfloat16*>(c2);
     const auto dp = reinterpret_cast<__nv_bfloat16*>(dc2);
     if (loss == 1)
-        launch_k(q_head_bwd_kernel<1>, dim3(H / 8, 2), 256, 0, as_stream(stream), nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
+        q_head_bwd_kernel<1><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
                  B, w_stride);
     else
-        launch_k(q_head_bwd_kernel<2>, dim3(H / 8, 2), 256, 0, as_stream(stream), nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
+        q_head_bwd_kernel<2><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
                  B, w_stride);
     return check_launch("q_head_bwd_kernel");
 }
@@ -720,7 +695,7 @@ int drq_q_head_bwd_loss_bf16(int loss, const float* q, const float* tq, const fl
 int drq_actor_loss(const float* q1, const float* q2, float* dq1, float* dq2, float* metrics, int B,
                    void* stream) {
     DRQ_REQUIRE(q1 && q2 && dq1 && dq2 && B > 0, "actor_loss: bad args");
-    launch_k(actor_loss_kernel, 1, 256, 0, as_stream(stream), q1, q2, dq1, dq2, metrics, B);
+    actor_loss_kernel<<<1, 256, 0, as_stream(stream)>>>(q1, q2, dq1, dq2, metrics, B);
     return check_launch("actor_loss_kernel");
 }
 

@@ -10,8 +10,6 @@ namespace drq {
 struct PackJobs { drq_pack_job j[DRQ_PACK_MAX_JOBS]; int first_block[DRQ_PACK_MAX_JOBS + 1]; int n; };
 
 __global__ void __launch_bounds__(256) pack_multi_kernel(const PackJobs jobs) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ float sm[32 * 33];
     int ji = 0;
     while (ji + 1 < jobs.n && (int)blockIdx.x >= jobs.first_block[ji + 1]) ++ji;
@@ -38,8 +36,6 @@ struct ColsumJobs { drq_colsum_job j[DRQ_COLSUM_MAX_JOBS]; };
 //   TB bf16   : 4 units x 64 row lanes, one 16-byte load (8 columns of one row) per thread and step.
 __global__ void __launch_bounds__(256) colsum_multi_kernel(const ColsumJobs jobs) {
     __shared__ float red[64][33];
-    pdl_trigger();
-    pdl_wait();
     const drq_colsum_job& jb = jobs.j[blockIdx.y];
     if (blockIdx.x * 32 >= jb.N) return;
     if (jb.tb) {
@@ -92,8 +88,6 @@ struct WgReduceJobs { drq_wgrad_reduce_job j[DRQ_WGRAD_REDUCE_MAX_JOBS]; int G[D
 // all weight-gradient partial reductions of the encoder backward in one launch: blockIdx.y = layer
 __global__ void __launch_bounds__(256) wgrad_reduce_multi_kernel(const WgReduceJobs jobs) {
     __shared__ float red[8][33], redb[8][33];
-    pdl_trigger();
-    pdl_wait();
     const drq_wgrad_reduce_job& jb = jobs.j[blockIdx.y];
     const int G = jobs.G[blockIdx.y];
     if (jb.cin > 0) {
@@ -135,7 +129,7 @@ int drq_pack_multi(const drq_pack_job* jobs, int njobs, void* stream) {
         }
     }
     pj.first_block[njobs] = blocks;
-    launch_k(pack_multi_kernel, blocks, 256, 0, as_stream(stream), pj);
+    pack_multi_kernel<<<blocks, 256, 0, as_stream(stream)>>>(pj);
     return check_launch("pack_multi_kernel");
 }
 
@@ -148,7 +142,7 @@ int drq_colsum_multi(const drq_colsum_job* jobs, int njobs, void* stream) {
         cj.j[i] = jobs[i];
         nmax = jobs[i].N > nmax ? jobs[i].N : nmax;
     }
-    launch_k(colsum_multi_kernel, dim3((nmax + 31) / 32, njobs), 256, 0, as_stream(stream), cj);
+    colsum_multi_kernel<<<dim3((nmax + 31) / 32, njobs), 256, 0, as_stream(stream)>>>(cj);
     return check_launch("colsum_multi_kernel");
 }
 
@@ -160,10 +154,9 @@ int drq_conv_wgrad_reduce_multi(const drq_wgrad_reduce_job* jobs, int njobs, voi
         DRQ_REQUIRE(jb.partial && jb.dw && jb.db && jb.n_images > 0 && jb.cin >= 0 && jb.cin * 9 + 1 <= 96 &&
                     (jb.cin > 0 || (jb.hout > 0 && jb.hout <= DRQ_PW - 2)), "wgrad_reduce_multi: bad job %d", i);
         wj.j[i] = jb;
-        // ctas > 0: the layer's weight-gradient kernel was launched under another SM limit than the current one
-        wj.G[i] = jb.ctas > 0 ? jb.ctas : (jb.cin > 0 ? conv1_wgrad_ctas(jb.n_images) : conv_wgrad_ctas(jb.n_images, jb.hout));
+        wj.G[i] = jb.cin > 0 ? conv1_wgrad_ctas(jb.n_images) : conv_wgrad_ctas(jb.n_images, jb.hout);
     }
-    launch_k(wgrad_reduce_multi_kernel, dim3(kWgReduceBlocks, njobs), 256, 0, as_stream(stream), wj);
+    wgrad_reduce_multi_kernel<<<dim3(kWgReduceBlocks, njobs), 256, 0, as_stream(stream)>>>(wj);
     return check_launch("wgrad_reduce_multi_kernel");
 }
 

@@ -64,8 +64,6 @@ __global__ void __launch_bounds__(256)
 adam_ema_kernel(float* p, const float* g, float* m, float* v, long long n_adam, const float* sc,
                 const float* ema_src, float* ema_dst, long long n_ema, float tau, float omt,
                 int adam_blocks) {
-    pdl_trigger();
-    pdl_wait();
     if ((int)blockIdx.x < adam_blocks) {
         adam_range(p, g, m, v, n_adam, sc, blockIdx.x * 256ll + threadIdx.x, adam_blocks * 256ll);
     } else {
@@ -84,9 +82,6 @@ constexpr int kOptTile = 2048;            // elements per block of the flat kind
 constexpr int kGenK = 4;                  // generic LINEAR / CONV1: scalar elements per thread
 constexpr int kGenTile = 256 * kGenK;
 constexpr int kTrunkW = 245;              // TRUNK: pixels per block (35*35 = 5 * 245), 8 channels x 245 pixels
-#ifndef OPT_MIN_BLOCKS
-#define OPT_MIN_BLOCKS 4     // measured on the B=256 update: 1815 vs 1808 updates/s with 3 (gpurun_out r2_b2_minb4 / _default)
-#endif
 
 struct OptArgs {
     drq_opt_seg s[DRQ_OPT_MAX_SEGS];
@@ -195,13 +190,9 @@ __device__ __forceinline__ void upd_scalar(const Upd& u, const int (&o)[K], cons
     }
 }
 
-// MINB = resident blocks per SM the register allocation aims for (3: 80 registers; 4: 64 registers, a few spilled
-// words on the generic LINEAR / CONV1 paths): more loads in flight per SM against fewer registers per thread
-static int g_opt_min_blocks = OPT_MIN_BLOCKS;
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB) adam_pack_kernel(const OptArgs a) {
-    pdl_trigger();
-    pdl_wait();
+// 4 resident blocks per SM (64 registers, a few spilled words on the generic LINEAR / CONV1 paths) rather than 3
+// (80 registers): more loads in flight per SM; measured on the B=256 update, 1815 vs 1808 updates/s
+__global__ void __launch_bounds__(256, 4) adam_pack_kernel(const OptArgs a) {
     __shared__ __align__(16) unsigned char smraw[kOptShBytes];
     int lo = 0, hi = a.n - 1;                    // last segment whose first block is <= blockIdx.x
     while (lo < hi) {
@@ -355,12 +346,6 @@ __global__ void __launch_bounds__(256, MINB) adam_pack_kernel(const OptArgs a) {
 
 static inline bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 
-// Optional L2 residency of the Adam moments (drq_set_l2_persist): the optimiser kernels are launched with a
-// persisting access-policy window over [base, base + bytes) so that m and v (8 of the 28 bytes per parameter
-// read, 8 written) stay in the L2 set-aside between updates instead of streaming from HBM.
-static const void* g_persist_base = nullptr;
-static size_t g_persist_bytes = 0;
-
 static int blocks_for(long long n) {
     long long b = (n / 4 + 255) / 256;
     if (b < 1) b = 1;
@@ -386,23 +371,8 @@ int drq_adam_ema_step(float* p, const float* g, float* m, float* v, int64_t n_ad
                 "adam_ema: ema arenas must be 16-byte aligned");
     const int ab = n_adam ? blocks_for(n_adam) : 0;
     const int eb = n_ema ? blocks_for(n_ema) : 0;
-    if (g_persist_bytes) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3(ab + eb); cfg.blockDim = dim3(256); cfg.stream = as_stream(stream);
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
-        attr[0].val.accessPolicyWindow.base_ptr = const_cast<void*>(g_persist_base);
-        attr[0].val.accessPolicyWindow.num_bytes = g_persist_bytes;
-        attr[0].val.accessPolicyWindow.hitRatio = 1.0f;
-        attr[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        cudaLaunchKernelEx(&cfg, adam_ema_kernel, p, (const float*)g, m, v, (long long)n_adam, scalars, ema_src, ema_dst,
-                           (long long)n_ema, tau, one_minus_tau, ab);
-    } else {
-        launch_k(adam_ema_kernel, ab + eb, 256, 0, as_stream(stream), p, g, m, v, n_adam, scalars, ema_src, ema_dst,
-                 n_ema, tau, one_minus_tau, ab);
-    }
+    adam_ema_kernel<<<ab + eb, 256, 0, as_stream(stream)>>>(p, g, m, v, n_adam, scalars, ema_src, ema_dst, n_ema, tau,
+                                                         one_minus_tau, ab);
     return check_launch("adam_ema_kernel");
 }
 
@@ -458,30 +428,8 @@ int drq_adam_pack_step(float* p, const float* g, float* m, float* v, const float
     }
     DRQ_REQUIRE(blocks < (1ll << 31), "adam_pack: too many blocks");
     a.first_block[nsegs] = (int)blocks;
-    if (g_opt_min_blocks >= 4) launch_k(adam_pack_kernel<4>, (unsigned)blocks, 256, 0, as_stream(stream), a);
-    else launch_k(adam_pack_kernel<3>, (unsigned)blocks, 256, 0, as_stream(stream), a);
+    adam_pack_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(a);
     return check_launch("adam_pack_kernel");
-}
-
-int drq_debug_opt_min_blocks(int min_blocks) { g_opt_min_blocks = min_blocks; return DRQ_OK; }
-
-int drq_set_l2_persist(const void* base, int64_t bytes) {
-    if (!base || bytes <= 0) { g_persist_base = nullptr; g_persist_bytes = 0; return DRQ_OK; }
-    int dev = 0, max_persist = 0, max_window = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-    cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-    size_t want = (size_t)bytes;
-    if (want > (size_t)max_persist) want = (size_t)max_persist;
-    if (want > (size_t)max_window) want = (size_t)max_window;
-    if (want == 0) { set_error("l2_persist: device has no persisting L2"); return DRQ_ERR_CUDA; }
-    if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("l2_persist: cudaDeviceSetLimit failed");
-        return DRQ_ERR_CUDA;
-    }
-    g_persist_base = base; g_persist_bytes = want;
-    return DRQ_OK;
 }
 
 int drq_adam_step(float* p, const float* g, float* m, float* v, int64_t n, const float* scalars,

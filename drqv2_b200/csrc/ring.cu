@@ -8,8 +8,6 @@
 namespace drq {
 
 static thread_local char g_err[512] = "";
-int g_pdl = 0;
-int g_pdl_once = 0;
 int g_sm_limit = 148;
 
 void set_error(const char* fmt, ...) {
@@ -72,8 +70,6 @@ ring_gather_kernel(const uint8_t* __restrict__ frames, const float* __restrict__
                    float gamma, uint8_t* __restrict__ obs_out, uint8_t* __restrict__ next_out,
                    float* __restrict__ action_out, float* __restrict__ reward_out,
                    float* __restrict__ discount_out) {
-    pdl_trigger();
-    pdl_wait();
     const int b = blockIdx.x;
     const int y = blockIdx.y;
     const long long start = ep_start[b];
@@ -127,8 +123,6 @@ __device__ __forceinline__ void ring_sample_elem(const int* __restrict__ ep_tabl
 __global__ void ring_sample_kernel(const int* __restrict__ ep_table, const int* __restrict__ n_episodes, int nstep,
                                    unsigned long long seed, const unsigned long long* counter,
                                    int* __restrict__ ep_start_out, int* __restrict__ idx_out, int B) {
-    pdl_trigger();
-    pdl_wait();
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     ring_sample_elem(ep_table, *n_episodes, nstep, seed, *counter, ep_start_out, idx_out, b);
@@ -138,8 +132,6 @@ __global__ void ring_sample_kernel(const int* __restrict__ ep_table, const int* 
 __global__ void __launch_bounds__(256) ring_sample_step_kernel(const int* __restrict__ ep_table, const int* __restrict__ n_episodes,
                                                                int nstep, unsigned long long seed, unsigned long long* counter,
                                                                int* __restrict__ ep_start_out, int* __restrict__ idx_out, int B) {
-    pdl_trigger();
-    pdl_wait();
     const unsigned long long c = *counter;
     const int E = *n_episodes;
     for (int b = threadIdx.x; b < B; b += blockDim.x) ring_sample_elem(ep_table, E, nstep, seed, c, ep_start_out, idx_out, b);
@@ -182,8 +174,6 @@ __global__ void rng_update_draws_kernel(unsigned long long seed, const unsigned 
                                         int pad, int* __restrict__ shift_obs,
                                         int* __restrict__ shift_next, float* __restrict__ eps_c,
                                         float* __restrict__ eps_a, int B, int A) {
-    pdl_trigger();
-    pdl_wait();
     update_draws_elem(seed, *counter, pad, shift_obs, shift_next, eps_c, eps_a, B, A, blockIdx.x * blockDim.x + threadIdx.x);
 }
 
@@ -193,8 +183,6 @@ __global__ void __launch_bounds__(1024) update_prologue_kernel(const float* scal
                                                                float* scal_out, unsigned long long seed, unsigned long long* counter,
                                                                int pad, int* __restrict__ shift_obs, int* __restrict__ shift_next,
                                                                float* __restrict__ eps_c, float* __restrict__ eps_a, int B, int A) {
-    pdl_trigger();
-    pdl_wait();
     if (threadIdx.x < DRQ_SCAL_SLOT) {
         const unsigned long long cur = *cursor;
         scal_out[threadIdx.x] = *reinterpret_cast<const volatile float*>(scal_ring + (cur % (unsigned long long)slots) * DRQ_SCAL_SLOT + threadIdx.x);
@@ -223,8 +211,6 @@ __global__ void __launch_bounds__(1024) update_prologue_ring_kernel(const float*
                                                                     const drq_ring_src src, float* __restrict__ action_out,
                                                                     float* __restrict__ reward_out, float* __restrict__ discount_out,
                                                                     int part) {
-    pdl_trigger();
-    pdl_wait();
     const bool head = part & 1, rest = part & 2;
     if (rest && threadIdx.x < DRQ_SCAL_SLOT) {
         const unsigned long long cur = *cursor;
@@ -274,8 +260,6 @@ __global__ void __launch_bounds__(1024) update_prologue_ring_kernel(const float*
 // out[i] ~ N(0,1): stream 5, Box-Muller on pair (i >> 1)
 __global__ void rng_normal_kernel(unsigned long long seed, const unsigned long long* counter,
                                   float* __restrict__ out, int n) {
-    pdl_trigger();
-    pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     uint32_t r[4];
@@ -288,16 +272,12 @@ __global__ void rng_normal_kernel(unsigned long long seed, const unsigned long l
     out[i] = (i & 1) ? rad * s : rad * co;
 }
 
-__global__ void counter_advance_kernel(unsigned long long* counter) {
-    pdl_trigger();
-    pdl_wait(); *counter += 1ull; }
+__global__ void counter_advance_kernel(unsigned long long* counter) { *counter += 1ull; }
 
 // out[0..DRQ_SCAL_SLOT) = ring[cursor % slots][..]; cursor += 1.  The ring is pinned host memory the host fills one
 // update ahead of the device: a CUDA graph cannot take new scalars per replay, and a fixed staging buffer
 // would be overwritten by a host that enqueues updates faster than the device runs them.
 __global__ void scalars_fetch_kernel(const float* ring, int slots, unsigned long long* cursor, float* out) {
-    pdl_trigger();
-    pdl_wait();
     const unsigned long long c = *cursor;
     const float v = *reinterpret_cast<const volatile float*>(ring + (c % (unsigned long long)slots) * DRQ_SCAL_SLOT + threadIdx.x);
     out[threadIdx.x] = v;
@@ -308,8 +288,6 @@ __global__ void scalars_fetch_kernel(const float* ring, int slots, unsigned long
 // out[n,c,r,col] = in[n,c,clamp(r+sy-pad),clamp(col+sx-pad)]
 __global__ void random_shift_f32_kernel(const float* __restrict__ in, const int* __restrict__ shift,
                                         float* __restrict__ out, int C, int H, int W, int pad) {
-    pdl_trigger();
-    pdl_wait();
     const int n = blockIdx.y;
     const int sx = shift[2 * n], sy = shift[2 * n + 1];
     const long long per = (long long)C * H * W;
@@ -325,8 +303,6 @@ __global__ void random_shift_f32_kernel(const float* __restrict__ in, const int*
 
 __global__ void copy2d_kernel(const float* __restrict__ src, long long ld_src, float* __restrict__ dst,
                               long long ld_dst, int rows, int cols) {
-    pdl_trigger();
-    pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rows * cols) return;
     const int r = i / cols, c = i - r * cols;
@@ -338,8 +314,6 @@ __global__ void copy2d_kernel(const float* __restrict__ src, long long ld_src, f
 using namespace drq;
 
 extern "C" {
-
-int drq_set_pdl(int on) { g_pdl = on == 2 ? 2 : (on ? 1 : 0); return DRQ_OK; }
 
 int drq_set_sm_limit(int sms) {
     DRQ_REQUIRE(sms >= 1 && sms <= 148, "set_sm_limit: 1..148");
@@ -376,7 +350,7 @@ int drq_ring_gather_nstep(const uint8_t* frames, const float* action, const floa
                     ((uintptr_t)obs_out % 16) == 0 && ((uintptr_t)next_obs_out % 16) == 0,
                 "ring_gather: frames must be 16-byte aligned");
     dim3 grid(B, 2 * stack + 1);
-    launch_k(ring_gather_kernel, grid, 256, 0, as_stream(stream), 
+    ring_gather_kernel<<<grid, 256, 0, as_stream(stream)>>>(
         frames, action, reward, discount, (long long)capacity, frame_bytes, stack, A, ep_start, idx,
         nstep, gamma, obs_out, next_obs_out, action_out, reward_out, discount_out);
     return check_launch("ring_gather_kernel");
@@ -386,7 +360,7 @@ int drq_ring_sample(const int32_t* ep_table, const int32_t* n_episodes, int nste
                     const uint64_t* counter, int32_t* ep_start_out, int32_t* idx_out, int B, void* stream) {
     DRQ_REQUIRE(ep_table && n_episodes && counter && ep_start_out && idx_out, "ring_sample: null pointer");
     DRQ_REQUIRE(nstep > 0 && B > 0, "ring_sample: bad dims");
-    launch_k(ring_sample_kernel, (B + 127) / 128, 128, 0, as_stream(stream), 
+    ring_sample_kernel<<<(B + 127) / 128, 128, 0, as_stream(stream)>>>(
         ep_table, n_episodes, nstep, (unsigned long long)seed, (const unsigned long long*)counter,
         ep_start_out, idx_out, B);
     return check_launch("ring_sample_kernel");
@@ -398,7 +372,7 @@ int drq_rng_update_draws(uint64_t seed, const uint64_t* counter, int pad, int32_
     DRQ_REQUIRE(counter && shift_obs && shift_next && eps_critic && eps_actor, "rng: null pointer");
     DRQ_REQUIRE(B > 0 && A > 0 && pad >= 0, "rng: bad dims");
     const int n = B * A > B ? B * A : B;
-    launch_k(rng_update_draws_kernel, (n + 127) / 128, 128, 0, as_stream(stream), 
+    rng_update_draws_kernel<<<(n + 127) / 128, 128, 0, as_stream(stream)>>>(
         (unsigned long long)seed, (const unsigned long long*)counter, pad, shift_obs, shift_next,
         eps_critic, eps_actor, B, A);
     return check_launch("rng_update_draws_kernel");
@@ -407,20 +381,20 @@ int drq_rng_update_draws(uint64_t seed, const uint64_t* counter, int pad, int32_
 int drq_copy2d_f32(const float* src, int64_t ld_src, float* dst, int64_t ld_dst, int rows, int cols,
                    void* stream) {
     DRQ_REQUIRE(src && dst && rows > 0 && cols > 0, "copy2d: bad args");
-    launch_k(copy2d_kernel, (rows * cols + 255) / 256, 256, 0, as_stream(stream), src, ld_src, dst, ld_dst, rows, cols);
+    copy2d_kernel<<<(rows * cols + 255) / 256, 256, 0, as_stream(stream)>>>(src, ld_src, dst, ld_dst, rows, cols);
     return check_launch("copy2d_kernel");
 }
 
 int drq_rng_normal_f32(uint64_t seed, const uint64_t* counter, float* out, int n, void* stream) {
     DRQ_REQUIRE(counter && out && n > 0, "rng_normal: bad args");
-    launch_k(rng_normal_kernel, (n + 127) / 128, 128, 0, as_stream(stream), 
+    rng_normal_kernel<<<(n + 127) / 128, 128, 0, as_stream(stream)>>>(
         (unsigned long long)seed, (const unsigned long long*)counter, out, n);
     return check_launch("rng_normal_kernel");
 }
 
 int drq_counter_advance(uint64_t* counter, void* stream) {
     DRQ_REQUIRE(counter, "counter_advance: null pointer");
-    launch_k(counter_advance_kernel, 1, 1, 0, as_stream(stream), (unsigned long long*)counter);
+    counter_advance_kernel<<<1, 1, 0, as_stream(stream)>>>((unsigned long long*)counter);
     return check_launch("counter_advance_kernel");
 }
 
@@ -428,7 +402,7 @@ int drq_ring_sample_step(const int32_t* ep_table, const int32_t* n_episodes, int
                          int32_t* ep_start_out, int32_t* idx_out, int B, void* stream) {
     DRQ_REQUIRE(ep_table && n_episodes && counter && ep_start_out && idx_out, "ring_sample_step: null pointer");
     DRQ_REQUIRE(B > 0 && nstep > 0, "ring_sample_step: bad dims");
-    launch_k(ring_sample_step_kernel, 1, 256, 0, as_stream(stream), ep_table, n_episodes, nstep, (unsigned long long)seed,
+    ring_sample_step_kernel<<<1, 256, 0, as_stream(stream)>>>(ep_table, n_episodes, nstep, (unsigned long long)seed,
              (unsigned long long*)counter, ep_start_out, idx_out, B);
     return check_launch("ring_sample_step_kernel");
 }
@@ -439,7 +413,7 @@ int drq_update_prologue(const float* scal_ring, int slots, uint64_t* cursor, flo
     DRQ_REQUIRE(scal_ring && cursor && scal_out && slots > 0, "update_prologue: bad scalar ring");
     const bool draws = shift_obs != nullptr;
     DRQ_REQUIRE(!draws || (counter && shift_next && eps_critic && eps_actor && B > 0 && A > 0 && pad >= 0), "update_prologue: bad draw arguments");
-    launch_k(update_prologue_kernel, 1, 1024, 0, as_stream(stream), scal_ring, slots, (unsigned long long*)cursor, scal_out,
+    update_prologue_kernel<<<1, 1024, 0, as_stream(stream)>>>(scal_ring, slots, (unsigned long long*)cursor, scal_out,
              (unsigned long long)seed, (unsigned long long*)counter, pad, shift_obs, shift_next, eps_critic, eps_actor, B, A);
     return check_launch("update_prologue_kernel");
 }
@@ -455,7 +429,7 @@ int drq_update_prologue_ring_part(const float* scal_ring, int slots, uint64_t* c
                     src->ep_start && src->idx, "update_prologue_ring: incomplete ring source");
     DRQ_REQUIRE(B > 0 && A > 0 && A == src->A && src->capacity > 0 && src->nstep > 0, "update_prologue_ring: bad dims");
     DRQ_REQUIRE(action_out && reward_out && discount_out, "update_prologue_ring: null output");
-    launch_k(update_prologue_ring_kernel, 1, 1024, 0, as_stream(stream), scal_ring, slots, (unsigned long long*)cursor, scal_out,
+    update_prologue_ring_kernel<<<1, 1024, 0, as_stream(stream)>>>(scal_ring, slots, (unsigned long long*)cursor, scal_out,
              (unsigned long long)seed, (unsigned long long*)counter, pad, shift_obs, shift_next, eps_critic, eps_actor, B, A,
              *src, action_out, reward_out, discount_out, part);
     return check_launch("update_prologue_ring_kernel");
@@ -471,7 +445,7 @@ int drq_update_prologue_ring(const float* scal_ring, int slots, uint64_t* cursor
 
 int drq_scalars_fetch(const float* ring, int slots, uint64_t* cursor, float* out, void* stream) {
     DRQ_REQUIRE(ring && cursor && out && slots > 0, "scalars_fetch: bad arguments");
-    launch_k(scalars_fetch_kernel, 1, DRQ_SCAL_SLOT, 0, as_stream(stream), ring, slots, (unsigned long long*)cursor, out);
+    scalars_fetch_kernel<<<1, DRQ_SCAL_SLOT, 0, as_stream(stream)>>>(ring, slots, (unsigned long long*)cursor, out);
     return check_launch("scalars_fetch_kernel");
 }
 
@@ -484,7 +458,7 @@ int drq_random_shift_f32(const float* in, const int32_t* shift, float* out, int 
     const long long per = (long long)C * H * W;
     int gx = (int)((per + 255) / 256);
     if (gx > 64) gx = 64;
-    launch_k(random_shift_f32_kernel, dim3(gx, N), 256, 0, as_stream(stream), in, shift, out, C, H, W, pad);
+    random_shift_f32_kernel<<<dim3(gx, N), 256, 0, as_stream(stream)>>>(in, shift, out, C, H, W, pad);
     return check_launch("random_shift_f32_kernel");
 }
 

@@ -223,8 +223,7 @@ class Actor(nn.Module):
         mu_pre = torch.empty(B, A, device=dev)
         keep = _mlp_fwd(self.policy, h.data_ptr(), Fd, B, Fd, H, A, mu_pre.data_ptr(), dev)
         mu = torch.empty(B, A, device=dev)
-        call("drq_actor_sample", mu_pre.data_ptr(), None, None, 0.0, mu.data_ptr(), A, None, None, None, 0, 0, B, A,
-             _stream())
+        call("drq_actor_sample", mu_pre.data_ptr(), None, None, 0.0, mu.data_ptr(), A, None, None, B, A, _stream())
         del keep
         return utils.TruncatedNormal(mu, torch.ones_like(mu) * std)
 
@@ -301,7 +300,7 @@ class _Arena:
         # actor's gradients (the last segment), see DrQV2Agent._sync_grads
         self._grads_full = torch.zeros(off + 8, device=device)
         self.grads, self.metrics_tail = self._grads_full[:off], self._grads_full[off:]
-        self.moments = torch.zeros(2, off, device=device)        # [exp_avg | exp_avg_sq], one range (L2 persistence)
+        self.moments = torch.zeros(2, off, device=device)        # [exp_avg | exp_avg_sq]
         self.exp_avg, self.exp_avg_sq = self.moments[0], self.moments[1]
         n_t = self.seg["critic"][2]
         self.target = torch.zeros(n_t, device=device)
@@ -441,8 +440,6 @@ class DrQV2Agent:
         # bf16 mode fed from the HBM ring: conv1 reads the frame stacks from the ring by index (DRQV2_B200_RING_DIRECT=0:
         # gather them into a batch buffer first)
         self.ring_direct = os.environ.get("DRQV2_B200_RING_DIRECT", "1") != "0"
-        # Linear(hidden, A) + the TruncatedNormal samples in one CUDA-core launch (0: tensor-core tile + sampling launches)
-        self.fused_policy_head = os.environ.get("DRQV2_B200_POLICY_HEAD", "1") != "0"
         # the actor pass' GEMMs in their 66 KB variant, co-resident with the encoder backward's conv CTAs.  A loss without
         # stream priorities (1769 vs 1834 updates/s: GEMM CTAs that share the encoder backward's SMs cost it more than their
         # own waiting costs), a gain with them (1940 -> 2000: the chain's CTAs are placed first and no longer queue behind a
@@ -451,15 +448,8 @@ class DrQV2Agent:
         self._side_stream = None
         self._side_stream2 = None
         self._main_stream = None
-        self._aux = None
-        self._ema = None
-        self._ema_own_stream = os.environ.get("DRQV2_B200_EMA_STREAM", "0") != "0"
-        self._critic_rest = None
         # schedule switches of the captured tensor-core update (DESIGN.md section 4); every one leaves the results bit-identical
         self.early_encoder_backward = os.environ.get("DRQV2_B200_EARLY_ENC", "1") != "0"
-        self.split_critic_step = os.environ.get("DRQV2_B200_SPLIT_CRITIC_STEP", "0") != "0"
-        self.split_actor_step = os.environ.get("DRQV2_B200_SPLIT_ACTOR_STEP", "0") != "0"
-        self.conv1_wgrad_sms = int(os.environ.get("DRQV2_B200_CONV1_WG_SMS", "0"))
         self.split_prologue = os.environ.get("DRQV2_B200_SPLIT_PROLOGUE", "1") != "0"
         self.encoder_backward_sms = int(os.environ.get("DRQV2_B200_ENC_BWD_SMS", "140"))
         # priorities of (main, encoder-backward, weight-gradient) streams inside the captured update; 0 = default (lowest)
@@ -524,9 +514,6 @@ class DrQV2Agent:
         self._bf16_ws = {}
         self._bf16_dirty = True
         self._prefetch, self._stage = None, {}
-        if os.environ.get("DRQV2_B200_L2_PERSIST", "0") == "1":
-            m = self._arena.moments
-            _lib.call("drq_set_l2_persist", m.data_ptr(), m.numel() * F32)
 
     def __getstate__(self):
         st = dict(self.__dict__)
@@ -538,8 +525,6 @@ class DrQV2Agent:
         st["_side_stream"] = None
         st["_side_stream2"] = None
         st["_main_stream"] = None
-        st["_aux"] = None
-        st["_ema"] = None
         return st
 
     def __setstate__(self, st):
@@ -749,7 +734,7 @@ class DrQV2Agent:
         _linear_fwd(w["p1"].data_ptr(), H, pa("policy.2.weight"), pa("policy.2.bias"), w["p2"].data_ptr(), H, n, H, H, True)
         _linear_fwd(w["p2"].data_ptr(), H, pa("policy.4.weight"), pa("policy.4.bias"), w["mu_pre"].data_ptr(), A, n, A, H, False)
         call("drq_actor_sample", w["mu_pre"].data_ptr(), w["eps"].data_ptr() if sample else None,
-             self._sc("stddev"), 0.0, w["out"].data_ptr(), A, None, None, None, 0, 0, n, A, _stream())
+             self._sc("stddev"), 0.0, w["out"].data_ptr(), A, None, None, n, A, _stream())
 
     # ------------------------------------------------------------------ update
     def update(self, replay_iter, step):
@@ -963,20 +948,6 @@ class DrQV2Agent:
             self._side_stream2 = torch.cuda.Stream(device=self._dev, priority=self._prio[2])
         return self._side_stream2
 
-    def _aux_stream(self):
-        """Fourth stream, at the main chain's priority (the split optimiser steps: DRQV2_B200_SPLIT_*_STEP)."""
-        if self._aux is None:
-            self._aux = torch.cuda.Stream(device=self._dev, priority=self._prio[0])
-        return self._aux
-
-    def _ema_stream(self):
-        """Stream of the soft target update inside the captured update (None: the weight-gradient stream)."""
-        if not self._ema_own_stream:
-            return None
-        if self._ema is None:
-            self._ema = torch.cuda.Stream(device=self._dev, priority=0)
-        return self._ema
-
     def _capture_stream(self):
         """Stream the update graph is captured on (None: torch's own capture stream).  Kernel nodes keep the priority of
         the stream they were captured on, so the three streams of the schedule can be ranked: when CTAs of two ready
@@ -1075,7 +1046,7 @@ class DrQV2Agent:
         _linear_fwd(ws.p1.data_ptr(), H, pa("policy.2.weight"), pa("policy.2.bias"), ws.p2.data_ptr(), H, B, H, H, True)
         _linear_fwd(ws.p2.data_ptr(), H, pa("policy.4.weight"), pa("policy.4.bias"), ws.mu_pre.data_ptr(), A, B, A, H, False)
         call("drq_actor_sample", ws.mu_pre.data_ptr(), ws.eps_c.data_ptr(), std_ptr, float(self.stddev_clip),
-             ws.xT.data_ptr() + F32 * Fd, Fd + A, None, None, None, 0, 0, B, A, s)
+             ws.xT.data_ptr() + F32 * Fd, Fd + A, None, None, B, A, s)
         # --- target critic on (next features, next action) (drqv2.py:184)
         _trunk_fwd(featn, B, self._t("trunk.0.weight"), self._t("trunk.0.bias"), self._t("trunk.1.weight"),
                    self._t("trunk.1.bias"), Fd, ws.partial.data_ptr(), ws.xT.data_ptr(), Fd + A)
@@ -1167,7 +1138,7 @@ class DrQV2Agent:
         _linear_fwd(ws.p1.data_ptr(), H, pa("policy.2.weight"), pa("policy.2.bias"), ws.p2.data_ptr(), H, B, H, H, True)
         _linear_fwd(ws.p2.data_ptr(), H, pa("policy.4.weight"), pa("policy.4.bias"), ws.mu_pre.data_ptr(), A, B, A, H, False)
         call("drq_actor_sample", ws.mu_pre.data_ptr(), ws.eps_a.data_ptr(), std_ptr, float(self.stddev_clip),
-             ws.xA.data_ptr() + F32 * Fd, Fd + A, ws.mu.data_ptr(), ws.metrics.data_ptr() + F32 * 6, None, 0, 0, B, A, s)
+             ws.xA.data_ptr() + F32 * Fd, Fd + A, ws.mu.data_ptr(), ws.metrics.data_ptr() + F32 * 6, B, A, s)
         # the just-updated critic on (features, action) (drqv2.py:213-216)
         _trunk_fwd(featp, B, pc("trunk.0.weight"), pc("trunk.0.bias"), pc("trunk.1.weight"), pc("trunk.1.bias"),
                    Fd, ws.partial.data_ptr(), ws.xA.data_ptr(), Fd + A)

@@ -42,7 +42,7 @@ extern "C" {
 #endif
 
 #define DRQ_SCAL_SLOT 32   /* floats per slot of the per-update host scalar ring (drq_scalars_fetch) */
-#define DRQ_ABI_VERSION 1
+#define DRQ_ABI_VERSION 2
 
 #define DRQ_OK 0
 #define DRQ_ERR_INVALID 1 /* bad argument */
@@ -70,11 +70,6 @@ int drq_abi_version(void);
 const char* drq_last_error(void);
 /* number of SMs of the current device (0 if none) — used to size persistent grids */
 int drq_device_sm_count(void);
-/* programmatic dependent launch: 0 (default) off; 1 every kernel of the library - the next kernel's launch latency and
- * CTA-local set-up overlap the running kernel's tail, each kernel waits for its predecessors (griddepcontrol.wait) before
- * touching global memory; 2 only the conv3x3 forward launches of the four-pixel-column kernel (the encoder's forward
- * chain: barrier / TMEM set-up and the weight expansion of layer k+1 run on the SMs that have finished layer k). */
-int drq_set_pdl(int on);
 /* SMs the persistent kernels (convs, GEMMs) size their grids for: 148 (default) or fewer.  A data-parallel update
  * leaves a few SMs to the NCCL all-reduce that runs beside the encoder backward - a persistent kernel keeps every SM it
  * got until it ends, so a collective that finds none free would either wait for it or make its late CTAs run their
@@ -341,9 +336,6 @@ int drq_debug_conv_stamps(int64_t* buf);
  * mbarrier wait that gives up writes {1 = plain / 2 = sleeping wait, block size, thread, barrier shared-memory address,
  * parity, block} there before it traps - tells which role of which kernel stopped making progress */
 int drq_debug_trap_note(uint32_t* mapped_host_words);
-/* self-test of the above: launches one thread that waits on a barrier nobody arrives on; the context dies with a launch
- * failure after the wait's bound (how long that takes is the bound of every wait in the library) */
-int drq_debug_force_timeout(void* stream);
 /* 12 clock64 totals of block 0 of the four-pixel-column conv kernels (device buffer, or null = off): producer {wait
  * stage, -, -, total}, UMMA warp {wait accumulator, wait stage, issue, total}, first epilogue warp {wait accumulator,
  * TMEM load, math + stores, total} */
@@ -385,7 +377,7 @@ int drq_colsum_multi(const drq_colsum_job* jobs, int njobs, void* stream);
  * drq_conv1_wgrad_bf16 called with dw == db == NULL leave their per-CTA partials in `partial`; this call
  * reduces them (fixed order) into dw / db.  cin > 0: a conv1 job (N images); cin == 0: a conv3x3 job (N, hout). */
 #define DRQ_WGRAD_REDUCE_MAX_JOBS 4
-typedef struct { const float* partial; float* dw; float* db; int32_t n_images; int32_t hout; int32_t cin; int32_t ctas; } drq_wgrad_reduce_job;
+typedef struct { const float* partial; float* dw; float* db; int32_t n_images; int32_t hout; int32_t cin; int32_t reserved; } drq_wgrad_reduce_job;
 int drq_conv_wgrad_reduce_multi(const drq_wgrad_reduce_job* jobs, int njobs, void* stream);
 
 /* ------------------------------------------------------------------ dense, fp32 */
@@ -452,8 +444,7 @@ int drq_ln_tanh_bwd(const float* dh, int64_t ld_dh, const float* h, int64_t ld_h
  * metrics (nullable) [2]: mean_b sum_j log_prob, mean_b sum_j entropy
  * (drqv2.py:212,226). */
 int drq_actor_sample(const float* mu_pre, const float* eps, const float* std_dev, float clip,
-                     float* action_out, int64_t ld_a, float* mu_out, float* metrics,
-                     uint16_t* action_bf16, int64_t rpad_ab, int feat_off, int B, int A, void* stream);
+                     float* action_out, int64_t ld_a, float* mu_out, float* metrics, int B, int A, void* stream);
 
 /* Policy head of the tensor-core mode in one launch (drqv2.py:81,88-92 + utils.py:112-126): mu_pre[m][a] =
  * p2[m][:] . bf16(w4[a][:]) + b4[a] for the M rows of the TB activation p2 (units per row), and - by the thread that
@@ -513,14 +504,6 @@ int drq_q_head_bwd_loss_bf16(int loss, const float* q, const float* tq, const fl
  * float64 exactly as torch/optim/adam.py:531-547 and cast to fp32.
  * One launch updates the contiguous range p[0..n): torch.optim.Adam x3 of
  * drqv2.py:148-150,201-202,221 over the flat parameter arena. */
-/* tuning switch: register allocation target of the fused optimiser kernel (3 or 4 resident blocks per SM) */
-int drq_debug_opt_min_blocks(int min_blocks);
-
-/* Optional: keep [base, base+bytes) (the Adam moment arenas) in the persisting L2 set-aside - the optimiser
- * kernels are then launched with a persisting access-policy window over it (clamped to the device limits).
- * base == NULL switches it off. */
-int drq_set_l2_persist(const void* base, int64_t bytes);
-
 int drq_adam_step(float* p, const float* g, float* m, float* v, int64_t n, const float* scalars,
                   void* stream);
 

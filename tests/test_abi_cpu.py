@@ -27,7 +27,7 @@ def test_library_exports_every_header_symbol():
         assert hasattr(h, s), f"{s} declared in include/drqv2_b200.h but not exported"
     # and the ctypes table binds exactly the declared set
     assert sorted(_lib.exported_symbols()) == syms
-    assert _lib.lib().drq_abi_version() == 1
+    assert _lib.lib().drq_abi_version() == 2
 
 
 def test_no_cuda_fails_loudly():

@@ -13,13 +13,12 @@ pytestmark = pytest.mark.gpu
 SCHED = "linear(1.0,0.1,100000)"
 
 PLAIN = {"DRQV2_B200_PRIO": "0,0,0", "DRQV2_B200_EARLY_ENC": "0", "DRQV2_B200_SPLIT_PROLOGUE": "0", "DRQV2_B200_SMALL_GEMMS": "0"}
-SPLIT_STEPS = {"DRQV2_B200_SPLIT_CRITIC_STEP": "1", "DRQV2_B200_SPLIT_ACTOR_STEP": "1", "DRQV2_B200_EMA_STREAM": "1"}
 
 
 def _run(monkeypatch, env, tag, overlap=True, steps=4):
     from drqv2_b200 import DrQV2Agent, make_replay_loader
     from drqv2_b200 import replay_buffer as R
-    for k in list(PLAIN) + list(SPLIT_STEPS):
+    for k in PLAIN:
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
@@ -55,11 +54,10 @@ def test_schedule_switches_are_bit_identical(monkeypatch):
         pytest.skip("no CUDA device")
     base_m, base = _run(monkeypatch, {}, "default")                       # priorities, early fork, split prologue, small GEMMs
     assert all(np.isfinite(m["critic_loss"]) for m in base_m)
-    for tag, env in (("plain", PLAIN), ("splitsteps", SPLIT_STEPS)):
-        ms, st = _run(monkeypatch, env, tag)
-        assert ms == base_m, tag
-        for k in base:
-            assert torch.equal(base[k], st[k]), (tag, k)
+    ms, st = _run(monkeypatch, PLAIN, "plain")
+    assert ms == base_m
+    for k in base:
+        assert torch.equal(base[k], st[k]), k
 
 
 def test_one_stream_equals_three_streams_up_to_the_wgrad_grid(monkeypatch):

@@ -14,7 +14,7 @@ STRUCTS = {   # header struct -> (ctypes mirror, fields)
     "drq_pack_job": ("PackJob", ["kind", "rows", "cols", "reserved", "w", "bias", "out", "out2"]),
     "drq_colsum_job": ("ColsumJob", ["X", "ld", "out", "M", "N", "tb", "reserved", "Y"]),
     "drq_opt_seg": ("OptSeg", ["kind", "ema", "rows", "cols", "off", "n", "out", "out2"]),
-    "drq_wgrad_reduce_job": ("WgReduceJob", ["partial", "dw", "db", "n_images", "hout", "cin", "ctas"]),
+    "drq_wgrad_reduce_job": ("WgReduceJob", ["partial", "dw", "db", "n_images", "hout", "cin", "reserved"]),
     "drq_ln_job": ("LnJob", ["partial", "ld_partial", "split_stride", "S", "bias", "gamma", "beta", "h_out", "ld_h", "xhat",
                              "rstd", "h_bf16", "units_bf16", "row0_bf16", "tail", "ld_tail", "n_tail"]),
     "drq_policy_sample": ("PolicySample", ["row0", "rows", "eps", "action_out", "ld_a", "mu_out", "metrics", "a_bf16",

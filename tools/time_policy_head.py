@@ -39,8 +39,8 @@ def fused(nj):
 
 def unfused():
     gemm(p2.ptr(), p2.units, w4b.ptr(), w4b.units, GEMM_KK, mu_pre.data_ptr(), A, M, A, H, TEPI_F32, bias=b4.data_ptr())
-    _lib.call("drq_actor_sample", mu_pre.data_ptr() + 4 * 256 * A, eps.data_ptr(), std.data_ptr(), 0.3, out1.data_ptr(), A, None, None, None, 0, 0, B, A, cur())
-    _lib.call("drq_actor_sample", mu_pre.data_ptr(), eps.data_ptr(), std.data_ptr(), 0.3, out2.data_ptr(), A, mu.data_ptr(), metrics.data_ptr(), None, 0, 0, B, A, cur())
+    _lib.call("drq_actor_sample", mu_pre.data_ptr() + 4 * 256 * A, eps.data_ptr(), std.data_ptr(), 0.3, out1.data_ptr(), A, None, None, B, A, cur())
+    _lib.call("drq_actor_sample", mu_pre.data_ptr(), eps.data_ptr(), std.data_ptr(), 0.3, out2.data_ptr(), A, mu.data_ptr(), metrics.data_ptr(), B, A, cur())
 
 
 def timeit(fn, n=200):
