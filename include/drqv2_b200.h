@@ -249,7 +249,11 @@ int drq_pack_conv_w_bf16(const float* w, uint16_t* w_fwd, uint16_t* w_dgrad, voi
  * feature matrix [N][hout*hout][32]; nhwc_out == 2: out is the TB feature matrix the tensor-core
  * trunk consumes (feature (c/8)*hout*hout*8 + (y*hout+x)*8 + c%8, feat_rpad = units per row = hout*hout*4); image n is row n
  * for n < feat_half and row n - feat_half + feat_half_row after it (the next_obs half of an update starts
- * on its own 128-row block); feat_half <= 0: row = image. */
+ * on its own 128-row block); feat_half <= 0: row = image.  What is written: WB out = rows < hout of images < N - the
+ * four-pixel-column kernel stores columns < hout only, the one-pixel kernel whole 41-pixel rows (columns hout..40 then
+ * hold values no later kernel reads); NHWC = images < N; TB = the rows of images < N.  Nothing else (guard rows, slack,
+ * TB rows of no image) is touched.  The data gradient writes rows < hout + 2 of images < N, all 41 columns, with exact
+ * zeros past column hout + 1. */
 int drq_conv3x3_fwd_bf16(const uint16_t* in, const uint16_t* w_fwd, const float* bias, uint16_t* out,
                          int N, int hout, int nhwc_out, int64_t feat_rpad, int feat_half, int feat_half_row,
                          void* stream);
