@@ -462,6 +462,10 @@ int drq_gemm_bf16(const uint16_t* A, int units_a, const uint16_t* B, int units_b
     DRQ_REQUIRE(!((epilogue == DRQ_TEPI_MASK_BF16 || epilogue == DRQ_TEPI_TRUNK_DGRAD) && !mask), "gemm_bf16: mask missing");
     DRQ_REQUIRE(!(epilogue == DRQ_TEPI_RELU_BF16 && !bias), "gemm_bf16: bias missing");
     DRQ_REQUIRE(!(splitk > 1 && (epilogue != DRQ_TEPI_F32 || mode == MODE_MNMN)), "gemm_bf16: split-K writes fp32 partials (modes KK, KMN)");
+    // the zero columns [N, n_store) of a TB output are written by the tiles of N: a column past the last one would be left
+    // unwritten (a caller's stale values read as features), so such an n_store is refused
+    DRQ_REQUIRE(!((epilogue == DRQ_TEPI_RELU_BF16 || epilogue == DRQ_TEPI_MASK_BF16) && n_store > (N + bn - 1) / bn * bn),
+                "gemm_bf16: n_store %d lies past the last %d-wide N tile (N = %d)", n_store, bn, N);
     DRQ_REQUIRE(!(mode == MODE_KK && bn == 128 && ((N + RW - 1) / RW) % 2 != 0),
                 "gemm_bf16: K-major bn = 128 reads pairs of 64-row weight blocks (N = %d)", N);
     // the blocked extents must cover what the tiles touch

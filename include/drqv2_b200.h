@@ -320,11 +320,20 @@ int64_t drq_conv1_wgrad_bf16_ws_floats(void);
 
 /* C[M,N] = sum_k A(m,k) B(n,k) on tcgen05 tensor cores, bf16 TB operands, fp32 accumulate (TMEM).
  * units_a / units_b: units per row of the operand buffers.  TB outputs write feature columns
- * [0, max(N, n_store)) with zeros beyond N.  batch > 1: grid z = zo * batch_inner + zi, operand z at
+ * [0, max(N, n_store)) with zeros beyond N; n_store may not lie past the last N tile (ceil(N / bn) * bn).  batch > 1: grid z = zo * batch_inner + zi, operand z at
  * offset zi * strides[0..4] + zo * strides[5..9] (elements; a, b, c, bias, mask; strides == NULL: 0;
  * strides has 11 entries).  splitk > 1 (DRQ_GEMM_KK, fp32): plane s of C (stride strides[10]) receives
  * the partial sum of K chunk s (bias is not applied); grid z = batch entry * splitk + s.
- * bn = N tile: 64 (all modes) or 128 (KMN, MNMN). */
+ * bn = N tile: 64 (all modes) or 128 (KMN, MNMN).
+ * What a launch reads:  a K-major operand (contraction over its features: A of KK / KMN, B of KK) is read up to
+ * ceil(K/16)*16 features of each chunk; an MN-major operand (contraction over its rows: B of KMN, A and B of MNMN) is
+ * read as whole row blocks (128 rows, weights 64), of which only the first ceil(K/16)*16 rows enter the UMMAs.  Rows
+ * of a K-major operand past M (N), and features of an MN-major operand past M (N), reach only outputs that are not
+ * stored: they may hold anything.  Padding INSIDE the read extent must be zero: features [K, ceil(K/16)*16) of K-major
+ * operands and rows [K, ceil(K/16)*16) of MN-major ones (the rows [B, ceil(B/16)*16) of every activation or gradient
+ * contracted over the batch).  The library keeps that: its TB buffers start zeroed and every producer of one (these
+ * epilogues, drq_ln_tanh_fwd*, drq_ln_tanh_bwd, drq_actor_sample_bwd, drq_policy_head_fwd_bf16, the conv4 feature
+ * epilogue) writes rows < B only.  (tests/test_gpu_gemm_edges.py fills everything past the extent with NaN.) */
 int drq_gemm_bf16(const uint16_t* A, int units_a, const uint16_t* B, int units_b, int mode, void* C, int64_t ldc,
                   int n_store, const float* bias, const uint16_t* mask, int units_mask, int M, int N, int K,
                   int epilogue, int accumulate, int batch, int batch_inner, const int64_t* strides, int splitk,

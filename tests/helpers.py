@@ -73,20 +73,28 @@ def nchw_from_wb(wb, N, H, W):
 # A bf16 NaN that no kernel computes: every output buffer is filled with it before a call, and every element the call
 # must not write has to hold it afterwards, bit for bit.
 SENTINEL_BITS = 0x7FA5
+F32_SENTINEL_BITS = 0x7FA5A5A5      # the same for fp32 outputs
+
+
+def _sentinel_view(buf):
+    import torch
+    if buf.dtype == torch.float32:
+        return buf.view(torch.int32), F32_SENTINEL_BITS
+    return buf.view(torch.int16), SENTINEL_BITS
 
 
 def fill_sentinel(buf):
-    import torch
-    buf.view(torch.int16).fill_(SENTINEL_BITS)
+    """bf16 or fp32 buffer -> every element the sentinel NaN of its type"""
+    bits, s = _sentinel_view(buf)
+    bits.fill_(s)
     return buf
 
 
 def assert_sentinel_outside(buf, written, what):
-    """every element of `buf` (bf16, any shape) where the bool tensor `written` (same number of elements) is False
+    """every element of `buf` (bf16 or fp32, any shape) where the bool tensor `written` (same number of elements) is False
     still holds the sentinel"""
-    import torch
-    bits = buf.reshape(-1).view(torch.int16)
-    stray = (bits != SENTINEL_BITS) & ~written.reshape(-1)
+    bits, s = _sentinel_view(buf.reshape(-1))
+    stray = (bits != s) & ~written.reshape(-1)
     n = int(stray.sum())
     assert n == 0, f"{what}: {n} elements outside the written set were overwritten, first at flat index " \
                    f"{int(stray.nonzero()[0])}"
@@ -116,6 +124,26 @@ def assert_conv_bound(got, want, absref, what, rel=2.0 ** -8, absc=2.0 ** -14):
     rounding = 2.0 ** -8 / (1 + 2.0 ** -8) * want.abs()
     rest = torch.where(live, (err - rounding).clamp_min(0) / (absc * absref).clamp_min(1e-300), torch.zeros_like(err))
     return float(ratio.max()), float(rest.max())
+
+
+def assert_f32_bound(got, want, absref, chain, c, what):
+    """|got - want| <= c * 2^-24 * chain * A element-wise, for fp32 outputs of the tensor-core GEMM.  chain is the UMMA
+    accumulation chain of the element's tile, ceil(K_chunk / 16) (scalar or broadcastable), A the same GEMM on absolute
+    values plus |bias|.  The bf16 products are exact in fp32, so the error is the fp32 accumulation alone.  Returns the
+    largest |got - want| / (2^-24 * chain * A): the c this output needed."""
+    import torch
+    got, want, absref = got.double(), want.double(), absref.double()
+    unit = 2.0 ** -24 * chain * absref
+    err = (got - want).abs()
+    bad = ~(err <= c * unit)                    # a NaN (an unwritten sentinel) fails too
+    if bad.any():
+        i = tuple(int(v) for v in bad.nonzero()[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} elements outside |got - want| <= {c:g} 2^-24 chain A, first at "
+                             f"{i}: got {float(got[i])!r}, want {float(want[i])!r}, A {float(absref[i])!r}")
+    if not err.numel():
+        return 0.0
+    need = torch.where(unit > 0, err / unit.clamp_min(1e-300), torch.zeros_like(err))
+    return float(need.max())
 
 
 def max_norm_ok(got, want):
