@@ -97,6 +97,9 @@ TEPI_F32, TEPI_RELU_BF16, TEPI_MASK_BF16, TEPI_TRUNK_WGRAD, TEPI_TRUNK_DGRAD = 0
 IMG, PW, PLANE, CONV_CH, REPR_DIM = 84, 41, 1696, 32, 39200
 PLB, GUARD, WB_SLACK = 1776, 88, 128
 TB_ACT, TB_W = 128, 64
+POLICY_MAX_A, POLICY_MAX_PARTIALS, POLICY_GROUP = 128, 16384, 32   # DRQ_POLICY_MAX_A, DRQ_POLICY_MAX_PARTIALS; heads.cu kPolicyGroup
+POLICY_STATIC_SMEM = 1040        # policy_head_fwd_kernel's static shared memory (block-sum buffer + last-block flag)
+LN_MAX_F = 256                   # the LayerNorm kernels' feature bound (heads.cu: 32 lanes x kMaxFPerLane)
 GEMM_KK, GEMM_KMN, GEMM_MNMN = 0, 1, 2
 
 

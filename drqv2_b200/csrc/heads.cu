@@ -83,8 +83,9 @@ ln_tanh_fwd_kernel(const LnJobs jobs, int B, int F, float eps) {
         }
     }
     if (jb.rstd && lane == 0) jb.rstd[row] = rstd;
-    if (jb.tail && h_bf && lane < jb.n_tail)
-        h_bf[fb_index(F + lane, jb.row0_bf16 + row, jb.units_bf16)] = __float2bfloat16_rn(jb.tail[(long long)row * jb.ld_tail + lane]);
+    if (jb.tail && h_bf)
+        for (int t = lane; t < jb.n_tail; t += 32)
+            h_bf[fb_index(F + t, jb.row0_bf16 + row, jb.units_bf16)] = __float2bfloat16_rn(jb.tail[(long long)row * jb.ld_tail + t]);
 }
 
 // per row: dy = dh*(1-h^2); dxhat = dy*gamma; dz = rstd*(dxhat - mean(dxhat) - xhat*mean(dxhat*xhat)).
@@ -210,26 +211,32 @@ actor_sample_kernel(const float* __restrict__ mu_pre, const float* __restrict__ 
 }
 
 // Policy head (drqv2.py:81,88-92): mu_pre[m][:] = p2[m][:] . bf16(W4)^T + b4 for all M rows of a TB activation - the
-// Linear(hidden, A) as dot products on the CUDA cores (A <= 32 outputs: a tensor-core tile would be > 75 % padding and
-// run on M / 128 CTAs) - and, by the thread that holds each mu_pre value, the TruncatedNormal samples of up to
-// DRQ_POLICY_MAX_JOBS row ranges (utils.py:112-126).  Block = 8 rows, one warp per row, lanes split the row's 16-byte
-// units (32 rows per block left the launch on M / 32 = 16 SMs: 12.6 us as a graph node).  The weights are rounded to
-// bf16 when they are staged, i.e. the arithmetic is that of the bf16 GEMM this replaces (bf16 x bf16 products, fp32
-// sums).  A job with metrics needs the batch mean of the log-probabilities: every block leaves its partial sum in
-// scratch[1 + block], the block that finishes last (ticket in scratch[0]) adds them in block order.
+// Linear(hidden, A) as dot products on the CUDA cores (A <= 128 outputs: a tensor-core tile would be > 75 % padding at
+// A <= 32 and run on M / 128 CTAs) - and, by the thread that holds each mu_pre value, the TruncatedNormal samples of up
+// to DRQ_POLICY_MAX_JOBS row ranges (utils.py:112-126).  Block = 8 rows x one group of at most 32 actions: blockIdx.y
+// picks the group, ceil(A / gridDim.y) actions each (A <= 32: one group, all of A), and a block stages only its group's
+// rows of W4.  One warp per row, lanes split the row's 16-byte units (32 rows per block left the launch on M / 32 = 16
+// SMs: 12.6 us as a graph node).  The weights are rounded to bf16 when they are staged, i.e. the arithmetic is that of
+// the bf16 GEMM this replaces (bf16 x bf16 products, fp32 sums).  A job with metrics needs the batch mean of the
+// log-probabilities: every block leaves its partial sum in scratch[1 + blockIdx.y * gridDim.x + blockIdx.x], the block
+// that finishes last (ticket in scratch[0]) adds them in that order.
 struct PolicyJobs { drq_policy_sample j[DRQ_POLICY_MAX_JOBS]; int n; int metrics_job; };
 constexpr int kPolicyRows = 8;
+constexpr int kPolicyGroup = 32;          // actions per block at most
 
 __global__ void __launch_bounds__(256)
 policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, const float* __restrict__ w4,
                        const float* __restrict__ b4, float* __restrict__ mu_pre, int M, int H, int A, const PolicyJobs jobs,
                        const float* __restrict__ std_dev, float clip, unsigned int* __restrict__ scratch) {
-    extern __shared__ float w_s[];                       // [A][H]
+    extern __shared__ float w_s[];                       // [na][H]: this block's group of W4 rows
     __shared__ float sh[256];
     __shared__ int s_last;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int m = blockIdx.x * kPolicyRows + warp;
     const int nu = H / 8;
+    const int ga = (A + gridDim.y - 1) / gridDim.y;
+    const int a_lo = blockIdx.y * ga;                    // the group: actions a_lo .. a_lo + na - 1
+    const int na = min(ga, A - a_lo);
     const __nv_bfloat16* x = p2 + fb_index(0, m < M ? m : 0, units);
     // the lane's first units of the row are requested before the weights are staged (hides the staging barrier)
     uint4 v[4];
@@ -238,8 +245,8 @@ policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, co
         const int u = lane + 32 * k;
         v[k] = (m < M && u < nu) ? __ldg(reinterpret_cast<const uint4*>(x + (long long)u * DRQ_TB_ACT * 8)) : make_uint4(0, 0, 0, 0);
     }
-    for (int k = threadIdx.x; k < A * H / 4; k += 256) {          // H % 8 == 0: whole float4s
-        const float4 w = __ldg(reinterpret_cast<const float4*>(w4) + k);
+    for (int k = threadIdx.x; k < na * H / 4; k += 256) {         // H % 8 == 0: whole float4s
+        const float4 w = __ldg(reinterpret_cast<const float4*>(w4 + (long long)a_lo * H) + k);
         reinterpret_cast<float4*>(w_s)[k] = make_float4(__bfloat162float(__float2bfloat16_rn(w.x)), __bfloat162float(__float2bfloat16_rn(w.y)),
                                                         __bfloat162float(__float2bfloat16_rn(w.z)), __bfloat162float(__float2bfloat16_rn(w.w)));
     }
@@ -248,7 +255,7 @@ policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, co
     const float lo = -1.0f + 1e-6f, hi = 1.0f - 1e-6f;  // utils.py:113 (python: -1.0 + 1e-6 -> fp32)
     float lp_acc = 0.f;                                  // this thread's log-prob terms of the metrics job
     __syncthreads();
-    for (int a0 = 0; a0 < A; a0 += 8) {
+    for (int a0 = 0; a0 < na; a0 += 8) {
         float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
         for (int u0 = lane; u0 < nu; u0 += 128) {     // 4 units of the row in flight per lane
             if (u0 != lane || a0 != 0) {
@@ -268,7 +275,7 @@ policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, co
                 for (int j = 0; j < 4; ++j) { xv[2 * j] = __uint_as_float(w[j] << 16); xv[2 * j + 1] = __uint_as_float(w[j] & 0xFFFF0000u); }
 #pragma unroll
                 for (int a = 0; a < 8; ++a) {
-                    if (a0 + a < A) {
+                    if (a0 + a < na) {
                         const float4 w0 = *reinterpret_cast<const float4*>(w_s + (a0 + a) * H + u * 8);
                         const float4 w1 = *reinterpret_cast<const float4*>(w_s + (a0 + a) * H + u * 8 + 4);
                         acc[a] = fmaf(xv[0], w0.x, acc[a]); acc[a] = fmaf(xv[1], w0.y, acc[a]);
@@ -279,15 +286,15 @@ policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, co
                 }
             }
         }
-        // the row's dot products: butterfly over the lanes (fixed order), lane a keeps output a0 + a and samples it
+        // the row's dot products: butterfly over the lanes (fixed order), lane a keeps output a_lo + a0 + a and samples it
         float mine = 0.f;
 #pragma unroll
         for (int a = 0; a < 8; ++a) {
             const float t = warp_sum(acc[a]);
             if (lane == a) mine = t;
         }
-        const int j = a0 + lane;
-        if (lane < 8 && m < M && j < A) {
+        const int j = a_lo + a0 + lane;
+        if (lane < 8 && m < M && a0 + lane < na) {
             const float pre = mine + b4[j];
             mu_pre[(long long)m * A + j] = pre;
             for (int i = 0; i < jobs.n; ++i) {
@@ -312,19 +319,21 @@ policy_head_fwd_kernel(const __nv_bfloat16* __restrict__ p2, long long units, co
         }
     }
     if (jobs.metrics_job < 0) return;
-    // batch mean of the log-probabilities: block partials, combined in block order by the block that finishes last
+    // batch mean of the log-probabilities: block partials (y-major, then x), combined in that order by the block that
+    // finishes last
+    const unsigned int nblk = gridDim.x * gridDim.y;
     const float bsum = block_sum_256(lp_acc, sh);
     if (threadIdx.x == 0) {
-        reinterpret_cast<float*>(scratch)[1 + blockIdx.x] = bsum;
+        reinterpret_cast<float*>(scratch)[1 + blockIdx.y * gridDim.x + blockIdx.x] = bsum;
         __threadfence();
-        s_last = atomicAdd(scratch, 1u) == gridDim.x - 1;
+        s_last = atomicAdd(scratch, 1u) == nblk - 1;
     }
     __syncthreads();
     if (!s_last) return;
     // the last block adds the partials: thread t takes blocks t, t + 256, ... in order, then the block-wide sum (a fixed tree)
     __threadfence();
     float mine = 0.f;
-    for (unsigned int b = threadIdx.x; b < gridDim.x; b += 256) mine += __ldcg(reinterpret_cast<const float*>(scratch) + 1 + b);
+    for (unsigned int b = threadIdx.x; b < nblk; b += 256) mine += __ldcg(reinterpret_cast<const float*>(scratch) + 1 + b);
     const float tot = block_sum_256(mine, sh);
     if (threadIdx.x == 0) {
         const drq_policy_sample& jb = jobs.j[jobs.metrics_job];
@@ -568,7 +577,9 @@ int drq_ln_tanh_fwd_multi(const drq_ln_job* jobs, int njobs, int B, int F, float
         js.j[i] = jobs[i];
         DRQ_REQUIRE(jobs[i].partial && jobs[i].bias && jobs[i].gamma && jobs[i].beta && jobs[i].h_out && jobs[i].S >= 1,
                     "ln_tanh_fwd: null pointer in job %d", i);
-        DRQ_REQUIRE(jobs[i].n_tail >= 0 && jobs[i].n_tail <= 32, "ln_tanh_fwd: tail of job %d wider than 32", i);
+        DRQ_REQUIRE(jobs[i].n_tail >= 0 && (jobs[i].n_tail == 0 || !jobs[i].tail || !jobs[i].h_bf16 ||
+                                            F + jobs[i].n_tail <= 8 * jobs[i].units_bf16),
+                    "ln_tanh_fwd: tail of job %d does not fit the bf16 row (F + n_tail > 8 * units_bf16)", i);
     }
     if (B == 0) return DRQ_OK;
     const dim3 grid(B, njobs);
@@ -620,7 +631,8 @@ int drq_policy_head_fwd_bf16(const uint16_t* p2, int64_t units, const float* w4,
                              int H, int A, const drq_policy_sample* jobs, int njobs, const float* std_dev, float clip,
                              uint32_t* ticket, void* stream) {
     DRQ_REQUIRE(p2 && w4 && b4 && mu_pre, "policy_head_fwd: null pointer");
-    DRQ_REQUIRE(M > 0 && H > 0 && H % 8 == 0 && units * 8 >= H && A > 0 && A <= 32, "policy_head_fwd: bad dims (A <= 32, H % 8 == 0)");
+    DRQ_REQUIRE(M > 0 && H > 0 && H % 8 == 0 && units * 8 >= H && A > 0 && A <= DRQ_POLICY_MAX_A,
+                "policy_head_fwd: bad dims (A <= %d, H %% 8 == 0)", DRQ_POLICY_MAX_A);
     DRQ_REQUIRE(njobs >= 0 && njobs <= DRQ_POLICY_MAX_JOBS && (njobs == 0 || jobs), "policy_head_fwd: 0..%d sample jobs", DRQ_POLICY_MAX_JOBS);
     PolicyJobs pj{};
     pj.n = njobs;
@@ -635,10 +647,14 @@ int drq_policy_head_fwd_bf16(const uint16_t* p2, int64_t units, const float* w4,
             pj.metrics_job = i;
         }
     }
-    DRQ_REQUIRE(pj.metrics_job < 0 || (M + kPolicyRows - 1) / kPolicyRows <= 4096, "policy_head_fwd: the metrics scratch holds 4096 block partials (M <= 32768)");
-    const size_t smem = (size_t)A * H * sizeof(float);
+    const int groups = (A + kPolicyGroup - 1) / kPolicyGroup;
+    const dim3 grid((M + kPolicyRows - 1) / kPolicyRows, groups);
+    DRQ_REQUIRE(pj.metrics_job < 0 || (long long)grid.x * grid.y <= DRQ_POLICY_MAX_PARTIALS,
+                "policy_head_fwd: the metrics scratch holds %d block partials (ceil(M / 8) x ceil(A / 32) blocks)",
+                DRQ_POLICY_MAX_PARTIALS);
+    const size_t smem = (size_t)((A + groups - 1) / groups) * H * sizeof(float);
     if (int rc = ensure_smem((const void*)policy_head_fwd_kernel, smem, "policy_head_fwd")) return rc;
-    policy_head_fwd_kernel<<<(M + kPolicyRows - 1) / kPolicyRows, 256, smem, as_stream(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(p2),
+    policy_head_fwd_kernel<<<grid, 256, smem, as_stream(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(p2),
              (long long)units, w4, b4, mu_pre, M, H, A, pj, std_dev, clip, ticket);
     return check_launch("policy_head_fwd_kernel");
 }

@@ -466,6 +466,8 @@ class DrQV2Agent:
                              f"1 <= C <= {max_cin} stacked channels (drqv2.py:53 fixes 84 x 84)")
         self.action_dim = int(action_shape[0])
         self.feature_dim, self.hidden_dim = int(feature_dim), int(hidden_dim)
+        if self.mode == "bf16":
+            self._check_bf16_dims(dev)
 
         # models: built on the host in the reference's order (so a seed reproduces its init)
         self.encoder = Encoder(self.obs_shape)
@@ -494,6 +496,27 @@ class DrQV2Agent:
         self.train()
         self.critic_target.train()
 
+    def _check_bf16_dims(self, dev):
+        """Refuse at construction the shapes the tensor-core mode's head kernels refuse (csrc/heads.cu), which would
+        otherwise fail at the first act() or update()."""
+        A, Fd, H = self.action_dim, self.feature_dim, self.hidden_dim
+        if not 1 <= A <= _lib.POLICY_MAX_A:
+            raise ValueError(f"action_shape ({A},): mode='bf16' supports 1 <= A <= {_lib.POLICY_MAX_A} action dimensions "
+                             "(the policy head kernel); mode='fp32' has no such limit")
+        if H % 8:
+            raise ValueError(f"hidden_dim {H}: mode='bf16' needs a multiple of 8 (16-byte rows of the bf16 operands); "
+                             "mode='fp32' has no such limit")
+        groups = -(-A // _lib.POLICY_GROUP)
+        slab = 4 * H * -(-A // groups)                 # fp32 weights of one policy-head block's action group
+        optin = torch.cuda.get_device_properties(dev).shared_memory_per_block_optin
+        if slab + _lib.POLICY_STATIC_SMEM > optin:
+            raise ValueError(f"hidden_dim {H} with {A} actions: mode='bf16' stages {slab} bytes of policy-head weights per "
+                             f"block, more than the {optin - _lib.POLICY_STATIC_SMEM} bytes of shared memory a block can "
+                             "have here; mode='fp32' has no such limit")
+        if not 1 <= Fd <= _lib.LN_MAX_F:
+            raise ValueError(f"feature_dim {Fd}: the LayerNorm kernels hold 1 <= F <= {_lib.LN_MAX_F} features "
+                             "(in mode='fp32' as well)")
+
     # ------------------------------------------------------------------ plumbing
     def _to_device(self, dev):
         self._dev = dev
@@ -507,7 +530,8 @@ class DrQV2Agent:
         self._scal_dev = torch.zeros(SCAL_SLOT, device=dev)   # layout: SCAL_OFF
         self._init_scalar_ring()
         self._counter = torch.zeros(1, dtype=torch.int64, device=dev)
-        self._policy_ticket = torch.zeros(1 + 4096, dtype=torch.int32, device=dev)   # drq_policy_head_fwd_bf16's scratch words
+        # drq_policy_head_fwd_bf16's scratch words: block ticket + one partial per block of the largest grid it takes
+        self._policy_ticket = torch.zeros(1 + _lib.POLICY_MAX_PARTIALS, dtype=torch.int32, device=dev)
         self._metrics_host = torch.zeros(8, dtype=torch.float32).pin_memory()
         self._injected = None
         self._bf16 = _bf16.Bf16State(self) if self.mode == "bf16" else None

@@ -432,7 +432,8 @@ typedef struct {
     float* h_out; int64_t ld_h; float* xhat; float* rstd;
     uint16_t* h_bf16; int64_t units_bf16; int64_t row0_bf16;
     const float* tail; int64_t ld_tail; int32_t n_tail;   /* nullable: tail[b][0..n_tail) is appended at feature F of the bf16 row
-                                                             (the action of torch.cat([h, action]), drqv2.py:117) */
+                                                             (the action of torch.cat([h, action]), drqv2.py:117);
+                                                             F + n_tail <= 8 * units_bf16 */
 } drq_ln_job;
 int drq_ln_tanh_fwd_multi(const drq_ln_job* jobs, int njobs, int B, int F, float eps, void* stream);
 
@@ -461,11 +462,15 @@ int drq_actor_sample(const float* mu_pre, const float* eps, const float* std_dev
 
 /* Policy head of the tensor-core mode in one launch (drqv2.py:81,88-92 + utils.py:112-126): mu_pre[m][a] =
  * p2[m][:] . bf16(w4[a][:]) + b4[a] for the M rows of the TB activation p2 (units per row), and - by the thread that
- * holds each value - drq_actor_sample's arithmetic on up to DRQ_POLICY_MAX_JOBS row ranges.  At most one job carries
- * metrics (it needs eps); `scratch` then is 1 + ceil(M / 8) (at most 4097) zero-initialised 32-bit words (block ticket + per-block
- * log-prob sums) that the kernel leaves zeroed.  Replaces a 128 x 64 tensor-core tile that was > 75 % padding
- * (A <= 32 outputs) followed by one or two sampling launches. */
+ * holds each value - drq_actor_sample's arithmetic on up to DRQ_POLICY_MAX_JOBS row ranges.  1 <= A <= DRQ_POLICY_MAX_A,
+ * H % 8 == 0; the actions are split into ceil(A / 32) balanced groups, and one group's ceil(A / groups) x H fp32 weights
+ * must fit a block's opt-in shared memory (128 KB at A = 32 or 128, H = 1024).  At most one job carries metrics (it
+ * needs eps); `scratch` then is 1 + ceil(M / 8) * ceil(A / 32) (at most 1 + DRQ_POLICY_MAX_PARTIALS) zero-initialised
+ * 32-bit words (block ticket + per-block log-prob sums) that the kernel leaves zeroed.  Replaces a 128 x 64 tensor-core
+ * tile that was > 75 % padding (A <= 32 outputs) followed by one or two sampling launches. */
 #define DRQ_POLICY_MAX_JOBS 2
+#define DRQ_POLICY_MAX_A 128
+#define DRQ_POLICY_MAX_PARTIALS 16384   /* M <= 32768 at every A <= 128 */
 typedef struct { int32_t row0; int32_t rows; const float* eps; float* action_out; int64_t ld_a; float* mu_out;
                  float* metrics; uint16_t* a_bf16; int64_t units_a; int32_t feat_off; int32_t reserved; } drq_policy_sample;
 int drq_policy_head_fwd_bf16(const uint16_t* p2, int64_t units, const float* w4, const float* b4, float* mu_pre, int M,
