@@ -466,6 +466,9 @@ class DrQV2Agent:
                              f"1 <= C <= {max_cin} stacked channels (drqv2.py:53 fixes 84 x 84)")
         self.action_dim = int(action_shape[0])
         self.feature_dim, self.hidden_dim = int(feature_dim), int(hidden_dim)
+        if not 1 <= self.feature_dim <= _lib.LN_MAX_F:
+            raise ValueError(f"feature_dim {self.feature_dim}: the LayerNorm kernels hold 1 <= F <= {_lib.LN_MAX_F} "
+                             "features (in mode='fp32' as well)")
         if self.mode == "bf16":
             self._check_bf16_dims(dev)
 
@@ -499,7 +502,7 @@ class DrQV2Agent:
     def _check_bf16_dims(self, dev):
         """Refuse at construction the shapes the tensor-core mode's head kernels refuse (csrc/heads.cu), which would
         otherwise fail at the first act() or update()."""
-        A, Fd, H = self.action_dim, self.feature_dim, self.hidden_dim
+        A, H = self.action_dim, self.hidden_dim
         if not 1 <= A <= _lib.POLICY_MAX_A:
             raise ValueError(f"action_shape ({A},): mode='bf16' supports 1 <= A <= {_lib.POLICY_MAX_A} action dimensions "
                              "(the policy head kernel); mode='fp32' has no such limit")
@@ -513,9 +516,6 @@ class DrQV2Agent:
             raise ValueError(f"hidden_dim {H} with {A} actions: mode='bf16' stages {slab} bytes of policy-head weights per "
                              f"block, more than the {optin - _lib.POLICY_STATIC_SMEM} bytes of shared memory a block can "
                              "have here; mode='fp32' has no such limit")
-        if not 1 <= Fd <= _lib.LN_MAX_F:
-            raise ValueError(f"feature_dim {Fd}: the LayerNorm kernels hold 1 <= F <= {_lib.LN_MAX_F} features "
-                             "(in mode='fp32' as well)")
 
     # ------------------------------------------------------------------ plumbing
     def _to_device(self, dev):

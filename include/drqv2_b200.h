@@ -202,34 +202,50 @@ int drq_random_shift_f32(const float* in, const int32_t* shift, float* out, int 
 /* conv1 of drqv2.py:55 (Cin->32, k3, stride 2) + ReLU, with RandomShiftsAug
  * (integer shift, pad 4) and `obs / 255.0 - 0.5` (drqv2.py:64) fused into the
  * loader.  obs u8 [N][cin][84][84]; shift int32 [N][2] (x,y) or NULL for no
- * augmentation (act path).  out: wide plane [N][32][DRQ_PLANE]. */
+ * augmentation (act path).  out: wide plane [N][32][DRQ_PLANE]; writes positions [0, 1681) of each
+ * plane (the 41 x 41 output) and nothing else - the plane's slack [1681, DRQ_PLANE) is left as it was. */
 int drq_conv1_fwd_f32(const uint8_t* obs, const int32_t* shift, const float* w, const float* b,
                       float* out, int N, int cin, int pad, void* stream);
 
 /* weight/bias gradient of conv1: dw [32][cin][3][3], db [32] from
- * dpre (wide, gradient w.r.t. the pre-ReLU output).  partial: workspace of
- * drq_conv_wgrad_ws_floats(cin) floats. */
+ * dpre (wide, gradient w.r.t. the pre-ReLU output; read on [0, 1681) of each plane only).
+ * partial: workspace of drq_conv_wgrad_ws_floats(cin) floats. */
 int drq_conv1_wgrad_f32(const uint8_t* obs, const int32_t* shift, const float* dpre,
                         float* partial, float* dw, float* db, int N, int cin, int pad,
                         void* stream);
 
 /* conv2..4 of drqv2.py:56-59 (32->32, k3, stride 1) + ReLU.
  * in: wide plane; hout = valid output rows = cols (39, 37 or 35).
- * compact_out != 0: write out as [N][32][hout][hout] (the flattened features
- * of drqv2.py:66) instead of the wide plane. */
+ * compact_out == 0: writes positions [0, hout*41) of each plane of the wide
+ * out (rows < hout, all 41 columns; columns >= hout hold values without
+ * meaning), nothing else.  compact_out != 0: writes exactly out[N][32][hout][hout]
+ * (the flattened features of drqv2.py:66) instead.  Valid outputs read `in`
+ * only inside hin x hin (hin = hout + 2); the rest of the plane may hold
+ * anything, NaN included. */
 int drq_conv3x3_fwd_f32(const float* in, const float* w, const float* b, float* out, int N,
                         int hout, int compact_out, void* stream);
 
 /* data gradient: din_pre[ci][q] = relu'(act_in[ci][q]) * sum_{co,tap} w[co][ci][tap] dout[co][q-off].
- * dout: wide, gradient w.r.t. this layer's PRE-ReLU output (zero outside the
- * valid hout x hout region).  act_in: this layer's input activation (post-ReLU
- * output of the layer below), used as the ReLU mask.  din: wide, gradient
- * w.r.t. the layer below's pre-ReLU output, zero outside (hout+2)^2. */
+ * dout: wide, gradient w.r.t. this layer's PRE-ReLU output.  It is read on
+ * positions [0, (hout+2)*41) of each plane, and there it must be +0 outside
+ * the valid hout x hout region: in rows hout, hout+1 and in columns >= hout.
+ * Rows >= hout+2 and the slack are not read.  act_in: this layer's input
+ * activation (post-ReLU output of the layer below), used as the ReLU mask and
+ * read inside hin x hin (hin = hout + 2) only.  din: wide, gradient w.r.t. the
+ * layer below's pre-ReLU output; written on [0, (hout+2)*41) of each plane -
+ * rows < hout+2, with +0 at columns >= hout+2 - and nowhere else: its rows
+ * >= hout+2 and its slack are left as they were, so a caller that passes din
+ * on as the next layer's dout (hout' = hout+2) keeps its rows hout', hout'+1
+ * at +0 itself (drqv2.py's workspace allocates them zeroed and no kernel
+ * writes them). */
 int drq_conv3x3_dgrad_f32(const float* dout, const float* w, const float* act_in, float* din,
                           int N, int hout, void* stream);
 
-/* weight/bias gradient of a 32->32 layer.  in: wide input activation, dpre:
- * wide gradient w.r.t. pre-ReLU output.  partial: workspace of
+/* weight/bias gradient of a 32->32 layer.  in: wide input activation, read on
+ * the whole plane [0, DRQ_PLANE): outside hin x hin it must be finite (it
+ * meets zeros of dpre there, and 0 * NaN is NaN).  dpre: wide gradient w.r.t.
+ * the pre-ReLU output, read on [0, hout*41) only, and +0 there outside the
+ * valid hout x hout region (columns >= hout).  partial: workspace of
  * drq_conv_wgrad_ws_floats(32) floats. */
 int drq_conv3x3_wgrad_f32(const float* in, const float* dpre, float* partial, float* dw,
                           float* db, int N, int hout, void* stream);
@@ -402,7 +418,13 @@ int drq_conv_wgrad_reduce_multi(const drq_wgrad_reduce_job* jobs, int njobs, voi
  * splitk > 1 (batch must be 1): K is cut in `splitk` chunks and chunk s writes
  * its raw partial sum to C + s*bs_c (bias/epilogue ignored) — reduced in fixed
  * order by drq_ln_tanh_fwd.
- * accumulate != 0: C += result (after epilogue).  mask has C's shape/ld. */
+ * accumulate != 0: C += result (after epilogue).  DRQ_EPI_MASK: mask(m, n) =
+ * mask[m*ldmask + n] (at mask + z*bs_mask per batch entry).  DRQ_EPI_MASK_WIDE
+ * (N = 39200): the mask is the compact feature matrix [M][ldmask] and column n
+ * = c*1225 + y*35 + x is stored at C[m*ldc + c*DRQ_PLANE + y*41 + x] - only
+ * those compact->wide positions are written; columns and rows 35..40 of each
+ * plane and its slack are left as they were.  Every epilogue writes rows < M,
+ * columns < N (split planes z < splitk) and nothing else. */
 int drq_gemm_f32(const float* A, int64_t sa_m, int64_t sa_k, const float* B, int64_t sb_k,
                  int64_t sb_n, float* C, int64_t ldc, const float* bias, const float* mask,
                  int64_t ldmask, int M, int N, int K, int epilogue, int accumulate, int batch,

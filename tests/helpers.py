@@ -1,6 +1,7 @@
 """Shared test helpers: the integer formulas the golden inputs were generated with
-(tests/golden/make_golden.py) and probe positions; WB / TB layout conversions; the element-wise error bound and the
-stray-store sentinels of the bf16 conv kernel tests (self-tested in test_conv_checks_cpu.py)."""
+(tests/golden/make_golden.py) and probe positions; WB / TB layout conversions; the element-wise error bounds and the
+stray-store sentinels of the kernel tests (self-tested in test_conv_checks_cpu.py, test_gemm_schedule_cpu.py and
+test_fp32_schedule_cpu.py)."""
 import numpy as np
 
 
@@ -144,6 +145,25 @@ def assert_f32_bound(got, want, absref, chain, c, what):
         return 0.0
     need = torch.where(unit > 0, err / unit.clamp_min(1e-300), torch.zeros_like(err))
     return float(need.max())
+
+
+def check_sum_bound(kernel, got, want, absref, n, ratios=None, c=2.0):
+    """|got - want| <= c 2^-24 (n + 8) A element-wise, for fp32 results that are sums along chains of at most n
+    sequential fp32 steps; A the same sum over absolute values (a NaN fails).  The largest |got - want| / bound goes into
+    ratios[kernel] (the share of c the kernel needed)."""
+    import torch
+    got, want = got.double(), want.double()
+    bound = c * 2.0 ** -24 * (n + 8) * absref.double()
+    err = (got - want).abs()
+    bad = ~(err <= bound)
+    if bad.any():
+        i = int(bad.reshape(-1).nonzero()[0])
+        raise AssertionError(f"{kernel}: {int(bad.sum())} elements out of bound, first at flat {i}: got "
+                             f"{float(got.reshape(-1)[i])!r} want {float(want.reshape(-1)[i])!r}")
+    r = float(torch.where(bound > 0, err / bound.clamp_min(1e-300), torch.zeros_like(err)).max()) if err.numel() else 0.0
+    if ratios is not None:
+        ratios[kernel] = max(ratios.get(kernel, 0.0), r)
+    return r
 
 
 def max_norm_ok(got, want):

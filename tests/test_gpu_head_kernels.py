@@ -12,7 +12,7 @@ import ctypes as C
 import pytest
 import torch
 
-from tests.helpers import assert_sentinel_outside, bits_equal, fill_sentinel
+from tests.helpers import assert_sentinel_outside, bits_equal, check_sum_bound, fill_sentinel
 
 pytestmark = pytest.mark.gpu
 
@@ -49,17 +49,8 @@ def _ceil(n, m):
 
 
 def _check(kernel, got, want, absref, n, c=SUM_C):
-    """|got - want| <= c 2^-24 (n + 8) A element-wise"""
-    got, want = got.double(), want.double()
-    bound = c * 2.0 ** -24 * (n + 8) * absref.double()
-    err = (got - want).abs()
-    bad = ~(err <= bound)
-    if bad.any():
-        i = int(bad.reshape(-1).nonzero()[0])
-        raise AssertionError(f"{kernel}: {int(bad.sum())} elements out of bound, first at flat {i}: got "
-                             f"{float(got.reshape(-1)[i])!r} want {float(want.reshape(-1)[i])!r}")
-    r = float(torch.where(bound > 0, err / bound.clamp_min(1e-300), torch.zeros_like(err)).max()) if err.numel() else 0.0
-    RATIOS[kernel] = max(RATIOS.get(kernel, 0.0), r)
+    """|got - want| <= c 2^-24 (n + 8) A element-wise (tests/helpers.check_sum_bound)"""
+    check_sum_bound(kernel, got, want, absref, n, RATIOS, c)
 
 
 def _tb(rows, feats, dev, batch=1):
@@ -83,7 +74,46 @@ def _rand(g, *shape, lo=-1.0, hi=1.0):
 
 
 # ---------------------------------------------------------------- trunk tail: split-K sum + bias + LayerNorm + tanh
-@pytest.mark.parametrize("S", [1, 35, 64, 65, 130])
+def check_ln_tanh_fwd(p, bias, gamma, beta, h, xhat, rstd, B, F, S, ratios):
+    """h_out [B + 1][ld_h] (and, when not None, xhat [>= B F] and rstd [B + 1]) of one trunk tail on the split planes
+    p [S][B][F] (fp64 of the fp32 partials) against fp64; everything but rows < B, columns < F of h_out (the tail columns
+    are the caller's), xhat[:B F] and rstd[:B] keeps the sentinel"""
+    dev = h.device
+    z = p.sum(0) + bias.double().cpu()
+    za = p.abs().sum(0) + bias.double().cpu().abs()
+    mean = z.mean(1, keepdim=True)
+    var = ((z - mean) ** 2).mean(1, keepdim=True)
+    r = 1 / torch.sqrt(var + 1e-5)
+    xh = (z - mean) * r
+    y = xh * gamma.double().cpu() + beta.double().cpu()
+    # z carries the fp32 sum's error (S + 4 terms of za); normalised by the row's spread it moves xhat and y
+    dz = 2.0 ** -24 * (S + 8) * za + 2.0 ** -22 * z.abs()
+    dx = (dz * r).amax(1, keepdim=True) * (1 + xh.abs()) * 2 + 2.0 ** -21 * (1 + xh.abs())
+    if rstd is not None:
+        rb = (4 * dz.amax(1) * r[:, 0] + 2.0 ** -20) * r[:, 0]      # std moves by at most max|dz|
+        re = (rstd[:B].cpu().double() - r[:, 0]).abs()
+        assert (re <= rb).all(), f"rstd error {float((re / rb).max())} x bound"
+        wr = torch.zeros(B + 1, dtype=torch.bool, device=dev)
+        wr[:B] = True
+        assert_sentinel_outside(rstd, wr, "rstd")
+    if xhat is not None:
+        dxe = (xhat[:B * F].view(B, F).cpu().double() - xh).abs()
+        assert (dxe <= dx).all(), f"xhat error {float((dxe / dx).max())} x bound"
+        ratios["ln_tanh_fwd xhat"] = max(ratios.get("ln_tanh_fwd xhat", 0), float((dxe / dx).max()))
+        wx = torch.zeros(xhat.numel(), dtype=torch.bool, device=dev)
+        wx[:B * F] = True
+        assert_sentinel_outside(xhat, wx, "xhat")
+    hw = torch.tanh(y)
+    dh = dx * gamma.double().cpu().abs() * (1 - hw ** 2) + 2.0 ** -21
+    hg = h[:B, :F].cpu().double()
+    assert ((hg - hw).abs() <= dh).all(), f"h error {float(((hg - hw).abs() / dh).max())} x bound"
+    ratios["ln_tanh_fwd h"] = max(ratios.get("ln_tanh_fwd h", 0), float(((hg - hw).abs() / dh).max()))
+    w = torch.zeros_like(h, dtype=torch.bool)
+    w[:B, :F] = True                                                  # the tail columns of h_out are the caller's
+    assert_sentinel_outside(h, w, "h_out")
+
+
+@pytest.mark.parametrize("S", [1, 35, 64, 65, 130, 145, 273])
 @pytest.mark.parametrize("B", [1, 3, 129, 512])
 @pytest.mark.parametrize("F", [50, 64, 65, 100, 128, 129, 256])
 def test_ln_tanh_fwd_multi(dev, F, B, S):
@@ -126,37 +156,7 @@ def test_ln_tanh_fwd_multi(dev, F, B, S):
             written |= w.view(tb.batch, nb, 128, tb.units, 8).permute(0, 1, 3, 2, 4).reshape(-1)
         assert_sentinel_outside(tb.buf, written, "ln_tanh_fwd TB")
     for (p, bias, gamma, beta, h, xhat, rstd, tail, nt, tb, row0) in ref:
-        z = p.sum(0) + bias.double().cpu()
-        za = p.abs().sum(0) + bias.double().cpu().abs()
-        mean = z.mean(1, keepdim=True)
-        var = ((z - mean) ** 2).mean(1, keepdim=True)
-        r = 1 / torch.sqrt(var + 1e-5)
-        xh = (z - mean) * r
-        y = xh * gamma.double().cpu() + beta.double().cpu()
-        # z carries the fp32 sum's error (S + 4 terms of za); normalised by the row's spread it moves xhat and y
-        dz = 2.0 ** -24 * (S + 8) * za + 2.0 ** -22 * z.abs()
-        dx = (dz * r).amax(1, keepdim=True) * (1 + xh.abs()) * 2 + 2.0 ** -21 * (1 + xh.abs())
-        rb = (4 * dz.amax(1) * r[:, 0] + 2.0 ** -20) * r[:, 0]      # std moves by at most max|dz|
-        re = (rstd[:B].cpu().double() - r[:, 0]).abs()
-        assert (re <= rb).all(), f"rstd error {float((re / rb).max())} x bound"
-        dxe = (xhat[:B * F].view(B, F).cpu().double() - xh).abs()
-        assert (dxe <= dx).all(), f"xhat error {float((dxe / dx).max())} x bound"
-        hw = torch.tanh(y)
-        dh = dx * gamma.double().cpu().abs() * (1 - hw ** 2) + 2.0 ** -21
-        hg = h[:B, :F].cpu().double()
-        assert ((hg - hw).abs() <= dh).all(), f"h error {float(((hg - hw).abs() / dh).max())} x bound"
-        RATIOS["ln_tanh_fwd h"] = max(RATIOS.get("ln_tanh_fwd h", 0), float(((hg - hw).abs() / dh).max()))
-        RATIOS["ln_tanh_fwd xhat"] = max(RATIOS.get("ln_tanh_fwd xhat", 0), float((dxe / dx).max()))
-        # sentinels of the fp32 outputs (the tail columns of h_out belong to the caller)
-        w = torch.zeros_like(h, dtype=torch.bool)
-        w[:B, :F] = True                                              # the tail columns of h_out are the caller's
-        assert_sentinel_outside(h, w, "h_out")
-        wx = torch.zeros(xhat.numel(), dtype=torch.bool, device=dev)
-        wx[:B * F] = True
-        assert_sentinel_outside(xhat, wx, "xhat")
-        wr = torch.zeros(B + 1, dtype=torch.bool, device=dev)
-        wr[:B] = True
-        assert_sentinel_outside(rstd, wr, "rstd")
+        check_ln_tanh_fwd(p, bias, gamma, beta, h, xhat, rstd, B, F, S, RATIOS)
         # the bf16 copy is RN-bf16 of h_out, the tail columns bf16(tail)
         v = tb.view(0)
         assert bits_equal(v[row0:row0 + B, :F], h[:B, :F].to(torch.bfloat16)), "TB copy != RN-bf16(h_out)"
