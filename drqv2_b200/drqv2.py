@@ -722,14 +722,15 @@ class DrQV2Agent:
         key = bool(sample)
         g = w["graph"].get(key)
         if g is None:
-            self._act_body(w, n, sample)          # warm-up (also opts kernels in to big smem)
+            # warm-up (also opts kernels in to big smem): its action is this call's, and a capture runs nothing - so
+            # the first call draws its noise once, as every later replay does
+            self._act_body(w, n, sample)
             if self.use_cuda_graph:
                 torch.cuda.synchronize()
                 g = torch.cuda.CUDAGraph()
                 with _capture(g):
                     self._act_body(w, n, sample)
                 w["graph"][key] = g
-                g.replay()
         else:
             g.replay()
         w["host_out"].copy_(w["out"], non_blocking=True)

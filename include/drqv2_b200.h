@@ -127,10 +127,21 @@ int drq_ring_sample(const int32_t* ep_table, const int32_t* n_episodes, int nste
 
 /* ------------------------------------------------------------------ RNG */
 
+/* Every draw is Philox4x32-10 with key `seed` and counter (element index lo, index hi, word lo, word hi) where
+ * word = (*counter << 3) | stream.  Streams: 0 = replay sample (the loader's seed), 1 = shifts, 3 = the update's
+ * noise, 5 = drq_rng_normal_f32.  Integers are multiply-shift reductions of a word w: (w * range) >> 32 - the
+ * sample's episode from word 0 (range E), its idx - 1 from word 1 (range len - nstep + 1); shift_obs (x, y) from
+ * words 0, 1 and shift_next (x, y) from words 2, 3 of element b (range 2 * pad + 1).  Normals are Box-Muller on
+ * the pair i >> 1: u = ((float)(w >> 8) + 0.5f) * 2^-24 in fp32, so above 2^23 the + 0.5 rounds to even and u
+ * lies on a 2^-23 grid, and w >> 8 == 0xFFFFFF gives u1 = 1.0 exactly: a normal of +0 or -0.  Element i is
+ * sqrt(-2 ln u1) * cos(2 pi u2), sin when i is odd; eps_critic takes words 0 (u1) and 1 (u2), eps_actor
+ * words 2 and 3, drq_rng_normal_f32 words 0 and 1.  A launch writes elements [0, B) / [0, B*A) / [0, n) and
+ * nothing past them (tests/test_gpu_draws.py holds every producer to this, tests/helpers.py restates it). */
+
 /* Per-update random draws, in the reference's order (drqv2.py:241-242 shifts,
  * utils.py:119 noise x2): shift_obs/shift_next int32 [B][2] = (x, y) in
  * [0, 2*pad], eps_critic/eps_actor f32 [B][A] ~ N(0,1).  Keyed by
- * (seed, *counter); `counter` is advanced by drq_counter_advance. */
+ * (seed, *counter) on streams 1 and 3; the kernel does not advance `counter` (drq_counter_advance does). */
 int drq_rng_update_draws(uint64_t seed, const uint64_t* counter, int pad, int32_t* shift_obs,
                          int32_t* shift_next, float* eps_critic, float* eps_actor, int B, int A,
                          void* stream);
@@ -172,7 +183,8 @@ int drq_update_prologue_ring(const float* scal_ring, int slots, uint64_t* cursor
 
 /* The same in two launches: part 1 = what the encoder's first kernel waits for (the two shift draws and the replay
  * sample (ep_start, idx)); part 2 = the rest (host scalars, the two noise draws, action copy, n-step reward / discount),
- * launched after part 1 - on a side stream it runs beside conv1.  part 3 = drq_update_prologue_ring.  Bit-identical. */
+ * launched after part 1 - on a side stream it runs beside conv1.  part 3 = drq_update_prologue_ring.  Bit-identical.
+ * Part 1 advances the sampler's counter only: it reads *counter but leaves it and the scalar cursor to part 2. */
 int drq_update_prologue_ring_part(const float* scal_ring, int slots, uint64_t* cursor, float* scal_out, uint64_t seed,
                                   uint64_t* counter, int pad, int32_t* shift_obs, int32_t* shift_next, float* eps_critic,
                                   float* eps_actor, int B, int A, const drq_ring_src* src, float* action_out,
@@ -183,7 +195,8 @@ int drq_ring_sample_step(const int32_t* ep_table, const int32_t* n_episodes, int
                          int32_t* ep_start_out, int32_t* idx_out, int B, void* stream);
 
 /* everything an update needs before its first real kernel, in one launch (one block): drq_scalars_fetch, then -
- * unless shift_obs == NULL (injected draws) - drq_rng_update_draws and *counter += 1. */
+ * unless shift_obs == NULL (injected draws) - drq_rng_update_draws and *counter += 1.  With shift_obs == NULL no draw
+ * buffer is written and the counter is neither read nor advanced (also in drq_update_prologue_ring[_part]). */
 int drq_update_prologue(const float* scal_ring, int slots, uint64_t* cursor, float* scal_out, uint64_t seed, uint64_t* counter,
                         int pad, int32_t* shift_obs, int32_t* shift_next, float* eps_critic, float* eps_actor, int B, int A,
                         void* stream);

@@ -230,3 +230,176 @@ def check_conv_fwd_outputs(out, feat, tb_view, tb_rows, want, absref, N, hout, w
     rows[list(tb_rows)] = True
     assert_sentinel_outside(tb_view, rows.view(-1, 1).expand(tb_view.shape), what + " TB")
     return ratio
+
+
+# ---- exact reference of the random draws (csrc/ring.cu): Philox4x32-10 keyed by the seed, counter word
+# (counter << 3) | stream, element index in the low 64 bits.  The integer draws are oracle.update_shifts and
+# oracle.sample_indices (multiply-shift reductions, bit-exact); normals are Box-Muller on a pair of words with u formed
+# in fp32 exactly as the kernels form it.
+STREAM_SAMPLE, STREAM_SHIFT, STREAM_EPS, STREAM_NOISE = 0, 1, 3, 5
+NORMAL_C = 8.0               # |got - want| <= NORMAL_C * 2^-24 * rad (sqrt(-2 ln u1))
+INT_SENTINEL = 0x7FFFFFFF
+
+
+def philox_words(seed, stream, counter, index):
+    """uint64 [len(index)][4]: the four 32-bit words of key `seed` at counter word (counter << 3) | stream"""
+    from oracle import drq_oracle as O
+    return O.philox4x32(int(seed), (int(counter) << 3) | int(stream), np.asarray(index, np.uint64))
+
+
+def uniform24(w):
+    """((float)(w >> 8) + 0.5f) * 2^-24 in fp32: above 2^23 the + 0.5 rounds to even, so the upper half lies on a
+    2^-23 grid and w >> 8 == 0xFFFFFF gives exactly 1.0"""
+    u = (np.asarray(w, np.uint64) >> np.uint64(8)).astype(np.float32)
+    return (u + np.float32(0.5)) * np.float32(2.0 ** -24)
+
+
+def box_muller(w_rad, w_ang, odd, use_sin_for_odd=True):
+    """(normal, rad) in fp64 from the fp32 uniforms of two words: rad * cos(2 pi u2), sin for odd elements"""
+    u1 = uniform24(w_rad).astype(np.float64)
+    u2 = uniform24(w_ang).astype(np.float64)
+    rad = np.sqrt(-2.0 * np.log(u1))
+    ang = 2.0 * np.pi * u2
+    odd = np.asarray(odd, bool) & use_sin_for_odd
+    return np.where(odd, rad * np.sin(ang), rad * np.cos(ang)), rad
+
+
+def normals_ref(seed, stream, counter, n, words=(0, 1)):
+    """element i of an N(0,1) draw: pair i >> 1 on words `words` of the Philox block"""
+    i = np.arange(n, dtype=np.int64)
+    r = philox_words(seed, stream, counter, i >> 1)
+    return box_muller(r[:, words[0]], r[:, words[1]], (i & 1).astype(bool))
+
+
+def update_draws_ref(seed, counter, pad, B, A):
+    """the four draws of one update: dict of shift_obs, shift_next, eps_critic / eps_actor (words 0-1 / 2-3 of
+    stream 3) and their rad"""
+    from oracle import drq_oracle as O
+    so, sn = O.update_shifts(seed, counter, pad, B)
+    ec, rc = normals_ref(seed, STREAM_EPS, counter, B * A, (0, 1))
+    ea, ra = normals_ref(seed, STREAM_EPS, counter, B * A, (2, 3))
+    return dict(shift_obs=so, shift_next=sn, eps_critic=ec, rad_critic=rc, eps_actor=ea, rad_actor=ra)
+
+
+def check_normals(got, want, rad, what):
+    """|got - want| <= NORMAL_C 2^-24 rad element-wise (a NaN fails).  Returns the largest |got - want| / (2^-24 rad):
+    the constant this draw needed.  A word or pair mix-up is off by O(1) and misses the bound by ~10^6."""
+    got = np.asarray(got, np.float64).ravel()
+    want, rad = np.asarray(want, np.float64).ravel(), np.asarray(rad, np.float64).ravel()
+    assert got.shape == want.shape, (what, got.shape, want.shape)
+    unit = 2.0 ** -24 * rad
+    err = np.abs(got - want)
+    bad = ~(err <= NORMAL_C * unit)
+    if bad.any():
+        i = int(np.flatnonzero(bad)[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} of {got.size} normals outside |got - want| <= {NORMAL_C:g} "
+                             f"2^-24 rad, first at {i}: got {got[i]!r}, want {want[i]!r}, rad {rad[i]!r}")
+    live = unit > 0
+    return float((err[live] / unit[live]).max()) if live.any() else 0.0
+
+
+def assert_bits_equal(got, want, what):
+    """integer draws and gathered values: equal bit for bit, with the first difference named"""
+    got, want = np.asarray(got), np.asarray(want)
+    assert got.shape == want.shape, (what, got.shape, want.shape)
+    if got.dtype.kind == "f":
+        got, want = got.view(np.int32 if got.itemsize == 4 else np.int64), want.astype(got.dtype).view(
+            np.int32 if got.itemsize == 4 else np.int64)
+    diff = got != want
+    if diff.any():
+        i = np.unravel_index(int(np.flatnonzero(diff)[0]), got.shape)
+        raise AssertionError(f"{what}: {int(diff.sum())} of {got.size} differ, first at {tuple(int(v) for v in i)}: "
+                             f"got {got[i]!r}, want {want[i]!r}")
+
+
+# ---- the agent's key schedule: which (seed, stream, counter) keys each public call consumes
+def key_schedule(calls, seed, loader_seed):
+    """calls: sequence of "act", "act_eval", "update", "update_skip", "stage_critic", "stage_actor" -> list of
+    (call, agent counter before, [keys consumed]) with a key (seed, stream, counter).  Each call that draws takes the
+    agent counter once and advances it by one; an update also takes the loader's counter (its own seed, stream 0)."""
+    c = lc = 0
+    out = []
+    for call in calls:
+        keys = []
+        if call in ("act", "stage_critic", "stage_actor"):
+            keys = [(seed, STREAM_NOISE, c)]
+        elif call == "update":
+            keys = [(seed, STREAM_SHIFT, c), (seed, STREAM_EPS, c), (loader_seed, STREAM_SAMPLE, lc)]
+            lc += 1
+        else:
+            assert call in ("act_eval", "update_skip"), call
+        out.append((call, c, keys))
+        if keys:
+            c += 1
+    return out
+
+
+def assert_keys_disjoint(schedule):
+    """no (seed, stream, counter) key is consumed twice"""
+    seen = {}
+    for k, (call, _, keys) in enumerate(schedule):
+        for key in keys:
+            assert key not in seen, f"key {key} of call {k} ({call}) was consumed before by call {seen[key]}"
+            seen[key] = k
+
+
+# ---- host model of the replay ring's episode bookkeeping (replay_buffer.GpuRing), by slot ownership
+class RingModel:
+    """Episodes are written one after another at the head, modulo capacity; an episode stays resident while every slot
+    it was written to still holds it (FIFO eviction of whole episodes).  table(min_len) is what the sampler sees:
+    (start slot, len = rows - 1) of the resident episodes with len >= min_len, the newest max_episodes of them."""
+
+    def __init__(self, capacity, max_episodes):
+        self.cap, self.max_episodes = capacity, max_episodes
+        self.owner = np.full(capacity, -1, np.int64)
+        self.head, self.n_added = 0, 0
+        self.episodes = []                   # (episode id, start slot, rows), oldest first
+
+    def add(self, rows):
+        eid, start = self.n_added, self.head
+        self.n_added += 1
+        self.owner[(start + np.arange(rows)) % self.cap] = eid
+        self.head = (start + rows) % self.cap
+        self.episodes = [(e, s, r) for e, s, r in self.episodes + [(eid, start, rows)]
+                         if (self.owner[(s + np.arange(r)) % self.cap] == e).all()]
+        return eid
+
+    def resident(self):
+        return [(s, r) for _, s, r in self.episodes]
+
+    def table(self, min_len):
+        return [(s, r - 1) for _, s, r in self.episodes if r - 1 >= min_len][-self.max_episodes:]
+
+
+def episode_content(eid, rows, A, frame_c=3):
+    """distinct per-(episode, row) frames / action / reward / discount for the ring tests; discounts hold zeros"""
+    t = np.arange(rows)
+    frames = ((eid * 131 + t.reshape(-1, 1, 1, 1) * 7 + np.arange(frame_c).reshape(1, -1, 1, 1) * 3 +
+               np.arange(84).reshape(1, 1, -1, 1) + 2 * np.arange(84).reshape(1, 1, 1, -1)) % 251).astype(np.uint8)
+    action = (eid * 1000 + t.reshape(-1, 1) * 10 + np.arange(A).reshape(1, -1)).astype(np.float32)
+    reward = (eid + t / 1024.0).astype(np.float32)
+    discount = np.where((eid + t) % 4 == 0, 0.0, 1.0 - t / 4096.0).astype(np.float32)
+    return frames, action, reward, discount
+
+
+def check_ring_holds(table, frames, action, reward, discount, contents, cap, what):
+    """every table entry (start, len) still holds, in slots [start, start + len + 1) mod cap, the frames / action /
+    reward / discount of the episode written there.  contents: {start slot: (frames, action, reward, discount)} of the
+    resident episodes"""
+    for s, ln in table:
+        want = contents.get(int(s))
+        assert want is not None, f"{what}: table entry at slot {s} is no resident episode"
+        rows = int(ln) + 1
+        assert want[0].shape[0] == rows, f"{what}: table entry at slot {s}: len {ln}, the episode has {want[0].shape[0]} rows"
+        slots = (int(s) + np.arange(rows)) % cap
+        for name, arr, w in (("frames", frames, want[0]), ("action", action, want[1]), ("reward", reward, want[2]),
+                             ("discount", discount, want[3])):
+            assert np.array_equal(arr[slots], w.reshape(arr[slots].shape)), \
+                f"{what}: {name} of the episode at slot {s} was overwritten"
+
+
+# the sequence of public calls whose keys test_gpu_draws.py reads back and test_draws_cpu.py models: two exploration
+# acts, an eval act, a step update() skips, updates (eager warm-up, graph capture + replay, replays), a batched
+# exploration act and the stage API's two noise draws
+AGENT_SCRIPT = ("act", "act", "act_eval", "update_skip", "update", "update", "update", "update", "act",
+                "stage_critic", "stage_actor")
