@@ -39,6 +39,7 @@ SIGNATURES = {
     "drq_conv3x3_fwd_f32": [P, P, P, P, I, I, I, P],
     "drq_conv3x3_dgrad_f32": [P, P, P, P, I, I, P],
     "drq_conv3x3_wgrad_f32": [P, P, P, P, P, I, I, P],
+    "drq_feature_grad_wide_f32": [P, P, P, I, P],
     "drq_pack_conv_w_bf16": [P, P, P, P],
     "drq_conv3x3_fwd_bf16": [P, P, P, P, I, I, I, L, I, I, P],
     "drq_conv3x3_dgrad_bf16": [P, P, P, I, P, I, I, P],

@@ -330,6 +330,28 @@ conv1_wgrad_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shif
     }
 }
 
+// ---------------------------------------------------------------- compact feature gradient -> conv4's wide dpre
+// One thread per wide position p < 37*41 of a plane: the ReLU-masked feature gradient inside 35 x 35, +0 at rows
+// 35-36 and columns 35-40 (what drq_conv3x3_dgrad_f32 reads at hout = 35 and requires to be zero).
+constexpr int kFeatHW = 35;
+constexpr int kFeatGradPos = (kFeatHW + 2) * kPW;   // 1517
+
+__global__ void __launch_bounds__(256)
+feature_grad_wide_kernel(const float* __restrict__ dfeat, const float* __restrict__ feat,
+                         float* __restrict__ dpre, long long total) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const long long plane = i / kFeatGradPos;           // n * 32 + c
+    const int p = (int)(i - plane * kFeatGradPos);
+    const int y = p / kPW, x = p - y * kPW;
+    float v = 0.f;
+    if (y < kFeatHW && x < kFeatHW) {
+        const long long k = plane * (kFeatHW * kFeatHW) + y * kFeatHW + x;   // c*1225 + y*35 + x of image n
+        v = __ldg(feat + k) > 0.f ? __ldg(dfeat + k) : 0.f;
+    }
+    dpre[plane * kPlane + p] = v;
+}
+
 template <typename K>
 static int set_smem(K kernel, size_t bytes, const char* what) {
     return ensure_smem(reinterpret_cast<const void*>(kernel), bytes, what);
@@ -411,6 +433,15 @@ int drq_conv3x3_wgrad_f32(const float* in, const float* dpre, float* partial, fl
     const int nw = kCh * kCh * 9;
     wgrad_reduce_kernel<<<(nw + kCh + 127) / 128, 128, 0, as_stream(stream)>>>(partial, G, nw, kCh, dw, db);
     return check_launch("wgrad_reduce_kernel");
+}
+
+int drq_feature_grad_wide_f32(const float* dfeat, const float* feat, float* dpre, int N, void* stream) {
+    DRQ_REQUIRE(dfeat && feat && dpre, "feature_grad_wide: null pointer");
+    DRQ_REQUIRE(N >= 0, "feature_grad_wide: bad dims");
+    if (N == 0) return DRQ_OK;
+    const long long total = (long long)N * kCh * kFeatGradPos;
+    feature_grad_wide_kernel<<<(unsigned)((total + 255) / 256), 256, 0, as_stream(stream)>>>(dfeat, feat, dpre, total);
+    return check_launch("feature_grad_wide_kernel");
 }
 
 }  // extern "C"

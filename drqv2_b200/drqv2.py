@@ -111,6 +111,215 @@ def _encoder_fwd(obs_u8, shift, w, b, acts, feat, N, cin, pad=4):
     call("drq_conv3x3_fwd_f32", acts[2], w[3], b[3], feat, N, 35, 1, s)
 
 
+# ----------------------------------------------------------------------------- autograd of the module API
+# Encoder / Actor / Critic built with differentiable=True record these Functions, so that the reference's own
+# update_critic / update_actor bodies (drqv2.py:177-228: loss.backward(); opt.step()) train through the library's
+# fp32 kernels.  The forwards launch exactly the kernels of the plain module forwards (bit-identical outputs) and keep
+# what the backward reads; each backward is the chain the fused fp32 update runs (_critic_pass, _actor_pass,
+# _encoder_bwd), fed by whatever gradient autograd has summed over every consumer of an output.
+def _grad_like(t, need):
+    return torch.empty_like(t) if need else None
+
+
+def _trunk_bwd(dh, B, Fd, feat, h, ld_h, xhat, rstd, gamma, W, need_feat, need_w, need_b, need_gamma, need_beta):
+    """Backward of Linear(39200->F) + LayerNorm + tanh from dh [B, F]: (dfeat, dW, db, dgamma, dbeta), None where not
+    needed.  The feature gradient dz @ W (39200 columns) runs only when the features need it."""
+    s = _stream()
+    dev = dh.device
+    dz = torch.empty(2 * B * Fd, device=dev)        # [dz | dy], drq_ln_tanh_bwd
+    dgamma, dbeta = torch.empty(Fd, device=dev), torch.empty(Fd, device=dev)
+    call("drq_ln_tanh_bwd", dh.data_ptr(), Fd, h.data_ptr(), ld_h, xhat.data_ptr(), rstd.data_ptr(), gamma.data_ptr(),
+         dz.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), None, 0, B, Fd, 1, 0, s)
+    dW, db = _grad_like(W, need_w), torch.empty(Fd, device=dev) if need_b else None
+    if need_w:
+        _linear_wgrad(dz.data_ptr(), Fd, feat.data_ptr(), REPR_DIM, dW.data_ptr(), B, Fd, REPR_DIM)
+    if need_b:
+        _colsum(dz.data_ptr(), Fd, db.data_ptr(), B, Fd)
+    dfeat = None
+    if need_feat:
+        dfeat = torch.empty(B, REPR_DIM, device=dev)
+        _linear_dgrad(dz.data_ptr(), Fd, W.data_ptr(), dfeat.data_ptr(), REPR_DIM, B, Fd, REPR_DIM)
+    return dfeat, dW, db, dgamma if need_gamma else None, dbeta if need_beta else None
+
+
+def _mlp_bwd(dy, B, n_in, H, n_out, x, ldx, h1, h2, ws, need):
+    """Backward of the 3-layer ReLU MLP (weights ws = (W1, b1, W2, b2, W3, b3)) from dy [B, n_out]: the six parameter
+    gradients (None where need[i] is False) and dh1, the gradient w.r.t. the first layer's pre-ReLU output, from which
+    the caller takes the input gradient over the column ranges it needs."""
+    dev = dy.device
+    W1, _, W2, _, W3, _ = ws
+    g = [_grad_like(w, n) for w, n in zip(ws, need)]
+    dh2, dh1 = torch.empty(B, H, device=dev), torch.empty(B, H, device=dev)
+    dyp, h1p, h2p = dy.data_ptr(), h1.data_ptr(), h2.data_ptr()
+    if need[4]:
+        _linear_wgrad(dyp, n_out, h2p, H, g[4].data_ptr(), B, n_out, H)
+    if need[5]:
+        _colsum(dyp, n_out, g[5].data_ptr(), B, n_out)
+    _linear_dgrad(dyp, n_out, W3.data_ptr(), dh2.data_ptr(), H, B, n_out, H, mask=h2p, ldmask=H)
+    if need[2]:
+        _linear_wgrad(dh2.data_ptr(), H, h1p, H, g[2].data_ptr(), B, H, H)
+    if need[3]:
+        _colsum(dh2.data_ptr(), H, g[3].data_ptr(), B, H)
+    _linear_dgrad(dh2.data_ptr(), H, W2.data_ptr(), dh1.data_ptr(), H, B, H, H, mask=h1p, ldmask=H)
+    if need[0]:
+        _linear_wgrad(dh1.data_ptr(), H, x.data_ptr(), ldx, g[0].data_ptr(), B, H, n_in)
+    if need[1]:
+        _colsum(dh1.data_ptr(), H, g[1].data_ptr(), B, H)
+    return g, dh1
+
+
+class _EncoderFn(torch.autograd.Function):
+    """features = Encoder(pixels) (drqv2.py:63-67) through drq_conv1_fwd_f32 / drq_conv3x3_fwd_f32; backward
+    drq_feature_grad_wide_f32 -> drq_conv3x3_{wgrad,dgrad}_f32 for conv4..2 -> drq_conv1_wgrad_f32 (no shift: the pixels
+    arrive augmented).  Inputs: u8 pixels, then (weight, bias) of conv1..4."""
+
+    @staticmethod
+    def forward(ctx, u8, *params):
+        n, cin = u8.shape[0], u8.shape[1]
+        dev = u8.device
+        # zeroed, not empty: drq_conv3x3_wgrad_f32 reads the whole plane of its input activation, slack included
+        acts = [torch.zeros(n * 32 * PLANE, device=dev) for _ in range(3)]
+        feat = torch.empty(n, REPR_DIM, device=dev)
+        _encoder_fwd(u8.data_ptr(), 0, [p.data_ptr() for p in params[0::2]], [p.data_ptr() for p in params[1::2]],
+                     [a.data_ptr() for a in acts], feat.data_ptr(), n, cin)
+        ctx.save_for_backward(u8, *acts, feat, *params[2::2])
+        return feat
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dfeat):
+        u8, a1, a2, a3, feat, w2, w3, w4 = ctx.saved_tensors
+        need = ctx.needs_input_grad[1:]
+        if not any(need):
+            return (None,) * 9
+        n, cin = u8.shape[0], u8.shape[1]
+        dev, s = feat.device, _stream()
+        dfeat = dfeat.float().contiguous()
+        acts, ws = (a1, a2, a3), (None, w2, w3, w4)
+        # d[l] = gradient w.r.t. conv(l+1)'s pre-ReLU output.  Zeroed: the data gradient leaves rows hout+2.. of its
+        # output alone and the next layer's data gradient reads two of them, which must be +0
+        d = [torch.zeros(n * 32 * PLANE, device=dev) for _ in range(4)]
+        wsp = torch.empty(int(_lib.lib().drq_conv_wgrad_ws_floats(32)), device=dev)    # cin <= 16 < 32
+        grads = [torch.empty(shape, device=dev) for shape in [(32, cin, 3, 3), (32,)] + [(32, 32, 3, 3), (32,)] * 3]
+        call("drq_feature_grad_wide_f32", dfeat.data_ptr(), feat.data_ptr(), d[3].data_ptr(), n, s)
+        for layer, hout in ((3, 35), (2, 37), (1, 39)):
+            call("drq_conv3x3_wgrad_f32", acts[layer - 1].data_ptr(), d[layer].data_ptr(), wsp.data_ptr(),
+                 grads[2 * layer].data_ptr(), grads[2 * layer + 1].data_ptr(), n, hout, s)
+            call("drq_conv3x3_dgrad_f32", d[layer].data_ptr(), ws[layer].data_ptr(), acts[layer - 1].data_ptr(),
+                 d[layer - 1].data_ptr(), n, hout, s)
+        call("drq_conv1_wgrad_f32", u8.data_ptr(), None, d[0].data_ptr(), wsp.data_ptr(), grads[0].data_ptr(),
+             grads[1].data_ptr(), n, cin, 4, s)
+        return (None,) + tuple(g if nd else None for g, nd in zip(grads, need))
+
+
+class _ActorFn(torch.autograd.Function):
+    """mu = tanh(policy(trunk(features))) (drqv2.py:85-89); backward drq_actor_sample_bwd (tanh'), the policy MLP's
+    weight / bias / masked data gradients and the trunk backward.  Inputs: features, trunk (W, b, gamma, beta), policy
+    (W1, b1, W2, b2, W3, b3)."""
+
+    @staticmethod
+    def forward(ctx, feat, tW, tb, gamma, beta, *pw):
+        B, dev = feat.shape[0], feat.device
+        Fd, H, A = tW.shape[0], pw[0].shape[0], pw[4].shape[0]
+        partial = torch.empty(_splitk_for(B) * B * Fd, device=dev)
+        h, xhat, rstd = torch.empty(B, Fd, device=dev), torch.empty(B, Fd, device=dev), torch.empty(B, device=dev)
+        _trunk_fwd(feat.data_ptr(), B, tW.data_ptr(), tb.data_ptr(), gamma.data_ptr(), beta.data_ptr(), Fd,
+                   partial.data_ptr(), h.data_ptr(), Fd, xhat.data_ptr(), rstd.data_ptr())
+        p1, p2, mu_pre = torch.empty(B, H, device=dev), torch.empty(B, H, device=dev), torch.empty(B, A, device=dev)
+        _linear_fwd(h.data_ptr(), Fd, pw[0].data_ptr(), pw[1].data_ptr(), p1.data_ptr(), H, B, H, Fd, True)
+        _linear_fwd(p1.data_ptr(), H, pw[2].data_ptr(), pw[3].data_ptr(), p2.data_ptr(), H, B, H, H, True)
+        _linear_fwd(p2.data_ptr(), H, pw[4].data_ptr(), pw[5].data_ptr(), mu_pre.data_ptr(), A, B, A, H, False)
+        mu = torch.empty(B, A, device=dev)
+        call("drq_actor_sample", mu_pre.data_ptr(), None, None, 0.0, mu.data_ptr(), A, None, None, B, A, _stream())
+        ctx.save_for_backward(feat, h, xhat, rstd, p1, p2, mu, tW, gamma, *pw)
+        return mu
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dmu):
+        feat, h, xhat, rstd, p1, p2, mu, tW, gamma, *pw = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        B, Fd, H, A = feat.shape[0], tW.shape[0], pw[0].shape[0], pw[4].shape[0]
+        dev = feat.device
+        dmu = dmu.float().contiguous()
+        dmu_pre = torch.empty(B, A, device=dev)
+        call("drq_actor_sample_bwd", dmu.data_ptr(), A, mu.data_ptr(), dmu_pre.data_ptr(), None, 0, B, A, 1, 0, _stream())
+        gp, dp1 = _mlp_bwd(dmu_pre, B, Fd, H, A, h, Fd, p1, p2, pw, need[5:])
+        gt = (None,) * 5
+        if any(need[:5]):
+            dh = torch.empty(B, Fd, device=dev)
+            _linear_dgrad(dp1.data_ptr(), H, pw[0].data_ptr(), dh.data_ptr(), Fd, B, H, Fd)
+            gt = _trunk_bwd(dh, B, Fd, feat, h, Fd, xhat, rstd, gamma, tW, *need[:5])
+        return (*gt, *gp)
+
+
+class _CriticFn(torch.autograd.Function):
+    """(Q1, Q2) = Critic(features, action) (drqv2.py:115-121); backward per Q head that received a gradient (a None
+    gradient skips its head): weight / bias / masked data gradients, then the gradients w.r.t. h and w.r.t. the action
+    from the first layer's two column ranges, then the trunk backward.  Inputs: features, action, trunk (W, b, gamma,
+    beta), Q1 (W1, b1, W2, b2, W3, b3), Q2 (the same)."""
+
+    @staticmethod
+    def forward(ctx, feat, action, tW, tb, gamma, beta, *qw):
+        ctx.set_materialize_grads(False)
+        B, dev = feat.shape[0], feat.device
+        Fd, H = tW.shape[0], qw[0].shape[0]
+        A = qw[0].shape[1] - Fd
+        partial = torch.empty(_splitk_for(B) * B * Fd, device=dev)
+        x, xhat, rstd = torch.empty(B, Fd + A, device=dev), torch.empty(B, Fd, device=dev), torch.empty(B, device=dev)
+        _trunk_fwd(feat.data_ptr(), B, tW.data_ptr(), tb.data_ptr(), gamma.data_ptr(), beta.data_ptr(), Fd,
+                   partial.data_ptr(), x.data_ptr(), Fd + A, xhat.data_ptr(), rstd.data_ptr())
+        call("drq_copy2d_f32", action.data_ptr(), A, x.data_ptr() + F32 * Fd, Fd + A, B, A, _stream())
+        qs, hidden = [], []
+        for z in range(2):
+            w = qw[6 * z:6 * z + 6]
+            q, h1, h2 = torch.empty(B, 1, device=dev), torch.empty(B, H, device=dev), torch.empty(B, H, device=dev)
+            _linear_fwd(x.data_ptr(), Fd + A, w[0].data_ptr(), w[1].data_ptr(), h1.data_ptr(), H, B, H, Fd + A, True)
+            _linear_fwd(h1.data_ptr(), H, w[2].data_ptr(), w[3].data_ptr(), h2.data_ptr(), H, B, H, H, True)
+            _linear_fwd(h2.data_ptr(), H, w[4].data_ptr(), w[5].data_ptr(), q.data_ptr(), 1, B, 1, H, False)
+            qs.append(q)
+            hidden += [h1, h2]
+        ctx.save_for_backward(feat, x, xhat, rstd, *hidden, tW, gamma, *qw)
+        return qs[0], qs[1]
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dq1, dq2):
+        feat, x, xhat, rstd, h1a, h2a, h1b, h2b, tW, gamma, *qw = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        B, Fd, H = feat.shape[0], tW.shape[0], qw[0].shape[0]
+        A = qw[0].shape[1] - Fd
+        dev = feat.device
+        if dq1 is None and dq2 is None:
+            return (None,) * 18
+        need_h = any(need[0:1] + need[2:6])
+        dh = torch.zeros(B, Fd, device=dev) if need_h else None
+        dact = torch.zeros(B, A, device=dev) if need[1] else None
+        gq = [None] * 12
+        for z, (dq, h1, h2) in enumerate(((dq1, h1a, h2a), (dq2, h1b, h2b))):
+            if dq is None:
+                continue
+            w = qw[6 * z:6 * z + 6]
+            dq = dq.float().contiguous()
+            gq[6 * z:6 * z + 6], dc1 = _mlp_bwd(dq, B, Fd + A, H, 1, x, Fd + A, h1, h2, w, need[6 + 6 * z:12 + 6 * z])
+            # d[h | action] = dc1 @ W1, over the two column ranges separately (each only when needed)
+            if need_h:
+                _linear_dgrad(dc1.data_ptr(), H, w[0].data_ptr(), dh.data_ptr(), Fd, B, H, Fd + A, n_cols=Fd, acc=1)
+            if need[1]:
+                _linear_dgrad(dc1.data_ptr(), H, w[0].data_ptr(), dact.data_ptr(), A, B, H, Fd + A, w_col0=Fd,
+                              n_cols=A, acc=1)
+        gt = (None,) * 5
+        if need_h:
+            gt = _trunk_bwd(dh, B, Fd, feat, x, Fd + A, xhat, rstd, gamma, tW, need[0], *need[2:6])
+        return (gt[0], dact, *gt[1:], *gq)
+
+
+def _wants_graph(module, *inputs):
+    """record a Function: the module was built differentiable, autograd records, and something needs a gradient"""
+    return (module.differentiable and torch.is_grad_enabled()
+            and any(t.requires_grad for t in (*inputs, *module.parameters())))
+
+
 # ----------------------------------------------------------------------------- modules
 class RandomShiftsAug(nn.Module):
     """Random translation by up to ±pad pixels after replicate padding, as the exact
@@ -146,9 +355,14 @@ def _as_u8_pixels(obs):
 
 
 class Encoder(nn.Module):
-    def __init__(self, obs_shape):
+    differentiable = False      # class default: instances pickled before the flag existed read it too
+
+    def __init__(self, obs_shape, *, differentiable=False):
+        """differentiable=True: forward records an autograd node (_EncoderFn) whenever autograd records and a parameter
+        requires grad, so that a loss on the features trains the convs; off (the default), outputs are plain tensors."""
         super().__init__()
         assert len(obs_shape) == 3
+        self.differentiable = bool(differentiable)
         self.repr_dim = 32 * 35 * 35
         chans = [int(obs_shape[0]), 32, 32, 32]
         mods = []
@@ -166,7 +380,12 @@ class Encoder(nn.Module):
         produced by RandomShiftsAug).  Returns features [N, 39200]."""
         _need_cuda(obs, "Encoder")
         _need_cuda(self.convnet[0].weight, "Encoder parameters")
+        if self.differentiable and torch.is_grad_enabled() and obs.requires_grad:
+            raise ValueError("Encoder(differentiable=True): the pixels require grad, but the integer-shift encoder has no "
+                             "gradient w.r.t. its input pixels; pass them detached")
         u8 = _as_u8_pixels(obs)
+        if _wants_graph(self):
+            return _EncoderFn.apply(u8, *self.parameters())
         n, cin = u8.shape[0], u8.shape[1]
         acts = [torch.empty(n * 32 * PLANE, device=u8.device) for _ in range(3)]
         feat = torch.empty(n, self.repr_dim, device=u8.device)
@@ -204,8 +423,13 @@ def _mlp_fwd(seq, x, ldx, B, n_in, hidden, n_out, out, dev):
 
 
 class Actor(nn.Module):
-    def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim):
+    differentiable = False      # class default: instances pickled before the flag existed read it too
+
+    def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim, *, differentiable=False):
+        """differentiable=True: the returned distribution's mean carries an autograd node (_ActorFn) whenever autograd
+        records and the features or a parameter require grad."""
         super().__init__()
+        self.differentiable = bool(differentiable)
         self.trunk = _Trunk(repr_dim, feature_dim)
         self.policy = _mlp(feature_dim, hidden_dim, action_shape[0])
         self.apply(utils.weight_init)
@@ -215,6 +439,9 @@ class Actor(nn.Module):
         B, dev = obs.shape[0], obs.device
         Fd, H, A = self.trunk[0].out_features, self.policy[0].out_features, self.policy[4].out_features
         obs = obs.float().contiguous()
+        if _wants_graph(self, obs):
+            mu = _ActorFn.apply(obs, *self.trunk[0].parameters(), *self.trunk[1].parameters(), *self.policy.parameters())
+            return utils.TruncatedNormal(mu, torch.ones_like(mu) * std)
         partial = torch.empty(_splitk_for(B) * B * Fd, device=dev)
         h = torch.empty(B, Fd, device=dev)
         t = self.trunk
@@ -229,8 +456,13 @@ class Actor(nn.Module):
 
 
 class Critic(nn.Module):
-    def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim):
+    differentiable = False      # class default: instances pickled before the flag existed read it too
+
+    def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim, *, differentiable=False):
+        """differentiable=True: Q1 and Q2 carry an autograd node (_CriticFn) whenever autograd records and the features,
+        the action or a parameter require grad."""
         super().__init__()
+        self.differentiable = bool(differentiable)
         self.trunk = _Trunk(repr_dim, feature_dim)
         self.Q1 = _mlp(feature_dim + action_shape[0], hidden_dim, 1)
         self.Q2 = _mlp(feature_dim + action_shape[0], hidden_dim, 1)
@@ -243,6 +475,9 @@ class Critic(nn.Module):
         A = self.Q1[0].in_features - Fd
         obs = obs.float().contiguous()
         action = action.float().contiguous()
+        if _wants_graph(self, obs, action):
+            return _CriticFn.apply(obs, action, *self.trunk[0].parameters(), *self.trunk[1].parameters(),
+                                   *self.Q1.parameters(), *self.Q2.parameters())
         partial = torch.empty(_splitk_for(B) * B * Fd, device=dev)
         x = torch.empty(B, Fd + A, device=dev)
         t = self.trunk
@@ -376,8 +611,9 @@ class _Workspace:
 
 class _Opt:
     """Stand-in for the reference's three torch.optim.Adam objects (drqv2.py:148-150):
-    the update itself is drq_adam_ema_step over the flat arena; this object only carries
-    hyper-parameters and the step count for inspection / pickling."""
+    the update itself is drq_adam_ema_step over the flat arena; this object carries the
+    hyper-parameters and the step count for inspection / pickling, and step() for code that
+    trains through autograd (DrQV2Agent(differentiable=True))."""
 
     def __init__(self, agent, net, lr):
         self._agent, self.net = agent, net
@@ -397,6 +633,31 @@ class _Opt:
         off, n, _ = self._agent._arena.seg[self.net]
         self._agent._arena.grads[off:off + n].zero_()
 
+    def step(self, closure=None):
+        """One torch.optim.Adam step of this network: drq_adam_step over its arena range, with this optimiser's own
+        step count and Adam scalars (fetched through the scalar ring in stream order, as the stage API does; the
+        exploration stddev act() reads is left as it was).  Unlike torch.optim.Adam, which skips a parameter whose
+        .grad is None, this steps every parameter of the network: the arena's gradients are never None (zero_grad
+        zeroes them).  The reference's update_critic / update_actor give every parameter they step a gradient, so
+        they see no difference.  In the tensor-core mode the bf16 operand copies are re-derived before the next
+        act() / update()."""
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        ag = self._agent
+        with torch.cuda.device(ag._dev):
+            ag._host_scalars(None, (self.net,))
+            ag._fetch_scalars()
+            ag._scalars_enqueued()
+            a = ag._arena
+            off, n = a.seg[self.net][0], a.seg[self.net][2]
+            call("drq_adam_step", a.params.data_ptr() + F32 * off, a.grads.data_ptr() + F32 * off,
+                 a.exp_avg.data_ptr() + F32 * off, a.exp_avg_sq.data_ptr() + F32 * off, n, ag._sc(self.net), _stream())
+            ag._opt_steps[self.net] += 1
+            ag._bf16_dirty = True
+        return loss
+
 
 METRIC_KEYS = ("batch_reward", "critic_target_q", "critic_q1", "critic_q2", "critic_loss",
                "actor_loss", "actor_logprob", "actor_ent")
@@ -405,7 +666,7 @@ METRIC_KEYS = ("batch_reward", "critic_target_q", "critic_q1", "critic_q2", "cri
 class DrQV2Agent:
     def __init__(self, obs_shape, action_shape, device, lr, feature_dim, hidden_dim, critic_target_tau,
                  num_expl_steps, update_every_steps, stddev_schedule, stddev_clip, use_tb,
-                 use_cuda_graph=True, seed=None, mode=None, data_parallel=False, prefetch=False):
+                 use_cuda_graph=True, seed=None, mode=None, data_parallel=False, prefetch=False, differentiable=False):
         """Reference signature (drqv2.py:125-127) plus three keyword-only extras: use_cuda_graph,
         seed (device RNG key) and mode — "fp32" (parity mode, CUDA-core kernels, <= 1e-4 vs the
         reference on pre-optimiser quantities) or "bf16" (tcgen05 tensor-core kernels, bf16
@@ -416,7 +677,14 @@ class DrQV2Agent:
         parameters are broadcast from rank 0 at construction (drqv2_b200/dist.py).
         prefetch=True: with a host-side replay iterator, pull the next batch at the end of every update and
         copy it to the device on a side stream while that update still runs (the reference's DataLoader
-        workers run ahead in the same way); the default keeps drqv2.py:236's one next() per update."""
+        workers run ahead in the same way); the default keeps drqv2.py:236's one next() per update.
+        differentiable=True: encoder, actor and critic record autograd nodes (Encoder / Actor / Critic above) and their
+        parameters require grad, so the reference's own update_critic / update_actor bodies (loss.backward();
+        opt.step()) train this agent: gradients land in the arena that encoder_opt / critic_opt / actor_opt.step() read
+        (INTEGRATION.md).  The fused update() is unaffected.  Not with data_parallel (those steps do not all-reduce)."""
+        if differentiable and data_parallel:
+            raise ValueError("DrQV2Agent: differentiable=True with data_parallel=True is not supported - the optimisers' "
+                             "step() does not average gradients over ranks")
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError(f"DrQV2Agent(device={device!r}): drqv2_b200 has no CPU path; use a CUDA device")
@@ -473,12 +741,18 @@ class DrQV2Agent:
             self._check_bf16_dims(dev)
 
         # models: built on the host in the reference's order (so a seed reproduces its init)
-        self.encoder = Encoder(self.obs_shape)
-        self.actor = Actor(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim)
-        self.critic = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim)
+        self.differentiable = bool(differentiable)
+        self.encoder = Encoder(self.obs_shape, differentiable=self.differentiable)
+        self.actor = Actor(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim, differentiable=self.differentiable)
+        self.critic = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim,
+                             differentiable=self.differentiable)
         self.critic_target = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim)
         self.critic_target.load_state_dict(self.critic.state_dict())
         self._to_device(dev)
+        if self.differentiable:
+            # .grad stays the arena view _Arena._adopt set: autograd adds into an existing .grad in place
+            for m in (self.encoder, self.actor, self.critic):
+                m.requires_grad_(True)
 
         self.encoder_opt = _Opt(self, "encoder", lr)
         self.actor_opt = _Opt(self, "actor", lr)
@@ -925,20 +1199,22 @@ class DrQV2Agent:
 
     def _host_scalars(self, step, stepping=("encoder", "critic", "actor")):
         """Adam scalars of the coming step of the optimisers in `stepping` (each with its own step count, as
-        torch.optim.Adam) and stddev(step) into the ring slot the device reads next."""
+        torch.optim.Adam) and stddev(step) into the ring slot the device reads next (step None: the stddev last
+        written, unchanged - an optimiser step on its own)."""
         half = self._SCAL_SLOTS // 2
         slot = self._scal_enq % self._SCAL_SLOTS
         if slot % half == 0:                       # entering a half of the ring: its previous readers must be done
             ev = self._scal_events[slot // half]
             if ev is not None:
                 ev.synchronize()
-        stddev = utils.schedule(self.stddev_schedule, step)
         for net in stepping:
             o = SCAL_OFF[net]
             self._scal_host[o:o + 8] = torch.from_numpy(utils.adam_scalars(self.lr, self._opt_steps[net] + 1))
-        self._scal_host[SCAL_OFF["stddev"]] = stddev
+        if step is not None:
+            stddev = utils.schedule(self.stddev_schedule, step)
+            self._scal_host[SCAL_OFF["stddev"]] = stddev
+            self._stddev = stddev
         self._scal_ring[slot].copy_(self._scal_host)
-        self._stddev = stddev
 
     def _fetch_scalars(self):
         """device side of _host_scalars: one tiny kernel, in stream order (graph-capturable)"""

@@ -264,6 +264,15 @@ int drq_conv3x3_wgrad_f32(const float* in, const float* dpre, float* partial, fl
                           float* db, int N, int hout, void* stream);
 int64_t drq_conv_wgrad_ws_floats(int cin);
 
+/* conv4's pre-ReLU gradient from an arbitrary gradient of the features (the backward of the autograd Encoder,
+ * drqv2.py:66-67: whatever losses consumed the features, their gradients already summed).  dfeat and feat are
+ * compact [N][39200] (c*1225 + y*35 + x; feat = conv4's post-ReLU output, the mask); dpre is wide [N][32][DRQ_PLANE]:
+ * dpre[n][c][y*41 + x] = feat > 0 ? dfeat : +0 inside 35 x 35, and +0 at rows 35-36 and at columns 35-40 of rows
+ * < 35.  Writes exactly positions [0, 37*41) of each plane - the set drq_conv3x3_dgrad_f32 reads at hout = 35, with
+ * the zeros it requires - and nothing else.  DRQ_EPI_MASK_WIDE does the same fused into the trunk's data-gradient
+ * GEMM, for one consumer and without the zero rows. */
+int drq_feature_grad_wide_f32(const float* dfeat, const float* feat, float* dpre, int N, void* stream);
+
 /* ------------------------------------------------------------------ encoder, bf16 tensor cores */
 
 /* bf16 elements of a WB buffer holding n_images images. */
