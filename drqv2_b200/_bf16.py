@@ -744,3 +744,389 @@ def act_body(agent, w, n, sample):
                          w["h"].data_ptr(), Fd, None, None, w["h_b"].ptr(), w["h_b"].units, 0)], n, Fd)
     actor_mlp_fwd(agent, w["h_b"], w["p1_b"], w["p2_b"], w["mu_pre"].data_ptr(), n, samples=[
         PolicySample(0, n, w["eps"].data_ptr() if sample else None, w["out"].data_ptr(), A, None, None, None, 0, 0, 0)])
+
+
+# ----------------------------------------------------------------------------- autograd on the tensor cores
+# Encoder / Actor / Critic built with differentiable="bf16" run their forwards on the kernels act() and update() run
+# (bf16 operands, fp32 accumulation) and, when autograd records, the tensor-core twins of drqv2.py's _EncoderFn,
+# _ActorFn and _CriticFn.  The module boundary carries fp32 tensors in the reference's layouts (features [N, 39200]
+# in the order c*1225 + y*35 + x, drqv2.py:66); drq_features_to_ref and drq_pack_features_tb convert at it.  Every
+# launch goes to the current stream.
+
+# rows drq_pack_features_tb and drq_features_to_ref take (DRQ_FEATURE_MAX_ROWS): the largest batch of every module
+MAX_BATCH = 65408
+
+
+def check_batch(n, what):
+    if not 1 <= n <= MAX_BATCH:
+        raise ValueError(f"{what}(differentiable='bf16'): batch {n} outside 1..{MAX_BATCH}, the rows the feature layout "
+                         "conversions take; differentiable=True has no such limit")
+
+
+def _wrap(buf, rows, feats, batch=1, rblk=TB_ACT):
+    """a TB around a saved buffer"""
+    tb = TB.__new__(TB)
+    tb.rows, tb.feats, tb.batch, tb.rblk = rows, feats, batch, rblk
+    tb.units = _ceil(feats, 16) // 8
+    tb.rpad = _ceil(rows, rblk)
+    tb.stride = tb.units * tb.rpad * 8
+    tb.buf = buf
+    return tb
+
+
+class Operands:
+    """The bf16 operand copies one module's forward and backward read: `conv1`, `wf`, `wd` (encoder), `trunk` /
+    `trunk_units` and `p0`, `p2`, `p4` (actor) or `q0`, `q2` with head z at entry z0 + z (critic)."""
+
+    def __init__(self, **kw):
+        self.__dict__.update(kw)
+
+
+def _param_key(module):
+    return tuple((p.data_ptr(), p._version) for p in module.parameters())
+
+
+def _own_operands(module, kind):
+    """Copies owned by a standalone module (drq_pack_multi of its parameters: the pack kinds the agent's copies use),
+    re-derived on first use, when a parameter was replaced or changed in place (its version counter moved), or after
+    refresh() / utils.soft_update_params marked them stale."""
+    key = _param_key(module)
+    ops = module.__dict__.get("_bf16_ops")
+    if ops is not None and ops.key == key and not module.__dict__.get("_bf16_stale", False):
+        return ops
+    dev = next(module.parameters()).device
+    zb = lambda n: torch.zeros(n, dtype=torch.bfloat16, device=dev)
+    if ops is None or ops.kind != kind or ops.dev != dev:
+        if kind == "encoder":
+            ops = Operands(conv1=zb(_lib.lib().drq_conv1_w_packed_elems()), wf=[zb(36 * 32 * 8) for _ in range(3)],
+                           wd=[zb(36 * 32 * 8) for _ in range(3)])
+        elif kind == "actor":
+            Fd, H, A = module.trunk[0].out_features, module.policy[0].out_features, module.policy[4].out_features
+            tr = TB(Fd, REPR_DIM, dev, rblk=TB_W)
+            ops = Operands(tr=tr, trunk=tr.ptr(), trunk_units=tr.units, p0=TB(H, Fd, dev, rblk=TB_W),
+                           p2=TB(H, H, dev, rblk=TB_W), p4=TB(A, H, dev, rblk=TB_W))
+        else:
+            Fd, H = module.trunk[0].out_features, module.Q1[0].out_features
+            A = module.Q1[0].in_features - Fd
+            tr = TB(Fd, REPR_DIM, dev, rblk=TB_W)
+            ops = Operands(tr=tr, trunk=tr.ptr(), trunk_units=tr.units, q0=TB(H, Fd + A, dev, batch=2, rblk=TB_W),
+                           q2=TB(H, H, dev, batch=2, rblk=TB_W), z0=0)
+        ops.kind, ops.dev = kind, dev
+    if kind == "encoder":
+        c = [module.convnet[i] for i in (0, 2, 4, 6)]
+        jobs = [PackJob(PACK_CONV1, 0, c[0].in_channels, 0, c[0].weight.data_ptr(), c[0].bias.data_ptr(),
+                        ops.conv1.data_ptr(), None)]
+        jobs += [PackJob(PACK_CONV, 0, 0, 0, c[i + 1].weight.data_ptr(), None, ops.wf[i].data_ptr(), ops.wd[i].data_ptr())
+                 for i in range(3)]
+    elif kind == "actor":
+        t, p = module.trunk[0], module.policy
+        jobs = [PackJob(PACK_TRUNK, t.out_features, REPR_DIM, 0, t.weight.data_ptr(), None, ops.trunk, None)]
+        jobs += [PackJob(PACK_LINEAR, p[i].out_features, p[i].in_features, 0, p[i].weight.data_ptr(), None, out.ptr(), None)
+                 for i, out in ((0, ops.p0), (2, ops.p2), (4, ops.p4))]
+    else:
+        t = module.trunk[0]
+        jobs = [PackJob(PACK_TRUNK, t.out_features, REPR_DIM, 0, t.weight.data_ptr(), None, ops.trunk, None)]
+        for z, q in enumerate((module.Q1, module.Q2)):
+            jobs += [PackJob(PACK_LINEAR, q[i].out_features, q[i].in_features, 0, q[i].weight.data_ptr(), None,
+                             out.ptr(z), None) for i, out in ((0, ops.q0), (2, ops.q2))]
+    pack_multi(jobs)
+    ops.key = key
+    module.__dict__["_bf16_ops"] = ops
+    module.__dict__["_bf16_stale"] = False
+    return ops
+
+
+def _agent_operands(agent, role):
+    """An agent's module reads the agent's own copies (Bf16State), which its optimiser steps, update() and the stage API
+    keep current; a parameter changed from outside (load_state_dict, an in-place edit) moves a version counter, and any
+    other change sets _bf16_dirty: either re-derives every copy first."""
+    keys = agent.__dict__.get("_bf16_keys")
+    if agent._bf16_dirty or keys is None or any(keys[r] != _param_key(getattr(agent, r)) for r in keys):
+        agent.refresh()
+    st = agent._bf16
+    if role == "encoder":
+        return Operands(conv1=st.conv1_w, wf=st.conv_wf, wd=st.conv_wd)
+    if role == "actor":
+        return Operands(trunk=st.trunk_ptr(st.ACTOR), trunk_units=st.trunk.units, p0=st.p0, p2=st.p2, p4=st.p4)
+    slot, z0 = (st.CRITIC, 0) if role == "critic" else (st.TARGET, 2)
+    return Operands(trunk=st.trunk_ptr(slot), trunk_units=st.trunk.units, q0=st.q0, q2=st.q2, z0=z0)
+
+
+def mark_stale(module):
+    owner = module.__dict__.get("_bf16_owner")
+    if owner is not None:
+        owner[0]._bf16_dirty = True
+    else:
+        module.__dict__["_bf16_stale"] = True
+
+
+def operands(module, kind):
+    owner = module.__dict__.get("_bf16_owner")
+    if owner is not None:
+        return _agent_operands(*owner)
+    return _own_operands(module, kind)
+
+
+def _zb(n, dev):
+    return torch.zeros(n, dtype=torch.bfloat16, device=dev)
+
+
+# ---- Encoder
+def encoder_forward(ops, u8, biases):
+    """conv1 (pixels arrive augmented: no shift, as act() runs it) .. conv4 into TB features, then fp32 features in
+    the reference order.  Returns (features, [conv1..3 WB activations])."""
+    n, cin = u8.shape[0], u8.shape[1]
+    dev, s = u8.device, _stream()
+    nel = _lib.lib().drq_wb_elems(n)
+    acts = [_zb(nel, dev) for _ in range(3)]     # zeroed: guard rows and the slack are read as zero padding
+    ft = TB(n, REPR_DIM, dev)
+    a = [t.data_ptr() for t in acts]
+    call("drq_conv1_fwd_bf16", u8.data_ptr(), None, ops.conv1.data_ptr(), a[0], n, cin, 4, s)
+    call("drq_conv3x3_fwd_bf16", a[0], ops.wf[0].data_ptr(), biases[0], a[1], n, 39, 0, 0, 0, 0, s)
+    call("drq_conv3x3_fwd_bf16", a[1], ops.wf[1].data_ptr(), biases[1], a[2], n, 37, 0, 0, 0, 0, s)
+    call("drq_conv3x3_fwd_bf16", a[2], ops.wf[2].data_ptr(), biases[2], ft.ptr(), n, 35, 2, ft.units, 0, 0, s)
+    feat = torch.empty(n, REPR_DIM, device=dev)
+    call("drq_features_to_ref", ft.ptr(), 1, feat.data_ptr(), n, s)
+    return feat, acts
+
+
+class EncoderFn(torch.autograd.Function):
+    """features = Encoder(pixels) on the tensor cores; backward drq_feature_grad_wide_bf16 -> conv4..2
+    drq_conv3x3_{wgrad (partials), dgrad}_bf16 -> drq_conv1_wgrad_bf16 -> one drq_conv_wgrad_reduce_multi.
+    Inputs: operand copies, u8 pixels, then (weight, bias) of conv1..4."""
+
+    @staticmethod
+    def forward(ctx, ops, u8, *params):
+        feat, acts = encoder_forward(ops, u8, [p.data_ptr() for p in params[3::2]])
+        ctx.ops = ops
+        ctx.save_for_backward(u8, *acts, feat)
+        return feat
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dfeat):
+        u8, a1, a2, a3, feat = ctx.saved_tensors
+        need = ctx.needs_input_grad[2:]
+        if not any(need):
+            return (None,) * 10
+        n, cin = u8.shape[0], u8.shape[1]
+        dev, s, L = feat.device, _stream(), _lib.lib()
+        dfeat = dfeat.float().contiguous()
+        nel = L.drq_wb_elems(n)
+        acts = [a1.data_ptr(), a2.data_ptr(), a3.data_ptr()]
+        # d[l]: gradient w.r.t. conv(l+1)'s pre-ReLU output.  d[3] is written whole by drq_feature_grad_wide_bf16; the
+        # data gradients write rows < hout + 2 of each image, the rest must stay zero
+        d = [_zb(nel, dev) for _ in range(3)] + [torch.empty(nel, dtype=torch.bfloat16, device=dev)]
+        dp = [t.data_ptr() for t in d]
+        ws = [torch.zeros(L.drq_conv1_wgrad_bf16_ws_floats(), device=dev)] + \
+             [torch.zeros(L.drq_conv_wgrad_bf16_ws_floats(), device=dev) for _ in range(3)]
+        grads = [torch.empty(shape, device=dev) for shape in [(32, cin, 3, 3), (32,)] + [(32, 32, 3, 3), (32,)] * 3]
+        call("drq_feature_grad_wide_bf16", dfeat.data_ptr(), feat.data_ptr(), dp[3], n, s)
+        jobs = []
+        for layer, hout in ((3, 35), (2, 37), (1, 39)):
+            call("drq_conv3x3_wgrad_bf16", acts[layer - 1], n, dp[layer], ws[layer].data_ptr(), None, None, n, hout, s)
+            jobs.append(WgReduceJob(ws[layer].data_ptr(), grads[2 * layer].data_ptr(), grads[2 * layer + 1].data_ptr(),
+                                    n, hout, 0, 0))
+            call("drq_conv3x3_dgrad_bf16", dp[layer], ctx.ops.wd[layer - 1].data_ptr(), acts[layer - 1], n, dp[layer - 1],
+                 n, hout, s)
+        call("drq_conv1_wgrad_bf16", u8.data_ptr(), None, dp[0], ws[0].data_ptr(), None, None, n, cin, 4, s)
+        jobs.append(WgReduceJob(ws[0].data_ptr(), grads[0].data_ptr(), grads[1].data_ptr(), n, 0, cin, 0))
+        call("drq_conv_wgrad_reduce_multi", (WgReduceJob * len(jobs))(*jobs), len(jobs), s)
+        return (None, None) + tuple(g if nd else None for g, nd in zip(grads, need))
+
+
+# ---- heads: the trunk (Linear(39200 -> F) + LayerNorm + tanh) shared by Actor and Critic
+def _trunk_forward(ops, feat, Fd, tb, gamma, beta, h_ld, tail=None, A=0):
+    """pack the fp32 features, the split-K trunk GEMM with act()'s split rule, the LayerNorm tail.  Returns
+    (feature TB, h fp32 [B, h_ld], xhat, rstd, bf16 h TB of Fd + A features (the action appended when tail))."""
+    B, dev, s = feat.shape[0], feat.device, _stream()
+    ft = TB(B, REPR_DIM, dev)
+    call("drq_pack_features_tb", feat.data_ptr(), ft.ptr(), B, s)
+    FP = _ceil(Fd, TB_W)
+    S = splitk_for((ft.rpad // TB_ACT) * (FP // 64))
+    part = torch.empty(S * B * FP, device=dev)
+    gemm(ft.ptr(), ft.units, ops.trunk, ops.trunk_units, GEMM_KK, part.data_ptr(), FP, B, FP, REPR_DIM, TEPI_F32,
+         splitk=S, strides=_strides(split=B * FP))
+    h, xhat, rstd = torch.empty(B, Fd, device=dev), torch.empty(B, Fd, device=dev), torch.empty(B, device=dev)
+    hb = TB(B, Fd + A, dev)
+    ln_tanh_multi([LnJob(part.data_ptr(), FP, B * FP, S, tb, gamma, beta, h.data_ptr(), Fd, xhat.data_ptr(),
+                         rstd.data_ptr(), hb.buf.data_ptr(), hb.units, 0, tail, A, A if tail else 0)], B, Fd)
+    return ft, h, xhat, rstd, hb
+
+
+def _trunk_backward(ops, dh_planes, ld, n_planes, plane_stride, B, Fd, ft, h, xhat, rstd, gamma, need_feat, jobs, gp):
+    """tanh / LayerNorm backward from dh (n_planes summed on the fly), the trunk weight gradient (reference column
+    order) and, when need_feat, the feature gradient in the reference order.  gp = (dW, db, dgamma, dbeta): db / dgamma
+    / dbeta join the caller's colsum jobs.  Returns dfeat or None."""
+    dev, s = h.device, _stream()
+    dz = torch.empty(2 * B * Fd, device=dev)        # [dz | dy]
+    zt = TB(B, Fd, dev)
+    call("drq_ln_tanh_bwd", dh_planes, ld, h.data_ptr(), Fd, xhat.data_ptr(), rstd.data_ptr(), gamma, dz.data_ptr(),
+         None, None, zt.ptr(), zt.units, B, Fd, n_planes, plane_stride, s)
+    gemm(zt.ptr(), zt.units, ft.ptr(), ft.units, GEMM_MNMN, gp[0].data_ptr(), REPR_DIM, Fd, REPR_DIM, B, TEPI_TRUNK_WGRAD,
+         bn=128)
+    dy = dz.data_ptr() + F32 * B * Fd
+    jobs += [ColsumJob(dz.data_ptr(), Fd, gp[1].data_ptr(), B, Fd, 0, 0),
+             ColsumJob(dy, Fd, gp[2].data_ptr(), B, Fd, 0, 0, xhat.data_ptr()),
+             ColsumJob(dy, Fd, gp[3].data_ptr(), B, Fd, 0, 0)]
+    colsum_multi(jobs)
+    if not need_feat:
+        return None
+    de = torch.empty(B, REPR_DIM, device=dev)       # encoder-output order
+    gemm(zt.ptr(), zt.units, ops.trunk, ops.trunk_units, GEMM_KMN, de.data_ptr(), REPR_DIM, B, REPR_DIM, Fd, TEPI_F32)
+    dfeat = torch.empty(B, REPR_DIM, device=dev)
+    call("drq_features_to_ref", de.data_ptr(), 0, dfeat.data_ptr(), B, s)
+    return dfeat
+
+
+# ---- Actor
+def actor_forward(ops, feat, tw):
+    """mu = tanh(policy(trunk(features))) (drqv2.py:85-89) as act() computes it in eval mode.  tw: the Actor's
+    (trunk.0 W, b, LayerNorm gamma, beta, policy W1, b1, W2, b2, W3, b3) tensors.  Returns (mu, saved)."""
+    B, dev, s = feat.shape[0], feat.device, _stream()
+    Fd, H, A = tw[0].shape[0], tw[4].shape[0], tw[8].shape[0]
+    ft, h, xhat, rstd, hb = _trunk_forward(ops, feat, Fd, tw[1].data_ptr(), tw[2].data_ptr(), tw[3].data_ptr(), Fd)
+    p1, p2 = TB(B, H, dev), TB(B, H, dev)
+    gemm(hb.ptr(), hb.units, ops.p0.ptr(), ops.p0.units, GEMM_KK, p1.ptr(), p1.units, B, H, Fd, TEPI_RELU_BF16,
+         bias=tw[5].data_ptr())
+    gemm(p1.ptr(), p1.units, ops.p2.ptr(), ops.p2.units, GEMM_KK, p2.ptr(), p2.units, B, H, H, TEPI_RELU_BF16,
+         bias=tw[7].data_ptr())
+    mu_pre, mu = torch.empty(B, A, device=dev), torch.empty(B, A, device=dev)
+    job = PolicySample(0, B, None, mu.data_ptr(), A, None, None, None, 0, 0, 0)
+    call("drq_policy_head_fwd_bf16", p2.ptr(), p2.units, tw[8].data_ptr(), tw[9].data_ptr(), mu_pre.data_ptr(), B, H, A,
+         (PolicySample * 1)(job), 1, None, 0.0, None, s)
+    return mu, (ft.buf, h, xhat, rstd, hb.buf, p1.buf, p2.buf, mu)
+
+
+class ActorFn(torch.autograd.Function):
+    """mu on the tensor cores; backward drq_actor_sample_bwd, the policy MLP's MNMN (weight) / KMN (data) GEMMs, the
+    trunk backward and one drq_colsum_multi for every bias, LayerNorm affine included.  Inputs: operand copies,
+    features, trunk (W, b, gamma, beta), policy (W1, b1, W2, b2, W3, b3)."""
+
+    @staticmethod
+    def forward(ctx, ops, feat, *tw):
+        mu, saved = actor_forward(ops, feat, tw)
+        ctx.ops = ops
+        ctx.save_for_backward(*saved, tw[2])
+        return mu
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dmu):
+        ftb, h, xhat, rstd, hbb, p1b, p2b, mu, gamma = ctx.saved_tensors
+        need = ctx.needs_input_grad[1:]
+        if not any(need):
+            return (None,) * 12
+        ops, s = ctx.ops, _stream()
+        B, A = mu.shape
+        Fd, H, dev = h.shape[1], ops.p0.rows, h.device
+        ft, hb = _wrap(ftb, B, REPR_DIM), _wrap(hbb, B, Fd)
+        p1, p2 = _wrap(p1b, B, H), _wrap(p2b, B, H)
+        U = p1.units
+        dmu = dmu.float().contiguous()
+        dmu_pre, dmt = torch.empty(B, A, device=dev), TB(B, A, dev)
+        call("drq_actor_sample_bwd", dmu.data_ptr(), A, mu.data_ptr(), dmu_pre.data_ptr(), dmt.ptr(), dmt.units, B, A, 1,
+             0, s)
+        g = [torch.empty(shape, device=dev) for shape in ((Fd, REPR_DIM), (Fd,), (Fd,), (Fd,), (H, Fd), (H,), (H, H), (H,),
+                                                         (A, H), (A,))]
+        dp1, dp2 = TB(B, H, dev), TB(B, H, dev)
+        gemm(dmt.ptr(), dmt.units, p2.ptr(), U, GEMM_MNMN, g[8].data_ptr(), H, A, H, B, TEPI_F32, bn=128)
+        gemm(dmt.ptr(), dmt.units, ops.p4.ptr(), ops.p4.units, GEMM_KMN, dp2.ptr(), U, B, H, A, TEPI_MASK_BF16,
+             mask=p2.ptr(), units_mask=U)
+        gemm(dp2.ptr(), U, p1.ptr(), U, GEMM_MNMN, g[6].data_ptr(), H, H, H, B, TEPI_F32, bn=128)
+        gemm(dp2.ptr(), U, ops.p2.ptr(), ops.p2.units, GEMM_KMN, dp1.ptr(), U, B, H, H, TEPI_MASK_BF16, mask=p1.ptr(),
+             units_mask=U)
+        gemm(dp1.ptr(), U, hb.ptr(), hb.units, GEMM_MNMN, g[4].data_ptr(), Fd, H, Fd, B, TEPI_F32)
+        dh = torch.empty(B, Fd, device=dev)
+        gemm(dp1.ptr(), U, ops.p0.ptr(), ops.p0.units, GEMM_KMN, dh.data_ptr(), Fd, B, Fd, H, TEPI_F32)
+        jobs = [ColsumJob(dmu_pre.data_ptr(), A, g[9].data_ptr(), B, A, 0, 0),
+                ColsumJob(dp2.ptr(), U, g[7].data_ptr(), B, H, 1, 0), ColsumJob(dp1.ptr(), U, g[5].data_ptr(), B, H, 1, 0)]
+        dfeat = _trunk_backward(ops, dh.data_ptr(), Fd, 1, 0, B, Fd, ft, h, xhat, rstd, gamma.data_ptr(), need[0], jobs,
+                                g[:4])
+        return (None, dfeat) + tuple(t if nd else None for t, nd in zip(g, need[1:]))
+
+
+# ---- Critic
+def critic_forward(ops, feat, action, cw):
+    """(Q1, Q2) = Critic(features, action) (drqv2.py:115-121).  cw: trunk (W, b, gamma, beta), Q1 (W1, b1, W2, b2, W3,
+    b3), Q2 (the same).  One launch per layer and head.  Returns (q1, q2, saved)."""
+    B, dev, s = feat.shape[0], feat.device, _stream()
+    Fd, H = cw[0].shape[0], cw[4].shape[0]
+    A = cw[4].shape[1] - Fd
+    ft, h, xhat, rstd, xb = _trunk_forward(ops, feat, Fd, cw[1].data_ptr(), cw[2].data_ptr(), cw[3].data_ptr(), Fd,
+                                           tail=action.data_ptr(), A=A)
+    c1, c2 = TB(B, H, dev, batch=2), TB(B, H, dev, batch=2)
+    qs = []
+    for z in range(2):
+        w = cw[4 + 6 * z:10 + 6 * z]
+        gemm(xb.ptr(), xb.units, ops.q0.ptr(ops.z0 + z), ops.q0.units, GEMM_KK, c1.ptr(z), c1.units, B, H, Fd + A,
+             TEPI_RELU_BF16, bias=w[1].data_ptr())
+        gemm(c1.ptr(z), c1.units, ops.q2.ptr(ops.z0 + z), ops.q2.units, GEMM_KK, c2.ptr(z), c2.units, B, H, H,
+             TEPI_RELU_BF16, bias=w[3].data_ptr())
+        q = torch.empty(B, 1, device=dev)
+        call("drq_q_head_fwd_bf16", c2.ptr(z), c2.units, c2.stride, w[4].data_ptr(), w[5].data_ptr(), q.data_ptr(), B, H,
+             1, 0, 1, 0, s)
+        qs.append(q)
+    return qs[0], qs[1], (ft.buf, xb.buf, h, xhat, rstd, c1.buf, c2.buf)
+
+
+class CriticFn(torch.autograd.Function):
+    """(Q1, Q2) on the tensor cores; backward per head that received a gradient (a None gradient skips its head):
+    drq_q_head_bwd_bf16, the Q MLP's weight / masked data GEMMs, the first layer's data gradient as split-K planes
+    [head][split], drq_plane_sum_f32 over their action columns, and the trunk backward (drq_ln_tanh_bwd sums the
+    same planes' h columns).  Inputs: operand copies, features, action, trunk (W, b, gamma, beta), Q1 and Q2 (W1, b1,
+    W2, b2, W3, b3 each)."""
+
+    @staticmethod
+    def forward(ctx, ops, feat, action, *cw):
+        ctx.set_materialize_grads(False)
+        q1, q2, saved = critic_forward(ops, feat, action, cw)
+        ctx.ops = ops
+        ctx.save_for_backward(*saved, cw[2], cw[8], cw[14])
+        return q1, q2
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dq1, dq2):
+        ftb, xbb, h, xhat, rstd, c1b, c2b, gamma, w3a, w3b = ctx.saved_tensors
+        need = ctx.needs_input_grad[1:]
+        if (dq1 is None and dq2 is None) or not any(need):
+            return (None,) * 19
+        ops, s = ctx.ops, _stream()
+        B, Fd = h.shape
+        H = ops.q2.rows
+        A = ops.q0.feats - Fd
+        dev = h.device
+        ft, xb = _wrap(ftb, B, REPR_DIM), _wrap(xbb, B, Fd + A)
+        c1, c2 = _wrap(c1b, B, H, batch=2), _wrap(c2b, B, H, batch=2)
+        U, K1 = c1.units, Fd + A
+        heads = [z for z, dq in enumerate((dq1, dq2)) if dq is not None]
+        SX = 8 if H % 1024 == 0 else 1                 # the fused update's split of this K = H contraction
+        PS = B * K1
+        dxf = torch.empty(len(heads) * SX, B, K1, device=dev)    # planes [head][split]
+        dc1, dc2 = TB(B, H, dev, batch=2), TB(B, H, dev, batch=2)
+        gq = [None] * 12
+        jobs = []
+        for i, z in enumerate(heads):
+            dq = (dq1, dq2)[z].float().contiguous()
+            g = [torch.empty(shape, device=dev) for shape in ((H, K1), (H,), (H, H), (H,), (1, H), (1,))]
+            call("drq_q_head_bwd_bf16", dq.data_ptr(), None, c2.ptr(z), U, c2.stride, (w3a, w3b)[z].data_ptr(), dc2.ptr(z),
+                 g[4].data_ptr(), g[5].data_ptr(), B, H, 0, s)
+            gemm(dc2.ptr(z), U, c1.ptr(z), U, GEMM_MNMN, g[2].data_ptr(), H, H, H, B, TEPI_F32, bn=128)
+            gemm(dc2.ptr(z), U, ops.q2.ptr(ops.z0 + z), ops.q2.units, GEMM_KMN, dc1.ptr(z), U, B, H, H, TEPI_MASK_BF16,
+                 mask=c1.ptr(z), units_mask=U)
+            gemm(dc1.ptr(z), U, xb.ptr(), xb.units, GEMM_MNMN, g[0].data_ptr(), K1, H, K1, B, TEPI_F32)
+            gemm(dc1.ptr(z), U, ops.q0.ptr(ops.z0 + z), ops.q0.units, GEMM_KMN, dxf[i * SX].data_ptr(), K1, B, K1, H,
+                 TEPI_F32, splitk=SX, strides=_strides(split=PS))
+            jobs += [ColsumJob(dc2.ptr(z), U, g[3].data_ptr(), B, H, 1, 0), ColsumJob(dc1.ptr(z), U, g[1].data_ptr(), B, H, 1, 0)]
+            gq[6 * z:6 * z + 6] = g
+        planes = len(heads) * SX
+        dact = None
+        if need[1]:
+            dact = torch.empty(B, A, device=dev)
+            call("drq_plane_sum_f32", dxf.data_ptr() + F32 * Fd, K1, PS, planes, dact.data_ptr(), A, B, A, s)
+        gt = [torch.empty(shape, device=dev) for shape in ((Fd, REPR_DIM), (Fd,), (Fd,), (Fd,))]
+        dfeat = _trunk_backward(ops, dxf.data_ptr(), K1, planes, PS, B, Fd, ft, h, xhat, rstd, gamma.data_ptr(), need[0],
+                                jobs, gt)
+        grads = gt + gq
+        return (None, dfeat, dact) + tuple(t if nd else None for t, nd in zip(grads, need[2:]))

@@ -73,6 +73,10 @@ SIGNATURES = {
     "drq_actor_sample_bwd": [P, L, P, P, P, L, I, I, I, L, P],
     "drq_q_head_fwd_bf16": [P, L, L, P, P, P, I, I, I, L, I, L, P],
     "drq_q_head_bwd_loss_bf16": [I, P, P, P, P, P, P, P, L, L, P, P, P, P, I, I, L, P],
+    "drq_q_head_bwd_bf16": [P, P, P, L, L, P, P, P, P, I, I, L, P],
+    "drq_features_to_ref": [P, I, P, I, P],
+    "drq_feature_grad_wide_bf16": [P, P, P, I, P],
+    "drq_plane_sum_f32": [P, L, L, I, P, L, I, I, P],
     "drq_critic_loss": [P, P, P, P, P, P, P, P, P, P, I, P],
     "drq_actor_loss": [P, P, P, P, P, I, P],
     "drq_copy2d_f32": [P, L, P, L, I, I, P],

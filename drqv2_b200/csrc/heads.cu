@@ -456,7 +456,7 @@ q_head_fwd_kernel(const __nv_bfloat16* __restrict__ c2, long long rpad, long lon
 
 // dc2[z][b][k] = dq[z][b] * w3[z][k] * (c2 > 0) (TB bf16); optionally dw3[z][k] = sum_b dq[z][b] c2[z][b][k]
 // and db3[z] = sum_b dq[z][b].  One block per 8-feature unit; fixed-order tree.
-// LOSS selects where dq comes from: 0 = given; 1 = the critic loss of drqv2.py:185-189 computed here from
+// LOSS selects where dq comes from: 0 = given (head z reads dq1 / dq2); 1 = the critic loss of drqv2.py:185-189 computed here from
 // (q, target q, reward, discount) - block (0,0) also writes the five metrics; 2 = the actor loss of
 // drqv2.py:213-216 (-mean(min(Q1,Q2))), block (0,0) writes actor_loss.  Heads = 2 for LOSS != 0.
 struct QLossArgs {
@@ -483,12 +483,13 @@ __device__ __forceinline__ float loss_dq(const QLossArgs& L, const float* dqz, i
 
 template <int LOSS>
 __global__ void __launch_bounds__(256)
-q_head_bwd_kernel(const float* __restrict__ dq, const QLossArgs L, const __nv_bfloat16* __restrict__ c2, long long rpad,
+q_head_bwd_kernel(const float* __restrict__ dq1, const float* __restrict__ dq2, const QLossArgs L,
+                  const __nv_bfloat16* __restrict__ c2, long long rpad,
                   long long bs_c2, const float* __restrict__ w3, __nv_bfloat16* __restrict__ dc2,
                   float* __restrict__ dw3, float* __restrict__ db3, int B, long long w_stride) {
     __shared__ float red[256][9];
     const int u = blockIdx.x, z = blockIdx.y;
-    const float* dqz = LOSS == 0 ? dq + (long long)z * B : nullptr;
+    const float* dqz = LOSS == 0 ? (z ? dq2 : dq1) : nullptr;
     const long long base = z * bs_c2;
     float w[8];
 #pragma unroll
@@ -700,11 +701,31 @@ int drq_q_head_bwd_loss_bf16(int loss, const float* q, const float* tq, const fl
     const auto c2p = reinterpret_cast<const __nv_bfloat16*>(c2);
     const auto dp = reinterpret_cast<__nv_bfloat16*>(dc2);
     if (loss == 1)
-        q_head_bwd_kernel<1><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
+        q_head_bwd_kernel<1><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
                  B, w_stride);
     else
-        q_head_bwd_kernel<2><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
+        q_head_bwd_kernel<2><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(nullptr, nullptr, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
                  B, w_stride);
+    return check_launch("q_head_bwd_kernel");
+}
+
+int drq_q_head_bwd_bf16(const float* dq1, const float* dq2, const uint16_t* c2, int64_t rpad, int64_t bs_c2,
+                        const float* w3, uint16_t* dc2, float* dw3, float* db3, int B, int H, int64_t w_stride,
+                        void* stream) {
+    DRQ_REQUIRE(c2 && w3 && dc2 && B > 0 && H > 0 && H % 8 == 0, "q_head_bwd: bad args");
+    if (!dq1 && !dq2) return DRQ_OK;
+    const QLossArgs L{};
+    const auto c2p = reinterpret_cast<const __nv_bfloat16*>(c2);
+    auto dp = reinterpret_cast<__nv_bfloat16*>(dc2);
+    if (dq1 && dq2) {
+        q_head_bwd_kernel<0><<<dim3(H / 8, 2), 256, 0, as_stream(stream)>>>(dq1, dq2, L, c2p, rpad, bs_c2, w3, dp, dw3, db3,
+                 B, w_stride);
+    } else {
+        // one head: its operands moved to z = 0
+        const long long zc = dq1 ? 0 : bs_c2, zw = dq1 ? 0 : w_stride;
+        q_head_bwd_kernel<0><<<dim3(H / 8, 1), 256, 0, as_stream(stream)>>>(dq1 ? dq1 : dq2, nullptr, L, c2p + zc, rpad, bs_c2,
+                 w3 + zw, dp + zc, dw3 ? dw3 + zw : nullptr, db3 ? db3 + zw : nullptr, B, w_stride);
+    }
     return check_launch("q_head_bwd_kernel");
 }
 

@@ -314,6 +314,49 @@ class _CriticFn(torch.autograd.Function):
         return (gt[0], dact, *gt[1:], *gq)
 
 
+def _flag(differentiable, what):
+    """the differentiable= value as stored: False, True or "bf16" (True and "bf16" stay distinct)"""
+    if isinstance(differentiable, str):
+        if differentiable != "bf16":
+            raise ValueError(f"{what}: differentiable must be False, True or 'bf16', got {differentiable!r}")
+        return differentiable
+    if differentiable not in (False, True):
+        raise ValueError(f"{what}: differentiable must be False, True or 'bf16', got {differentiable!r}")
+    return bool(differentiable)
+
+
+def _check_bf16_dims(A, H, Fd, dev=None):
+    """Refuse at construction the head shapes the tensor-core kernels refuse (csrc/heads.cu), which would otherwise
+    fail at the first act(), update() or forward.  dev None: the current device, when there is one (the shared-memory
+    bound needs its properties)."""
+    if not 1 <= A <= _lib.POLICY_MAX_A:
+        raise ValueError(f"action_shape ({A},): mode='bf16' supports 1 <= A <= {_lib.POLICY_MAX_A} action dimensions "
+                         "(the policy head kernel); mode='fp32' and differentiable=True have no such limit")
+    if H % 8:
+        raise ValueError(f"hidden_dim {H}: mode='bf16' needs a multiple of 8 (16-byte rows of the bf16 operands); "
+                         "mode='fp32' and differentiable=True have no such limit")
+    if not 1 <= Fd <= _lib.LN_MAX_F:
+        raise ValueError(f"feature_dim {Fd}: the LayerNorm kernels hold 1 <= F <= {_lib.LN_MAX_F} features "
+                         "(differentiable=True as well)")
+    if dev is None:
+        if not torch.cuda.is_available():
+            return
+        dev = torch.device("cuda", torch.cuda.current_device())
+    groups = -(-A // _lib.POLICY_GROUP)
+    slab = 4 * H * -(-A // groups)                 # fp32 weights of one policy-head block's action group
+    optin = torch.cuda.get_device_properties(dev).shared_memory_per_block_optin
+    if slab + _lib.POLICY_STATIC_SMEM > optin:
+        raise ValueError(f"hidden_dim {H} with {A} actions: mode='bf16' stages {slab} bytes of policy-head weights per "
+                         f"block, more than the {optin - _lib.POLICY_STATIC_SMEM} bytes of shared memory a block can "
+                         "have here; mode='fp32' and differentiable=True have no such limit")
+
+
+def _refresh_bf16(self):
+    """differentiable="bf16": re-derive the bf16 operand copies before the next forward - after a change of the
+    parameters their version counters do not show (writes through .data or raw pointers)."""
+    _bf16.mark_stale(self)
+
+
 def _wants_graph(module, *inputs):
     """record a Function: the module was built differentiable, autograd records, and something needs a gradient"""
     return (module.differentiable and torch.is_grad_enabled()
@@ -356,13 +399,19 @@ def _as_u8_pixels(obs):
 
 class Encoder(nn.Module):
     differentiable = False      # class default: instances pickled before the flag existed read it too
+    refresh = _refresh_bf16
 
     def __init__(self, obs_shape, *, differentiable=False):
         """differentiable=True: forward records an autograd node (_EncoderFn) whenever autograd records and a parameter
-        requires grad, so that a loss on the features trains the convs; off (the default), outputs are plain tensors."""
+        requires grad, so that a loss on the features trains the convs; off (the default), outputs are plain tensors.
+        differentiable="bf16": the same on the tensor-core kernels (bf16 operands, fp32 accumulation; _bf16.EncoderFn),
+        under no_grad too; up to 10 input channels."""
         super().__init__()
         assert len(obs_shape) == 3
-        self.differentiable = bool(differentiable)
+        self.differentiable = _flag(differentiable, "Encoder")
+        if self.differentiable == "bf16" and int(obs_shape[0]) * 9 + 1 > 96:
+            raise ValueError(f"Encoder(differentiable='bf16'): {int(obs_shape[0])} input channels; the tensor-core conv1 "
+                             "takes cin * 9 + 1 <= 96, at most 10 channels (differentiable=True takes up to 16)")
         self.repr_dim = 32 * 35 * 35
         chans = [int(obs_shape[0]), 32, 32, 32]
         mods = []
@@ -384,6 +433,12 @@ class Encoder(nn.Module):
             raise ValueError("Encoder(differentiable=True): the pixels require grad, but the integer-shift encoder has no "
                              "gradient w.r.t. its input pixels; pass them detached")
         u8 = _as_u8_pixels(obs)
+        if self.differentiable == "bf16":
+            _bf16.check_batch(u8.shape[0], "Encoder")
+            ops = _bf16.operands(self, "encoder")
+            if _wants_graph(self):
+                return _bf16.EncoderFn.apply(ops, u8, *self.parameters())
+            return _bf16.encoder_forward(ops, u8, [self.convnet[i].bias.data_ptr() for i in (2, 4, 6)])[0]
         if _wants_graph(self):
             return _EncoderFn.apply(u8, *self.parameters())
         n, cin = u8.shape[0], u8.shape[1]
@@ -424,12 +479,16 @@ def _mlp_fwd(seq, x, ldx, B, n_in, hidden, n_out, out, dev):
 
 class Actor(nn.Module):
     differentiable = False      # class default: instances pickled before the flag existed read it too
+    refresh = _refresh_bf16
 
     def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim, *, differentiable=False):
         """differentiable=True: the returned distribution's mean carries an autograd node (_ActorFn) whenever autograd
-        records and the features or a parameter require grad."""
+        records and the features or a parameter require grad.  differentiable="bf16": the same on the tensor-core
+        kernels (_bf16.ActorFn), under no_grad too, within the tensor-core mode's head shapes."""
         super().__init__()
-        self.differentiable = bool(differentiable)
+        self.differentiable = _flag(differentiable, "Actor")
+        if self.differentiable == "bf16":
+            _check_bf16_dims(int(action_shape[0]), int(hidden_dim), int(feature_dim))
         self.trunk = _Trunk(repr_dim, feature_dim)
         self.policy = _mlp(feature_dim, hidden_dim, action_shape[0])
         self.apply(utils.weight_init)
@@ -439,6 +498,12 @@ class Actor(nn.Module):
         B, dev = obs.shape[0], obs.device
         Fd, H, A = self.trunk[0].out_features, self.policy[0].out_features, self.policy[4].out_features
         obs = obs.float().contiguous()
+        if self.differentiable == "bf16":
+            _bf16.check_batch(B, "Actor")
+            ops = _bf16.operands(self, "actor")
+            tw = (*self.trunk[0].parameters(), *self.trunk[1].parameters(), *self.policy.parameters())
+            mu = _bf16.ActorFn.apply(ops, obs, *tw) if _wants_graph(self, obs) else _bf16.actor_forward(ops, obs, tw)[0]
+            return utils.TruncatedNormal(mu, torch.ones_like(mu) * std)
         if _wants_graph(self, obs):
             mu = _ActorFn.apply(obs, *self.trunk[0].parameters(), *self.trunk[1].parameters(), *self.policy.parameters())
             return utils.TruncatedNormal(mu, torch.ones_like(mu) * std)
@@ -457,12 +522,16 @@ class Actor(nn.Module):
 
 class Critic(nn.Module):
     differentiable = False      # class default: instances pickled before the flag existed read it too
+    refresh = _refresh_bf16
 
     def __init__(self, repr_dim, action_shape, feature_dim, hidden_dim, *, differentiable=False):
         """differentiable=True: Q1 and Q2 carry an autograd node (_CriticFn) whenever autograd records and the features,
-        the action or a parameter require grad."""
+        the action or a parameter require grad.  differentiable="bf16": the same on the tensor-core kernels
+        (_bf16.CriticFn), under no_grad too, within the tensor-core mode's head shapes."""
         super().__init__()
-        self.differentiable = bool(differentiable)
+        self.differentiable = _flag(differentiable, "Critic")
+        if self.differentiable == "bf16":
+            _check_bf16_dims(int(action_shape[0]), int(hidden_dim), int(feature_dim))
         self.trunk = _Trunk(repr_dim, feature_dim)
         self.Q1 = _mlp(feature_dim + action_shape[0], hidden_dim, 1)
         self.Q2 = _mlp(feature_dim + action_shape[0], hidden_dim, 1)
@@ -475,6 +544,13 @@ class Critic(nn.Module):
         A = self.Q1[0].in_features - Fd
         obs = obs.float().contiguous()
         action = action.float().contiguous()
+        if self.differentiable == "bf16":
+            _bf16.check_batch(B, "Critic")
+            ops = _bf16.operands(self, "critic")
+            cw = (*self.trunk[0].parameters(), *self.trunk[1].parameters(), *self.Q1.parameters(), *self.Q2.parameters())
+            if _wants_graph(self, obs, action):
+                return _bf16.CriticFn.apply(ops, obs, action, *cw)
+            return _bf16.critic_forward(ops, obs, action, cw)[:2]
         if _wants_graph(self, obs, action):
             return _CriticFn.apply(obs, action, *self.trunk[0].parameters(), *self.trunk[1].parameters(),
                                    *self.Q1.parameters(), *self.Q2.parameters())
@@ -652,10 +728,14 @@ class _Opt:
             ag._scalars_enqueued()
             a = ag._arena
             off, n = a.seg[self.net][0], a.seg[self.net][2]
-            call("drq_adam_step", a.params.data_ptr() + F32 * off, a.grads.data_ptr() + F32 * off,
-                 a.exp_avg.data_ptr() + F32 * off, a.exp_avg_sq.data_ptr() + F32 * off, n, ag._sc(self.net), _stream())
+            if ag.differentiable == "bf16":
+                # Adam and the refresh of this network's bf16 operand copies in one launch, as update() steps it
+                getattr(ag._bf16, f"step_{self.net}")()
+            else:
+                call("drq_adam_step", a.params.data_ptr() + F32 * off, a.grads.data_ptr() + F32 * off,
+                     a.exp_avg.data_ptr() + F32 * off, a.exp_avg_sq.data_ptr() + F32 * off, n, ag._sc(self.net), _stream())
+                ag._bf16_dirty = True
             ag._opt_steps[self.net] += 1
-            ag._bf16_dirty = True
         return loss
 
 
@@ -682,9 +762,13 @@ class DrQV2Agent:
         parameters require grad, so the reference's own update_critic / update_actor bodies (loss.backward();
         opt.step()) train this agent: gradients land in the arena that encoder_opt / critic_opt / actor_opt.step() read
         (INTEGRATION.md).  The fused update() is unaffected.  Not with data_parallel (those steps do not all-reduce)."""
+        differentiable = _flag(differentiable, "DrQV2Agent")
         if differentiable and data_parallel:
-            raise ValueError("DrQV2Agent: differentiable=True with data_parallel=True is not supported - the optimisers' "
-                             "step() does not average gradients over ranks")
+            raise ValueError(f"DrQV2Agent: differentiable={differentiable!r} with data_parallel=True is not supported - "
+                             "the optimisers' step() does not average gradients over ranks")
+        if differentiable == "bf16" and (mode or os.environ.get("DRQV2_B200_MODE", "bf16")) != "bf16":
+            raise ValueError("DrQV2Agent: differentiable='bf16' runs the tensor-core kernels and needs mode='bf16'; "
+                             "differentiable=True trains through the fp32 kernels in either mode")
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError(f"DrQV2Agent(device={device!r}): drqv2_b200 has no CPU path; use a CUDA device")
@@ -738,17 +822,24 @@ class DrQV2Agent:
             raise ValueError(f"feature_dim {self.feature_dim}: the LayerNorm kernels hold 1 <= F <= {_lib.LN_MAX_F} "
                              "features (in mode='fp32' as well)")
         if self.mode == "bf16":
-            self._check_bf16_dims(dev)
+            _check_bf16_dims(self.action_dim, self.hidden_dim, self.feature_dim, dev)
 
         # models: built on the host in the reference's order (so a seed reproduces its init)
-        self.differentiable = bool(differentiable)
+        self.differentiable = differentiable
         self.encoder = Encoder(self.obs_shape, differentiable=self.differentiable)
         self.actor = Actor(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim, differentiable=self.differentiable)
         self.critic = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim,
                              differentiable=self.differentiable)
-        self.critic_target = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim)
+        # differentiable="bf16": the target forwards on the tensor cores too (under no_grad: its parameters never
+        # require grad)
+        self.critic_target = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim,
+                                    differentiable="bf16" if self.differentiable == "bf16" else False)
         self.critic_target.load_state_dict(self.critic.state_dict())
         self._to_device(dev)
+        if self.differentiable == "bf16":
+            # the modules read this agent's own operand copies (_bf16.operands)
+            for role in ("encoder", "actor", "critic", "critic_target"):
+                getattr(self, role).__dict__["_bf16_owner"] = (self, role)
         if self.differentiable:
             # .grad stays the arena view _Arena._adopt set: autograd adds into an existing .grad in place
             for m in (self.encoder, self.actor, self.critic):
@@ -772,24 +863,6 @@ class DrQV2Agent:
             self._bf16_dirty = True
         self.train()
         self.critic_target.train()
-
-    def _check_bf16_dims(self, dev):
-        """Refuse at construction the shapes the tensor-core mode's head kernels refuse (csrc/heads.cu), which would
-        otherwise fail at the first act() or update()."""
-        A, H = self.action_dim, self.hidden_dim
-        if not 1 <= A <= _lib.POLICY_MAX_A:
-            raise ValueError(f"action_shape ({A},): mode='bf16' supports 1 <= A <= {_lib.POLICY_MAX_A} action dimensions "
-                             "(the policy head kernel); mode='fp32' has no such limit")
-        if H % 8:
-            raise ValueError(f"hidden_dim {H}: mode='bf16' needs a multiple of 8 (16-byte rows of the bf16 operands); "
-                             "mode='fp32' has no such limit")
-        groups = -(-A // _lib.POLICY_GROUP)
-        slab = 4 * H * -(-A // groups)                 # fp32 weights of one policy-head block's action group
-        optin = torch.cuda.get_device_properties(dev).shared_memory_per_block_optin
-        if slab + _lib.POLICY_STATIC_SMEM > optin:
-            raise ValueError(f"hidden_dim {H} with {A} actions: mode='bf16' stages {slab} bytes of policy-head weights per "
-                             f"block, more than the {optin - _lib.POLICY_STATIC_SMEM} bytes of shared memory a block can "
-                             "have here; mode='fp32' has no such limit")
 
     # ------------------------------------------------------------------ plumbing
     def _to_device(self, dev):
@@ -852,6 +925,8 @@ class DrQV2Agent:
         if self._bf16 is not None:
             self._bf16.repack_all()
         self._bf16_dirty = False
+        if self.differentiable == "bf16":     # the parameter versions the copies now match (_bf16.operands)
+            self._bf16_keys = {r: _bf16._param_key(getattr(self, r)) for r in ("encoder", "actor", "critic", "critic_target")}
 
     # ------------------------------------------------------------------ snapshot interop (train.py:192-204)
     _NETS = ("encoder", "actor", "critic")

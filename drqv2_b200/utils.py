@@ -80,7 +80,17 @@ def schedule(schdl, step):
 
 
 def soft_update_params(net, target_net, tau):
-    """tp = tau*p + (1-tau)*tp for every parameter pair, through drq_soft_update."""
+    """tp = tau*p + (1-tau)*tp for every parameter pair, through drq_soft_update.  On the critic / target pair of a
+    DrQV2Agent(differentiable="bf16") at the agent's tau: the agent's one-launch soft update, which refreshes the target's bf16 operand
+    copies with it; on other differentiable="bf16" targets the copies are re-derived before their next forward."""
+    owner = target_net.__dict__.get("_bf16_owner")
+    if (owner is not None and owner[1] == "critic_target" and net is owner[0].critic
+            and float(tau) == float(owner[0].critic_target_tau)):
+        with torch.cuda.device(owner[0]._dev):
+            if owner[0]._bf16_dirty:
+                owner[0].refresh()
+            owner[0]._bf16.step_target()
+        return
     stream = torch.cuda.current_stream().cuda_stream
     for p, tp in zip(net.parameters(), target_net.parameters()):
         if not (p.is_cuda and tp.is_cuda):
@@ -90,6 +100,8 @@ def soft_update_params(net, target_net, tau):
             # launch instead; per-tensor calls need 16-byte alignment
             raise RuntimeError("soft_update_params: tensors must be 16-byte aligned")
         _lib.call("drq_soft_update", p.data_ptr(), tp.data_ptr(), p.numel(), float(tau), float(1 - tau), stream)
+    if getattr(target_net, "differentiable", False) == "bf16":
+        target_net.refresh()
 
 
 class TruncatedNormal(pyd.Normal):

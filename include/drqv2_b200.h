@@ -559,6 +559,43 @@ int drq_q_head_bwd_loss_bf16(int loss, const float* q, const float* tq, const fl
                              const float* w3, uint16_t* dc2, float* dw3, float* db3, int B, int H, int64_t w_stride,
                              void* stream);
 
+/* drq_q_head_bwd_loss_bf16's backward from given upstream gradients (the autograd Critic of differentiable="bf16",
+ * drqv2.py:115-121): dq1 / dq2 [B] fp32, each nullable - a null one skips its head, whose outputs are then left alone.
+ * Head z (0 = Q1, 1 = Q2) reads c2 + z*bs_c2 and w3 + z*w_stride and writes dc2 + z*bs_c2 = RN-bf16(dq w3 (c2 > 0))
+ * at rows < B of its TB activation (rpad = units per row; features < H), and (each nullable) dw3 + z*w_stride [H]
+ * = sum_b dq c2, db3 + z*w_stride = sum_b dq - the sums of the loss modes, in the same fixed order. */
+int drq_q_head_bwd_bf16(const float* dq1, const float* dq2, const uint16_t* c2, int64_t rpad, int64_t bs_c2,
+                        const float* w3, uint16_t* dc2, float* dw3, float* db3, int B, int H, int64_t w_stride,
+                        void* stream);
+
+/* ------------------------------------------------------------------ autograd module boundary, bf16 tensor cores */
+
+/* Rows a feature conversion takes: one grid row per feature row, the same bound drq_pack_features_tb's grid has
+ * (511 blocks of DRQ_TB_ACT rows). */
+#define DRQ_FEATURE_MAX_ROWS 65408
+
+/* Features back to the reference's flatten order (drqv2.py:66): out [rows][39200] fp32, column c*1225 + y*35 + x,
+ * from src in the encoder-output order (c/8)*9800 + (y*35+x)*8 + c%8 - src_tb != 0: TB(DRQ_TB_ACT) bf16 rows (conv4's
+ * feature operand; `src` at a 128-row block boundary), exact; src_tb == 0: fp32 [rows][39200] (the trunk's data
+ * gradient from drq_gemm_bf16 KMN / DRQ_TEPI_F32, ldc = 39200).  Writes exactly out[0 .. rows*39200).  The inverse
+ * of drq_pack_features_tb on bf16-representable rows. */
+int drq_features_to_ref(const void* src, int src_tb, float* out, int rows, void* stream);
+
+/* The bf16 twin of drq_feature_grad_wide_f32: conv4's pre-ReLU gradient as the WB buffer of N images
+ * (drq_wb_elems(N) bf16) from an arbitrary gradient of the features.  dfeat and feat are compact fp32 [N][39200] in
+ * the reference order (feat = conv4's post-ReLU output, the mask).  dpre = RN-bf16(feat > 0 ? dfeat : +0) at the
+ * 35 x 35 pixels of every image and +0 at every other element of the buffer (guard rows, rows 35-40, columns 35-40,
+ * slack): every element of the N-image buffer is written, so that the zeros drq_conv3x3_dgrad_bf16 and
+ * drq_conv3x3_wgrad_bf16 require hold whatever the buffer held before. */
+int drq_feature_grad_wide_bf16(const float* dfeat, const float* feat, uint16_t* dpre, int N, void* stream);
+
+/* out[r*ld_out + c] = 0 + sum over s = 0, 1, .. n_planes-1 (in that order) of planes[s*plane_stride + r*ld + c], for
+ * r < rows, c < cols; writes exactly those elements.  The critic's action gradient: the split-K / per-head planes of
+ * its first layer's data gradient at the action columns (planes + F), summed in the order drq_ln_tanh_bwd and
+ * drq_actor_sample_bwd sum the same planes. */
+int drq_plane_sum_f32(const float* planes, int64_t ld, int64_t plane_stride, int n_planes, float* out, int64_t ld_out,
+                      int rows, int cols, void* stream);
+
 /* ------------------------------------------------------------------ optimiser */
 
 /* scalars (device, float[8]): [0] 1-beta1, [1] beta2, [2] 1-beta2,

@@ -4,6 +4,7 @@ drqv2.py:230-262) against the fused update() at the walker shape (B = 256, A = 6
 Arms, timed in alternating blocks so that a drift of the shared machine touches all alike:
   autograd     fp32 agent, differentiable=True: aug -> encoder -> update_critic -> update_actor -> soft update as the
                reference writes them (torch losses, loss.backward(), opt.step()), every draw from torch's generator
+  autograd_bf16  tensor-core agent, differentiable="bf16": the same body on the tcgen05 kernels
   update_fp32  fp32 agent, update() (CUDA graph) - the same kernels, fused and captured
   update_bf16  the default tensor-core agent, update() (CUDA graph)
 All arms take the same device-resident batch.  ms per update from CUDA events at block boundaries; the card's name and
@@ -103,13 +104,14 @@ def main():
         def __next__(self):
             return batch
 
-    runs = [dict(tag="autograd", agent=agent("fp32", True)), dict(tag="update_fp32", agent=agent("fp32")),
+    runs = [dict(tag="autograd", agent=agent("fp32", True)), dict(tag="autograd_bf16", agent=agent("bf16", "bf16")),
+            dict(tag="update_fp32", agent=agent("fp32")),
             dict(tag="update_bf16", agent=agent("bf16"))]
     for r in runs:
         r.update(step=0, ms=[], it=Forever())
 
         def step(r=r):
-            if r["tag"] == "autograd":
+            if r["tag"].startswith("autograd"):
                 reference_update(r["agent"], batch, r["step"])
             else:
                 r["agent"].update(r["it"], r["step"])
@@ -131,10 +133,11 @@ def main():
                                      ms_per_update_max=st["ms_per_step_max"], updates_per_s_median=st["value_median"])
         print(f"{r['tag']:>12}: {st['ms_per_step_median']:7.3f} ms/update (blocks {st['ms_per_step_min']:.3f} .. "
               f"{st['ms_per_step_max']:.3f}), {st['value_median']:7.1f} updates/s")
-    ag = out["arms"]["autograd"]["ms_per_update_median"]
-    for tag in ("update_fp32", "update_bf16"):
-        out[f"autograd_over_{tag}"] = ag / out["arms"][tag]["ms_per_update_median"]
-        print(f"autograd path / {tag}: {out[f'autograd_over_{tag}']:.2f}x")
+    for arm in ("autograd", "autograd_bf16"):
+        ag = out["arms"][arm]["ms_per_update_median"]
+        for tag in ("update_fp32", "update_bf16"):
+            out[f"{arm}_over_{tag}"] = ag / out["arms"][tag]["ms_per_update_median"]
+            print(f"{arm} path / {tag}: {out[f'{arm}_over_{tag}']:.2f}x")
     print(json.dumps(out))
 
 
