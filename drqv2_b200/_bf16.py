@@ -872,16 +872,38 @@ def _zb(n, dev):
 
 
 # ---- Encoder
-def encoder_forward(ops, u8, biases):
+def needed(ctx, skip=0):
+    """ctx.needs_input_grad narrowed to the inputs this backward pass reaches: under torch.autograd.grad(q, obs) the
+    parameters' edges are not executed, and their weight gradients are not computed.  ctx.next_functions lists the
+    tensor inputs only (skip = the leading non-tensor inputs).  A leaf under torch.autograd.grad cannot be asked, and
+    counts as needed - Encoder(pixels="float") hands its parameters in as views so that it can be asked."""
+    need = list(ctx.needs_input_grad)
+    ask = getattr(torch._C, "_will_engine_execute_node", None)     # private: absent -> ctx.needs_input_grad as it is
+    if ask is None:
+        return need
+    for i, (node, _) in enumerate(ctx.next_functions):
+        if need[skip + i] and node is not None:
+            try:
+                need[skip + i] = bool(ask(node))
+            except Exception:       # a leaf under torch.autograd.grad (RuntimeError), or an API that changed
+                pass
+    return need
+
+
+def encoder_forward(ops, px, biases):
     """conv1 (pixels arrive augmented: no shift, as act() runs it) .. conv4 into TB features, then fp32 features in
-    the reference order.  Returns (features, [conv1..3 WB activations])."""
-    n, cin = u8.shape[0], u8.shape[1]
-    dev, s = u8.device, _stream()
+    the reference order.  px: uint8 pixels, or fp32 ones (Encoder(pixels="float"): drq_conv1_fwd_bf16_from_f32).
+    Returns (features, [conv1..3 WB activations])."""
+    n, cin = px.shape[0], px.shape[1]
+    dev, s = px.device, _stream()
     nel = _lib.lib().drq_wb_elems(n)
     acts = [_zb(nel, dev) for _ in range(3)]     # zeroed: guard rows and the slack are read as zero padding
     ft = TB(n, REPR_DIM, dev)
     a = [t.data_ptr() for t in acts]
-    call("drq_conv1_fwd_bf16", u8.data_ptr(), None, ops.conv1.data_ptr(), a[0], n, cin, 4, s)
+    if px.dtype == torch.uint8:
+        call("drq_conv1_fwd_bf16", px.data_ptr(), None, ops.conv1.data_ptr(), a[0], n, cin, 4, s)
+    else:
+        call("drq_conv1_fwd_bf16_from_f32", px.data_ptr(), ops.conv1.data_ptr(), a[0], n, cin, s)
     call("drq_conv3x3_fwd_bf16", a[0], ops.wf[0].data_ptr(), biases[0], a[1], n, 39, 0, 0, 0, 0, s)
     call("drq_conv3x3_fwd_bf16", a[1], ops.wf[1].data_ptr(), biases[1], a[2], n, 37, 0, 0, 0, 0, s)
     call("drq_conv3x3_fwd_bf16", a[2], ops.wf[2].data_ptr(), biases[2], ft.ptr(), n, 35, 2, ft.units, 0, 0, s)
@@ -893,23 +915,26 @@ def encoder_forward(ops, u8, biases):
 class EncoderFn(torch.autograd.Function):
     """features = Encoder(pixels) on the tensor cores; backward drq_feature_grad_wide_bf16 -> conv4..2
     drq_conv3x3_{wgrad (partials), dgrad}_bf16 -> drq_conv1_wgrad_bf16 -> one drq_conv_wgrad_reduce_multi.
-    Inputs: operand copies, u8 pixels, then (weight, bias) of conv1..4."""
+    Inputs: operand copies, pixels - uint8, or fp32 on the 0..255 scale (Encoder(pixels="float"): the *_from_f32
+    conv1 kernels, and drq_conv1_dgrad_bf16 for pixels that require grad) - then (weight, bias) of conv1..4.  Every
+    weight gradient runs only when its parameter needs it."""
 
     @staticmethod
-    def forward(ctx, ops, u8, *params):
-        feat, acts = encoder_forward(ops, u8, [p.data_ptr() for p in params[3::2]])
+    def forward(ctx, ops, px, *params):
+        feat, acts = encoder_forward(ops, px, [p.data_ptr() for p in params[3::2]])
         ctx.ops = ops
-        ctx.save_for_backward(u8, *acts, feat)
+        ctx.save_for_backward(px, *acts, feat)
         return feat
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, dfeat):
-        u8, a1, a2, a3, feat = ctx.saved_tensors
-        need = ctx.needs_input_grad[2:]
-        if not any(need):
+        px, a1, a2, a3, feat = ctx.saved_tensors
+        need_all = needed(ctx, skip=1)
+        need_x, need = need_all[1], need_all[2:]
+        if not (need_x or any(need)):
             return (None,) * 10
-        n, cin = u8.shape[0], u8.shape[1]
+        n, cin = px.shape[0], px.shape[1]
         dev, s, L = feat.device, _stream(), _lib.lib()
         dfeat = dfeat.float().contiguous()
         nel = L.drq_wb_elems(n)
@@ -924,15 +949,27 @@ class EncoderFn(torch.autograd.Function):
         call("drq_feature_grad_wide_bf16", dfeat.data_ptr(), feat.data_ptr(), dp[3], n, s)
         jobs = []
         for layer, hout in ((3, 35), (2, 37), (1, 39)):
-            call("drq_conv3x3_wgrad_bf16", acts[layer - 1], n, dp[layer], ws[layer].data_ptr(), None, None, n, hout, s)
-            jobs.append(WgReduceJob(ws[layer].data_ptr(), grads[2 * layer].data_ptr(), grads[2 * layer + 1].data_ptr(),
-                                    n, hout, 0, 0))
-            call("drq_conv3x3_dgrad_bf16", dp[layer], ctx.ops.wd[layer - 1].data_ptr(), acts[layer - 1], n, dp[layer - 1],
-                 n, hout, s)
-        call("drq_conv1_wgrad_bf16", u8.data_ptr(), None, dp[0], ws[0].data_ptr(), None, None, n, cin, 4, s)
-        jobs.append(WgReduceJob(ws[0].data_ptr(), grads[0].data_ptr(), grads[1].data_ptr(), n, 0, cin, 0))
-        call("drq_conv_wgrad_reduce_multi", (WgReduceJob * len(jobs))(*jobs), len(jobs), s)
-        return (None, None) + tuple(g if nd else None for g, nd in zip(grads, need))
+            if need[2 * layer] or need[2 * layer + 1]:
+                call("drq_conv3x3_wgrad_bf16", acts[layer - 1], n, dp[layer], ws[layer].data_ptr(), None, None, n, hout, s)
+                jobs.append(WgReduceJob(ws[layer].data_ptr(), grads[2 * layer].data_ptr(),
+                                        grads[2 * layer + 1].data_ptr(), n, hout, 0, 0))
+            if need_x or any(need[:2 * layer]):
+                call("drq_conv3x3_dgrad_bf16", dp[layer], ctx.ops.wd[layer - 1].data_ptr(), acts[layer - 1], n,
+                     dp[layer - 1], n, hout, s)
+        if need[0] or need[1]:
+            if px.dtype == torch.uint8:
+                call("drq_conv1_wgrad_bf16", px.data_ptr(), None, dp[0], ws[0].data_ptr(), None, None, n, cin, 4, s)
+                jobs.append(WgReduceJob(ws[0].data_ptr(), grads[0].data_ptr(), grads[1].data_ptr(), n, 0, cin, 0))
+            else:
+                call("drq_conv1_wgrad_bf16_from_f32", px.data_ptr(), dp[0], ws[0].data_ptr(), grads[0].data_ptr(),
+                     grads[1].data_ptr(), n, cin, s)
+        if jobs:
+            call("drq_conv_wgrad_reduce_multi", (WgReduceJob * len(jobs))(*jobs), len(jobs), s)
+        dx = None
+        if need_x:
+            dx = torch.empty(px.shape, device=dev)
+            call("drq_conv1_dgrad_bf16", dp[0], ctx.ops.conv1.data_ptr(), dx.data_ptr(), n, cin, s)
+        return (None, dx) + tuple(g if nd else None for g, nd in zip(grads, need))
 
 
 # ---- heads: the trunk (Linear(39200 -> F) + LayerNorm + tanh) shared by Actor and Critic

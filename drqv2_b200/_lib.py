@@ -36,6 +36,10 @@ SIGNATURES = {
     "drq_random_shift_f32": [P, P, P, I, I, I, I, I, P],
     "drq_conv1_fwd_f32": [P, P, P, P, P, I, I, I, P],
     "drq_conv1_wgrad_f32": [P, P, P, P, P, P, I, I, I, P],
+    "drq_conv1_fwd_f32_from_f32": [P, P, P, P, I, I, P],
+    "drq_conv1_wgrad_f32_from_f32": [P, P, P, P, P, I, I, P],
+    "drq_conv1_dgrad_f32": [P, P, P, I, I, P],
+    "drq_random_shift_bwd_f32": [P, P, P, I, I, I, I, I, P],
     "drq_conv3x3_fwd_f32": [P, P, P, P, I, I, I, P],
     "drq_conv3x3_dgrad_f32": [P, P, P, P, I, I, P],
     "drq_conv3x3_wgrad_f32": [P, P, P, P, P, I, I, P],
@@ -47,6 +51,9 @@ SIGNATURES = {
     "drq_pack_conv1_w_bf16": [P, P, P, I, P],
     "drq_conv1_fwd_bf16": [P, P, P, P, I, I, I, P],
     "drq_conv1_wgrad_bf16": [P, P, P, P, P, P, I, I, I, P],
+    "drq_conv1_fwd_bf16_from_f32": [P, P, P, I, I, P],
+    "drq_conv1_wgrad_bf16_from_f32": [P, P, P, P, P, I, I, P],
+    "drq_conv1_dgrad_bf16": [P, P, P, I, I, P],
     "drq_gemm_bf16": [P, I, P, I, I, P, L, I, P, P, I, I, I, I, I, I, I, I, P, I, I, P],
     "drq_set_sm_limit": [I],
     "drq_set_gemm_small": [I],

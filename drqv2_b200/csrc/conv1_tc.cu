@@ -60,6 +60,7 @@ struct Conv1TcArgs {
     // rows straight from the replay ring (ring_frames != null; obs unused): see drq_conv1_fwd_bf16_ring
     const uint8_t* ring_frames; const int* ring_ep_start; const int* ring_idx;
     long long ring_capacity; int ring_B, ring_nstep, ring_stack, ring_frame_c;
+    const float* fobs;            // real-valued pixels [N][cin][84][84] (the *_from_f32 entry points; obs unused)
 };
 
 // first byte of channel `c` of image `n`: the gathered stack, or the ring frame the stack is made of
@@ -189,7 +190,29 @@ __device__ __forceinline__ void build_part(uint8_t* tile, const uint8_t* __restr
     }
 }
 
-template <bool WGRAD, int CIN>
+// The same K units from real-valued pixels (FSRC): entry k < cin*9 is RN-bf16(RN-fp32(x - 128)) of the pixel
+// x = fobs[n][c][2*oy + ky][2*ox + kx] (already augmented, no shift), entry cin*9 the constant 1.0, the rest 0.  On
+// integer pixels in 0..255 these are the bits build_part makes.
+template <int U0>
+__device__ __forceinline__ void build_part_f32(uint8_t* tile, const float* __restrict__ img, int kmax, int r, int oy, int ox) {
+    auto entry = [&](int k) -> float {
+        if (k >= kmax) return k == kmax ? 1.f : 0.f;
+        const int c = k / 9, ky = (k % 9) / 3, kx = k % 3;
+        return __fsub_rn(__ldg(img + (c * kImg + 2 * oy + ky) * kImg + 2 * ox + kx), 128.f);
+    };
+#pragma unroll
+    for (int u = 0; u < 3; ++u) {
+        uint32_t w[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int kA = (U0 + u) * 8 + 2 * e;
+            w[e] = pack_bf16x2(entry(kA), entry(kA + 1));
+        }
+        *reinterpret_cast<uint4*>(tile + (U0 + u) * (kC1Tile * 16) + r * 16) = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+}
+
+template <bool WGRAD, int CIN, bool FSRC = false>
 __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     constexpr int STAGE = kC1ABytes + (WGRAD ? kC1DBytes : 0);
@@ -248,11 +271,13 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
             const int rs = ord % kC1RawStages; const uint32_t rphase = (ord / kC1RawStages) & 1;
             const TileGeom cur = tile_geom(t, a.shift, a.pad);
             uint8_t* stg = in_s + (group * 2 + (it & 1)) * kC1InBytes;
-            mbar_wait(rfull + rs, rphase);
-            pad_rows(raw_s + rs * kC1RawBytes, stg, (cur.rlo * kImg) & 15, cur.nrows, a.cin, gb);
-            mbar_arrive(rempty + rs);
-            if (group == 0) asm volatile("bar.sync 1, 256;" ::: "memory");      // padded rows visible to the group
-            else            asm volatile("bar.sync 2, 256;" ::: "memory");
+            if (!FSRC) {
+                mbar_wait(rfull + rs, rphase);
+                pad_rows(raw_s + rs * kC1RawBytes, stg, (cur.rlo * kImg) & 15, cur.nrows, a.cin, gb);
+                mbar_arrive(rempty + rs);
+                if (group == 0) asm volatile("bar.sync 1, 256;" ::: "memory");      // padded rows visible to the group
+                else            asm volatile("bar.sync 2, 256;" ::: "memory");
+            }
             // Positions past the image (last tile) build from clamped, valid addresses in the forward (their rows
             // are never stored); in wgrad their im2col rows are zeroed below (the gradient tile's rows there
             // belong to the next image).
@@ -272,6 +297,10 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
 #pragma unroll
                 for (int u = 0; u < 6; ++u)
                     *reinterpret_cast<uint4*>(tile + (half * 6 + u) * (kC1Tile * 16) + r * 16) = make_uint4(0, 0, 0, 0);
+            } else if (FSRC) {
+                const float* img = a.fobs + (long long)cur.n * a.cin * (kImg * kImg);
+                if (half == 0) { build_part_f32<0>(tile, img, a.cin * 9, r, oy, ox); build_part_f32<3>(tile, img, a.cin * 9, r, oy, ox); }
+                else           { build_part_f32<6>(tile, img, a.cin * 9, r, oy, ox); build_part_f32<9>(tile, img, a.cin * 9, r, oy, ox); }
             } else if (half == 0) {
                 build_part<0, CIN>(tile, stg, a.cin, r, rowoff, gofs);
                 build_part<3, CIN>(tile, stg, a.cin, r, rowoff, gofs);
@@ -352,7 +381,7 @@ __global__ void __launch_bounds__(kC1Threads, 1) conv1_tc_kernel(Conv1TcArgs a) 
         }
     } else if (warp == 21) {
         // ------------------------------------------------ row producer: lane c copies channel c's rows of the tile
-        if (lane < a.cin) {
+        if (!FSRC && lane < a.cin) {
             int rs = 0; uint32_t rphase = 0;
             // As in conv1_planes_kernel's producer: the image's shift, ring index and episode start are requested
             // kAhead tiles ahead (their round trip to L2, and a 64-bit modulo per tile, were on this warp's serial path:
@@ -826,6 +855,138 @@ __global__ void __launch_bounds__(kP1Threads, 1) conv1_planes_kernel(const __gri
     if (warp == kBuildWarps) tmem_dealloc(tmem_base, kP1Acc * 32);
 }
 
+// ---------------------------------------------------------------- data gradient
+// d(pixels) of conv1 from its pre-ReLU gradient dY (WB bf16, K-major over co exactly as conv2's forward reads conv1's
+// output): per tile of three output rows (positions p0 = 123 t .. p0 + 127 of the image, rows 123.. unused)
+//   col[p][k] = sum_co dY[p][co] * W[co][k]                        M = 128 positions, N = 96 (k = 9c + tap), K = 32 co
+// one UMMA pair (two K16 steps) into 96 TMEM columns.  The packed conv1 weights [12 k units][32 co][8 k] are the
+// canonical MN-major B operand of this product (MN = k, K = co) as they stand.  Col2im in the epilogue: the tile's col
+// goes through shared memory and every input pixel sums its <= 4 entries, taps (ky, kx) ascending (the carried row:
+// ky = 2 of the previous tile first, then ky = 0 of this one).  A CTA takes whole
+// images and their 14 tiles in order: tile t completes input rows 6t .. 6t+5; row 6t+6 also takes taps of the next
+// tile, so its partial sum (ky = 2 of output row 3t+2) is carried in shared memory and the next tile adds its ky = 0
+// taps to it.  Row 83 takes no tap and is written as +0.  Fixed order, no atomics, no global scratch.
+constexpr int kDgTiles = 14;
+constexpr int kDgColPitch = 97;                 // fp32 col row pitch in shared memory (conflict-free gathers)
+constexpr int kDgThreads = 128;
+constexpr int kDgABytes = 4 * kC1Tile * 16;     // [4 co blocks][128 positions][16 B]
+constexpr size_t kDgOffA = kC1WBytes;
+constexpr size_t kDgOffCol = kDgOffA + 2 * kDgABytes;
+constexpr size_t kDgOffCarry = kDgOffCol + (size_t)kC1Tile * kDgColPitch * 4;
+constexpr size_t kDgOffBars = kDgOffCarry + 2 * 10 * kImg * 4;
+constexpr size_t kConv1DgradSmem = kDgOffBars + 4 * 8 + 16;
+
+__global__ void __launch_bounds__(kDgThreads) conv1_dgrad_tc_kernel(const __nv_bfloat16* __restrict__ d, long long cs_d,
+                                                                    const __nv_bfloat16* __restrict__ w_packed,
+                                                                    float* __restrict__ dx, int n_images, int cin) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    uint8_t* w_s = smem;
+    uint8_t* a_s = smem + kDgOffA;
+    float* col_s = reinterpret_cast<float*>(smem + kDgOffCol);
+    float* carry_s = reinterpret_cast<float*>(smem + kDgOffCarry);      // [2][cin][84]
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + kDgOffBars);   // [2]
+    uint64_t* mma = full + 2;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(mma + 1);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+
+    if (tid == 0) {
+        mbar_init(full, 1); mbar_init(full + 1, 1); mbar_init(mma, 1);
+        fence_barrier_init();
+    }
+    if (warp == 0) {
+        tmem_alloc(tmem_slot, 128);
+        tmem_relinquish();
+    }
+    {
+        const uint4* src = reinterpret_cast<const uint4*>(w_packed);
+        for (int i = tid; i < kC1WBytes / 16; i += kDgThreads) reinterpret_cast<uint4*>(w_s)[i] = __ldg(src + i);
+    }
+    fence_proxy_async();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+
+    // tile j of this CTA: image blockIdx.x + (j / 14) * gridDim.x, tile j % 14
+    auto load = [&](int j) {
+        const int n = blockIdx.x + (j / kDgTiles) * (int)gridDim.x, t = j % kDgTiles;
+        const int s = j & 1;
+        const long long row0 = (long long)n * DRQ_PLB + DRQ_GUARD + t * 3 * kPW;
+        mbar_arrive_expect_tx(full + s, kDgABytes);
+        for (int c = 0; c < 4; ++c)
+            bulk_g2s(a_s + s * kDgABytes + c * kC1Tile * 16, d + (c * cs_d + row0) * 8, kC1Tile * 16, full + s);
+    };
+    const int my_images = blockIdx.x < n_images ? (n_images - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+    const int my_tiles = my_images * kDgTiles;
+    if (tid == 0 && my_tiles > 0) load(0);
+    const uint64_t da0 = make_smem_desc(smem_u32(a_s), kC1Tile * 16, 128);   // dY, K-major (K = co)
+    const uint64_t db0 = make_smem_desc(smem_u32(w_s), 128, 512);            // W, MN-major (MN = k, K = co)
+    constexpr uint32_t idesc = make_idesc_bf16(128, kC1K, false, true);
+
+    for (int j = 0; j < my_tiles; ++j) {
+        const int n = blockIdx.x + (j / kDgTiles) * (int)gridDim.x, t = j % kDgTiles;
+        const int s = j & 1;
+        // the other stage's UMMAs retired before the previous tile's epilogue started
+        if (tid == 0 && j + 1 < my_tiles) load(j + 1);
+        mbar_wait(full + s, (j >> 1) & 1);
+        tc_fence_after();
+        if (warp == 0) {
+            if (elect_one()) {
+#pragma unroll
+                for (int ks = 0; ks < 2; ++ks)
+                    umma_bf16(tmem_base, da0 + (uint64_t)(s * (kDgABytes >> 4) + ks * 2 * kC1Tile), db0 + (uint64_t)(ks * 16),
+                              idesc, ks ? 1u : 0u);
+                umma_commit(mma);
+            }
+            __syncwarp();
+        }
+        mbar_wait(mma, j & 1);
+        tc_fence_after();
+#pragma unroll
+        for (int c0 = 0; c0 < kC1K; c0 += 32) {
+            float v[32];
+            tmem_ld_32x32(tmem_base + ((uint32_t)(warp * 32) << 16) + c0, v);
+            float* dst = col_s + (warp * 32 + lane) * kDgColPitch + c0;
+#pragma unroll
+            for (int i = 0; i < 32; ++i) dst[i] = v[i];
+        }
+        tc_fence_before();
+        __syncthreads();
+        // col2im of output rows oy0 .. oy0 + R - 1 into input rows 2 oy0 .. 2 oy0 + 2R (the last one carried unless t = 13)
+        const int oy0 = 3 * t, R = min(3, kPW - oy0), nrows = 2 * R + 1;
+        const float* carry_in = carry_s + ((t + 1) & 1) * (10 * kImg);
+        float* carry_out = carry_s + (t & 1) * (10 * kImg);
+        float* dx_n = dx + (long long)n * cin * (kImg * kImg);
+        for (int i = tid; i < cin * nrows * kImg; i += kDgThreads) {
+            const int c = i / (nrows * kImg), rem = i - c * (nrows * kImg), rl = rem / kImg, ix = rem - rl * kImg;
+            const int iy = 2 * oy0 + rl;
+            float acc = (rl == 0 && t > 0) ? carry_in[c * kImg + ix] : 0.f;
+#pragma unroll
+            for (int ky = 0; ky < 3; ++ky) {
+                const int oy2 = rl - ky;                       // 2 (oy - oy0)
+                if (oy2 < 0 || (oy2 & 1) || (oy2 >> 1) >= R) continue;
+#pragma unroll
+                for (int kx = 0; kx < 3; ++kx) {
+                    const int ox2 = ix - kx;
+                    if (ox2 < 0 || (ox2 & 1) || (ox2 >> 1) >= kPW) continue;
+                    acc += col_s[((oy2 >> 1) * kPW + (ox2 >> 1)) * kDgColPitch + c * 9 + ky * 3 + kx];
+                }
+            }
+            if (rl == nrows - 1 && t < kDgTiles - 1) carry_out[c * kImg + ix] = acc;
+            else dx_n[(c * kImg + iy) * kImg + ix] = __fdiv_rn(acc, 255.0f);
+        }
+        if (t == kDgTiles - 1)
+            for (int i = tid; i < cin * kImg; i += kDgThreads)
+                dx_n[((i / kImg) * kImg + kImg - 1) * kImg + i % kImg] = 0.f;
+        tc_fence_before();
+        __syncthreads();                 // col_s and the carry are re-written by the next tile; TMEM is re-accumulated
+        tc_fence_after();
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_dealloc(tmem_base, 128);
+}
+
 constexpr size_t kConv1PlanesSmem = kP1WBytes + 128 + kP1RawStages * kP1RawBytes + kP1Stages * kP1StageBytes + 128 +
                                     (2 * kP1Stages + 2 * kP1Acc + 2 * kP1RawStages) * 8 + 16;
 static_assert(kC1WBytes + 128 <= kP1RawStages * kP1RawBytes, "the packed weights are staged in the raw-row buffer");
@@ -981,6 +1142,52 @@ static int conv1_wgrad_launch(Conv1TcArgs& a, const int32_t* shift, const uint16
     if (int rc = check_launch("conv1_tc_kernel<wgrad>")) return rc;
     if (!dw) return DRQ_OK;                                   // partials only: reduced later by drq_conv_wgrad_reduce_multi
     conv1_wgrad_reduce_kernel<<<kC1ReduceBlocks, 256, 0, stream>>>(partial, G, cin, dw, db);
+    return check_launch("conv1_wgrad_reduce_kernel");
+}
+
+int drq_conv1_dgrad_bf16(const uint16_t* dpre, const uint16_t* w_packed, float* dx, int N, int cin, void* stream) {
+    DRQ_REQUIRE(dpre && w_packed && dx, "conv1_dgrad_bf16: null pointer");
+    DRQ_REQUIRE(N >= 0 && cin > 0 && cin * 9 + 1 <= kC1K, "conv1_dgrad_bf16: bad dims (cin <= 10)");
+    if (N == 0) return DRQ_OK;
+    if (int rc = ensure_smem((const void*)conv1_dgrad_tc_kernel, kConv1DgradSmem, "conv1_dgrad_bf16")) return rc;
+    const int G = N < 2 * sm_budget() ? N : 2 * sm_budget();
+    conv1_dgrad_tc_kernel<<<G, kDgThreads, kConv1DgradSmem, as_stream(stream)>>>(
+        reinterpret_cast<const __nv_bfloat16*>(dpre), (long long)N * DRQ_PLB + DRQ_WB_SLACK,
+        reinterpret_cast<const __nv_bfloat16*>(w_packed), dx, N, cin);
+    return check_launch("conv1_dgrad_tc_kernel");
+}
+
+int drq_conv1_fwd_bf16_from_f32(const float* obs, const uint16_t* w_packed, uint16_t* out, int N, int cin, void* stream) {
+    DRQ_REQUIRE(obs && w_packed && out, "conv1_fwd_bf16_from_f32: null pointer");
+    DRQ_REQUIRE(N > 0 && cin > 0 && cin * 9 + 1 <= kC1K, "conv1_fwd_bf16_from_f32: bad dims (cin <= 10)");
+    if (int rc = ensure_smem((const void*)conv1_tc_kernel<false, 0, true>, kConv1FwdSmem, "conv1_fwd_bf16_from_f32")) return rc;
+    Conv1TcArgs a{};
+    a.fobs = obs; a.cin = cin;
+    a.w = reinterpret_cast<const __nv_bfloat16*>(w_packed);
+    a.out = reinterpret_cast<__nv_bfloat16*>(out);
+    a.cs_out = (long long)N * DRQ_PLB + DRQ_WB_SLACK;
+    a.n_images = N;
+    const int tiles = N * 14;
+    const int G = tiles < sm_budget() ? tiles : sm_budget();
+    conv1_tc_kernel<false, 0, true><<<G, kC1Threads, kConv1FwdSmem, as_stream(stream)>>>(a);
+    return check_launch("conv1_tc_kernel<fwd, f32 pixels>");
+}
+
+int drq_conv1_wgrad_bf16_from_f32(const float* obs, const uint16_t* dpre, float* partial, float* dw, float* db, int N,
+                                  int cin, void* stream) {
+    DRQ_REQUIRE(obs && dpre && partial && dw && db, "conv1_wgrad_bf16_from_f32: null pointer");
+    DRQ_REQUIRE(N > 0 && cin > 0 && cin * 9 + 1 <= kC1K, "conv1_wgrad_bf16_from_f32: bad dims (cin <= 10)");
+    if (int rc = ensure_smem((const void*)conv1_tc_kernel<true, 0, true>, kConv1WgSmem, "conv1_wgrad_bf16_from_f32")) return rc;
+    Conv1TcArgs a{};
+    a.fobs = obs; a.cin = cin;
+    a.d = reinterpret_cast<const __nv_bfloat16*>(dpre);
+    a.cs_d = (long long)N * DRQ_PLB + DRQ_WB_SLACK;
+    a.partial = partial;
+    a.n_images = N;
+    const int G = conv1_wgrad_ctas(N);
+    conv1_tc_kernel<true, 0, true><<<G, kC1Threads, kConv1WgSmem, as_stream(stream)>>>(a);
+    if (int rc = check_launch("conv1_tc_kernel<wgrad, f32 pixels>")) return rc;
+    conv1_wgrad_reduce_kernel<<<kC1ReduceBlocks, 256, 0, as_stream(stream)>>>(partial, G, cin, dw, db);
     return check_launch("conv1_wgrad_reduce_kernel");
 }
 

@@ -198,8 +198,10 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ partial, int G, in
 
 // ---------------------------------------------------------------- conv1 (u8, aug fused)
 // Stages the augmented, normalised input rows of one output-row tile in shared
-// memory: the augmented image never exists in HBM.
-__device__ __forceinline__ void conv1_stage_input(const uint8_t* __restrict__ img, int cin, int sx,
+// memory: the augmented image never exists in HBM.  T = uint8_t (frames) or float
+// (real-valued pixels on the 0..255 scale, already augmented: no shift).
+template <typename T>
+__device__ __forceinline__ void conv1_stage_input(const T* __restrict__ img, int cin, int sx,
                                                   int sy, int pad, int oy0, float* x_s, int tid,
                                                   int nthreads) {
     const int total = cin * kC1InRows * kImg;
@@ -214,8 +216,9 @@ __device__ __forceinline__ void conv1_stage_input(const uint8_t* __restrict__ im
     }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(288)
-conv1_fwd_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shift,
+conv1_fwd_kernel(const T* __restrict__ obs, const int* __restrict__ shift,
                  const float* __restrict__ w, const float* __restrict__ bias,
                  float* __restrict__ out, int cin, int pad) {
     extern __shared__ __align__(16) float smem[];
@@ -264,8 +267,9 @@ conv1_fwd_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shift,
 }
 
 // thread = (co pair, ci): 2 x 9 accumulators; block walks (image, row tile) items.
+template <typename T>
 __global__ void __launch_bounds__(256)
-conv1_wgrad_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shift,
+conv1_wgrad_kernel(const T* __restrict__ obs, const int* __restrict__ shift,
                    const float* __restrict__ dpre, float* __restrict__ partial, int N, int cin,
                    int pad) {
     extern __shared__ __align__(16) float smem[];
@@ -330,6 +334,73 @@ conv1_wgrad_kernel(const uint8_t* __restrict__ obs, const int* __restrict__ shif
     }
 }
 
+// ---------------------------------------------------------------- conv1 data gradient
+// dx[n][c][iy][ix] = (1/255) sum_{ky,kx: iy = 2oy+ky, ix = 2ox+kx, oy,ox < 41} sum_co W[co][c][ky][kx] d[co][oy*41+ox]:
+// the stride-2 transpose, at most 2 x 2 taps per input pixel (one along an odd coordinate, two along an even one, none
+// at row / column 83).  Block = (12 input rows, image): the d rows those rows reach (oy = 6t-1 .. 6t+5) and the weights
+// are staged in shared memory.  Threads take pixels column-parity major within a row (42 even columns, then 42 odd
+// ones), so most warps take one tap pattern.  Fixed order: taps (ky, kx) ascending, co ascending within a tap.
+constexpr int kDgRows = 12;                   // input rows per block (84 = 7 x 12)
+constexpr int kDgDRows = kDgRows / 2 + 1;     // 7 d rows
+
+__global__ void __launch_bounds__(256)
+conv1_dgrad_kernel(const float* __restrict__ dpre, const float* __restrict__ w, float* __restrict__ dx, int cin) {
+    extern __shared__ __align__(16) float smem[];
+    float* w_s = smem;                          // [tap][co][16 ci]
+    float* d_s = smem + 9 * kCh * 16;           // [co][7][41]
+    const int tid = threadIdx.x, n = blockIdx.y, iy0 = blockIdx.x * kDgRows;
+    const int oy_lo = iy0 / 2 - 1;
+    for (int i = tid; i < 9 * kCh * 16; i += blockDim.x) {
+        const int tap = i / (kCh * 16), co = (i / 16) % kCh, ci = i % 16;
+        w_s[i] = ci < cin ? __ldg(w + (co * cin + ci) * 9 + tap) : 0.f;
+    }
+    const float* d_n = dpre + (long long)n * kCh * kPlane;
+    for (int i = tid; i < kCh * kDgDRows * kPW; i += blockDim.x) {
+        const int co = i / (kDgDRows * kPW), l = i - co * (kDgDRows * kPW);
+        const int oy = oy_lo + l / kPW;
+        d_s[i] = (oy >= 0 && oy < kPW) ? __ldg(d_n + co * kPlane + oy * kPW + l % kPW) : 0.f;
+    }
+    __syncthreads();
+    for (int q = tid; q < kDgRows * kImg; q += blockDim.x) {
+        const int iyl = q / kImg, rem = q - iyl * kImg, px = rem / (kImg / 2), ix = 2 * (rem - px * (kImg / 2)) + px;
+        const int iy = iy0 + iyl;
+        float acc[16];
+#pragma unroll
+        for (int c = 0; c < 16; ++c) acc[c] = 0.f;
+#pragma unroll
+        for (int ky = 0; ky < 3; ++ky) {
+            const int oy2 = iy - ky;
+            if (oy2 < 0 || (oy2 & 1) || (oy2 >> 1) >= kPW) continue;
+            const float* drow = d_s + ((oy2 >> 1) - oy_lo) * kPW;
+#pragma unroll
+            for (int kx = 0; kx < 3; ++kx) {
+                const int ox2 = ix - kx;
+                if (ox2 < 0 || (ox2 & 1) || (ox2 >> 1) >= kPW) continue;
+                const float* dp = drow + (ox2 >> 1);
+                const float* wp = w_s + (ky * 3 + kx) * kCh * 16;
+#pragma unroll 4
+                for (int co = 0; co < kCh; ++co) {
+                    const float dv = dp[co * kDgDRows * kPW];
+                    const float4* w4 = reinterpret_cast<const float4*>(wp + co * 16);
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        if (4 * j >= cin) break;
+                        const float4 v = w4[j];
+                        acc[4 * j + 0] = fmaf(dv, v.x, acc[4 * j + 0]);
+                        acc[4 * j + 1] = fmaf(dv, v.y, acc[4 * j + 1]);
+                        acc[4 * j + 2] = fmaf(dv, v.z, acc[4 * j + 2]);
+                        acc[4 * j + 3] = fmaf(dv, v.w, acc[4 * j + 3]);
+                    }
+                }
+            }
+        }
+        float* o = dx + (long long)n * cin * kImg * kImg + iy * kImg + ix;
+#pragma unroll
+        for (int c = 0; c < 16; ++c)
+            if (c < cin) o[c * kImg * kImg] = __fdiv_rn(acc[c], 255.0f);
+    }
+}
+
 // ---------------------------------------------------------------- compact feature gradient -> conv4's wide dpre
 // One thread per wide position p < 37*41 of a plane: the ReLU-masked feature gradient inside 35 x 35, +0 at rows
 // 35-36 and columns 35-40 (what drq_conv3x3_dgrad_f32 reads at hout = 35 and requires to be zero).
@@ -357,6 +428,34 @@ static int set_smem(K kernel, size_t bytes, const char* what) {
     return ensure_smem(reinterpret_cast<const void*>(kernel), bytes, what);
 }
 
+template <typename T>
+static int conv1_fwd_launch(const T* obs, const int32_t* shift, const float* w, const float* b, float* out, int N,
+                            int cin, int pad, void* stream) {
+    DRQ_REQUIRE(obs && w && b && out, "conv1_fwd: null pointer");
+    DRQ_REQUIRE(N >= 0 && cin > 0 && cin <= 16 && pad >= 0, "conv1_fwd: bad dims (cin<=16)");
+    if (N == 0) return DRQ_OK;
+    const size_t smem = (size_t)(cin * kC1InRows * kImg + cin * 9 * kCh) * sizeof(float);
+    if (int rc = set_smem(conv1_fwd_kernel<T>, smem, "conv1_fwd")) return rc;
+    conv1_fwd_kernel<T><<<dim3(kC1Tiles, N), 288, smem, as_stream(stream)>>>(obs, shift, w, b, out, cin, pad);
+    return check_launch("conv1_fwd_kernel");
+}
+
+template <typename T>
+static int conv1_wgrad_launch(const T* obs, const int32_t* shift, const float* dpre, float* partial, float* dw,
+                              float* db, int N, int cin, int pad, void* stream) {
+    DRQ_REQUIRE(obs && dpre && partial && dw && db, "conv1_wgrad: null pointer");
+    DRQ_REQUIRE(N > 0 && cin > 0 && cin <= 16 && pad >= 0, "conv1_wgrad: bad dims (cin<=16)");
+    const size_t smem = (size_t)(cin * kC1InRows * kImg + kCh * (kC1Rows * kPW + 1)) * sizeof(float);
+    if (int rc = set_smem(conv1_wgrad_kernel<T>, smem, "conv1_wgrad")) return rc;
+    const int items = N * kC1Tiles;
+    const int G = items < kWgradBlocks ? items : kWgradBlocks;
+    conv1_wgrad_kernel<T><<<G, 256, smem, as_stream(stream)>>>(obs, shift, dpre, partial, N, cin, pad);
+    if (int rc = check_launch("conv1_wgrad_kernel")) return rc;
+    const int nw = kCh * cin * 9;
+    wgrad_reduce_kernel<<<(nw + kCh + 127) / 128, 128, 0, as_stream(stream)>>>(partial, G, nw, kCh, dw, db);
+    return check_launch("wgrad_reduce_kernel");
+}
+
 }  // namespace drq
 
 using namespace drq;
@@ -367,28 +466,32 @@ int64_t drq_conv_wgrad_ws_floats(int cin) { return (int64_t)kWgradBlocks * (kCh 
 
 int drq_conv1_fwd_f32(const uint8_t* obs, const int32_t* shift, const float* w, const float* b,
                       float* out, int N, int cin, int pad, void* stream) {
-    DRQ_REQUIRE(obs && w && b && out, "conv1_fwd: null pointer");
-    DRQ_REQUIRE(N >= 0 && cin > 0 && cin <= 16 && pad >= 0, "conv1_fwd: bad dims (cin<=16)");
-    if (N == 0) return DRQ_OK;
-    const size_t smem = (size_t)(cin * kC1InRows * kImg + cin * 9 * kCh) * sizeof(float);
-    if (int rc = set_smem(conv1_fwd_kernel, smem, "conv1_fwd")) return rc;
-    conv1_fwd_kernel<<<dim3(kC1Tiles, N), 288, smem, as_stream(stream)>>>(obs, shift, w, b, out, cin, pad);
-    return check_launch("conv1_fwd_kernel");
+    return conv1_fwd_launch(obs, shift, w, b, out, N, cin, pad, stream);
+}
+
+int drq_conv1_fwd_f32_from_f32(const float* obs, const float* w, const float* b, float* out, int N, int cin,
+                               void* stream) {
+    return conv1_fwd_launch(obs, nullptr, w, b, out, N, cin, 0, stream);
 }
 
 int drq_conv1_wgrad_f32(const uint8_t* obs, const int32_t* shift, const float* dpre, float* partial,
                         float* dw, float* db, int N, int cin, int pad, void* stream) {
-    DRQ_REQUIRE(obs && dpre && partial && dw && db, "conv1_wgrad: null pointer");
-    DRQ_REQUIRE(N > 0 && cin > 0 && cin <= 16 && pad >= 0, "conv1_wgrad: bad dims (cin<=16)");
-    const size_t smem = (size_t)(cin * kC1InRows * kImg + kCh * (kC1Rows * kPW + 1)) * sizeof(float);
-    if (int rc = set_smem(conv1_wgrad_kernel, smem, "conv1_wgrad")) return rc;
-    const int items = N * kC1Tiles;
-    const int G = items < kWgradBlocks ? items : kWgradBlocks;
-    conv1_wgrad_kernel<<<G, 256, smem, as_stream(stream)>>>(obs, shift, dpre, partial, N, cin, pad);
-    if (int rc = check_launch("conv1_wgrad_kernel")) return rc;
-    const int nw = kCh * cin * 9;
-    wgrad_reduce_kernel<<<(nw + kCh + 127) / 128, 128, 0, as_stream(stream)>>>(partial, G, nw, kCh, dw, db);
-    return check_launch("wgrad_reduce_kernel");
+    return conv1_wgrad_launch(obs, shift, dpre, partial, dw, db, N, cin, pad, stream);
+}
+
+int drq_conv1_wgrad_f32_from_f32(const float* obs, const float* dpre, float* partial, float* dw, float* db, int N,
+                                 int cin, void* stream) {
+    return conv1_wgrad_launch(obs, nullptr, dpre, partial, dw, db, N, cin, 0, stream);
+}
+
+int drq_conv1_dgrad_f32(const float* dpre, const float* w, float* dx, int N, int cin, void* stream) {
+    DRQ_REQUIRE(dpre && w && dx, "conv1_dgrad: null pointer");
+    DRQ_REQUIRE(N >= 0 && cin > 0 && cin <= 16, "conv1_dgrad: bad dims (cin<=16)");
+    if (N == 0) return DRQ_OK;
+    const size_t smem = (size_t)(9 * kCh * 16 + kCh * kDgDRows * kPW) * sizeof(float);
+    if (int rc = set_smem(conv1_dgrad_kernel, smem, "conv1_dgrad")) return rc;
+    conv1_dgrad_kernel<<<dim3(kImg / kDgRows, N), 256, smem, as_stream(stream)>>>(dpre, w, dx, cin);
+    return check_launch("conv1_dgrad_kernel");
 }
 
 int drq_conv3x3_fwd_f32(const float* in, const float* w, const float* b, float* out, int N, int hout,

@@ -301,6 +301,31 @@ __global__ void random_shift_f32_kernel(const float* __restrict__ in, const int*
     }
 }
 
+// its transpose: dx[n,c,i,j] = sum of dout[n,c,r,col] over every (r, col) whose clamped source is (i, j), in ascending
+// (r, col) order.  Separable: the rows are r = i - dy (dy = sy - pad) in the interior, r <= -dy at i = 0 and
+// r >= H-1-dy at i = H-1, each range cut to [0, H); the columns likewise.  An empty range gives +0.
+// Grid: (pixel blocks of a plane, N * C planes); consecutive threads take consecutive columns, whose sources are
+// consecutive too away from the clamped edges.
+__global__ void random_shift_bwd_f32_kernel(const float* __restrict__ dout, const int* __restrict__ shift,
+                                            float* __restrict__ dx, int planes, int C, int H, int W, int pad) {
+  for (int plane = blockIdx.y; plane < planes; plane += gridDim.y) {
+    const int n = plane / C;
+    const int dxs = __ldg(shift + 2 * n) - pad, dys = __ldg(shift + 2 * n + 1) - pad;
+    const int hw = H * W;
+    const float* src = dout + (long long)plane * hw;
+    float* dst = dx + (long long)plane * hw;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < hw; i += gridDim.x * blockDim.x) {
+        const int r = i / W, col = i - r * W;
+        const int rlo = max(r == 0 ? 0 : r - dys, 0), rhi = min(r == H - 1 ? H - 1 : r - dys, H - 1);
+        const int clo = max(col == 0 ? 0 : col - dxs, 0), chi = min(col == W - 1 ? W - 1 : col - dxs, W - 1);
+        float acc = 0.f;
+        for (int rr = rlo; rr <= rhi; ++rr)
+            for (int cc = clo; cc <= chi; ++cc) acc += __ldg(src + rr * W + cc);
+        dst[i] = acc;
+    }
+  }
+}
+
 __global__ void copy2d_kernel(const float* __restrict__ src, long long ld_src, float* __restrict__ dst,
                               long long ld_dst, int rows, int cols) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -460,6 +485,20 @@ int drq_random_shift_f32(const float* in, const int32_t* shift, float* out, int 
     if (gx > 64) gx = 64;
     random_shift_f32_kernel<<<dim3(gx, N), 256, 0, as_stream(stream)>>>(in, shift, out, C, H, W, pad);
     return check_launch("random_shift_f32_kernel");
+}
+
+int drq_random_shift_bwd_f32(const float* dout, const int32_t* shift, float* dx, int N, int C, int H, int W, int pad,
+                             void* stream) {
+    DRQ_REQUIRE(dout && shift && dx, "random_shift_bwd: null pointer");
+    DRQ_REQUIRE(N >= 0 && C > 0 && H > 0 && W > 0 && pad >= 0, "random_shift_bwd: bad dims");
+    DRQ_REQUIRE(H == W, "random_shift_bwd: h != w (drqv2.py:21)");
+    DRQ_REQUIRE((long long)H * W < (1ll << 31) && (long long)N * C < (1ll << 31), "random_shift_bwd: too large");
+    if (N == 0) return DRQ_OK;
+    int gx = (H * W + 255) / 256;
+    if (gx > 1024) gx = 1024;
+    const int planes = N * C, gy = planes < 65535 ? planes : 65535;
+    random_shift_bwd_f32_kernel<<<dim3(gx, gy), 256, 0, as_stream(stream)>>>(dout, shift, dx, planes, C, H, W, pad);
+    return check_launch("random_shift_bwd_f32_kernel");
 }
 
 }  // extern "C"

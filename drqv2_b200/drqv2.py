@@ -168,31 +168,45 @@ def _mlp_bwd(dy, B, n_in, H, n_out, x, ldx, h1, h2, ws, need):
     return g, dh1
 
 
+def _encoder_fwd_f32_pixels(x, w, b, acts, feat, n, cin):
+    """_encoder_fwd from real-valued (already augmented) fp32 pixels"""
+    s = _stream()
+    call("drq_conv1_fwd_f32_from_f32", x, w[0], b[0], acts[0], n, cin, s)
+    call("drq_conv3x3_fwd_f32", acts[0], w[1], b[1], acts[1], n, 39, 0, s)
+    call("drq_conv3x3_fwd_f32", acts[1], w[2], b[2], acts[2], n, 37, 0, s)
+    call("drq_conv3x3_fwd_f32", acts[2], w[3], b[3], feat, n, 35, 1, s)
+
+
 class _EncoderFn(torch.autograd.Function):
     """features = Encoder(pixels) (drqv2.py:63-67) through drq_conv1_fwd_f32 / drq_conv3x3_fwd_f32; backward
     drq_feature_grad_wide_f32 -> drq_conv3x3_{wgrad,dgrad}_f32 for conv4..2 -> drq_conv1_wgrad_f32 (no shift: the pixels
-    arrive augmented).  Inputs: u8 pixels, then (weight, bias) of conv1..4."""
+    arrive augmented).  Inputs: the pixels - uint8, or fp32 on the 0..255 scale (Encoder(pixels="float"), the
+    *_from_f32 conv1 kernels) - then (weight, bias) of conv1..4.  fp32 pixels that require grad get
+    drq_conv1_dgrad_f32's gradient; every weight gradient runs only when its parameter needs it."""
 
     @staticmethod
-    def forward(ctx, u8, *params):
-        n, cin = u8.shape[0], u8.shape[1]
-        dev = u8.device
+    def forward(ctx, px, *params):
+        n, cin = px.shape[0], px.shape[1]
+        dev = px.device
         # zeroed, not empty: drq_conv3x3_wgrad_f32 reads the whole plane of its input activation, slack included
         acts = [torch.zeros(n * 32 * PLANE, device=dev) for _ in range(3)]
         feat = torch.empty(n, REPR_DIM, device=dev)
-        _encoder_fwd(u8.data_ptr(), 0, [p.data_ptr() for p in params[0::2]], [p.data_ptr() for p in params[1::2]],
-                     [a.data_ptr() for a in acts], feat.data_ptr(), n, cin)
-        ctx.save_for_backward(u8, *acts, feat, *params[2::2])
+        fwd = _encoder_fwd if px.dtype == torch.uint8 else _encoder_fwd_f32_pixels
+        args = (px.data_ptr(), 0) if px.dtype == torch.uint8 else (px.data_ptr(),)
+        fwd(*args, [p.data_ptr() for p in params[0::2]], [p.data_ptr() for p in params[1::2]],
+            [a.data_ptr() for a in acts], feat.data_ptr(), n, cin)
+        ctx.save_for_backward(px, *acts, feat, params[0], *params[2::2])
         return feat
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, dfeat):
-        u8, a1, a2, a3, feat, w2, w3, w4 = ctx.saved_tensors
-        need = ctx.needs_input_grad[1:]
-        if not any(need):
+        px, a1, a2, a3, feat, w1, w2, w3, w4 = ctx.saved_tensors
+        need_all = _bf16.needed(ctx)
+        need_x, need = need_all[0], need_all[1:]
+        if not (need_x or any(need)):
             return (None,) * 9
-        n, cin = u8.shape[0], u8.shape[1]
+        n, cin = px.shape[0], px.shape[1]
         dev, s = feat.device, _stream()
         dfeat = dfeat.float().contiguous()
         acts, ws = (a1, a2, a3), (None, w2, w3, w4)
@@ -203,13 +217,24 @@ class _EncoderFn(torch.autograd.Function):
         grads = [torch.empty(shape, device=dev) for shape in [(32, cin, 3, 3), (32,)] + [(32, 32, 3, 3), (32,)] * 3]
         call("drq_feature_grad_wide_f32", dfeat.data_ptr(), feat.data_ptr(), d[3].data_ptr(), n, s)
         for layer, hout in ((3, 35), (2, 37), (1, 39)):
-            call("drq_conv3x3_wgrad_f32", acts[layer - 1].data_ptr(), d[layer].data_ptr(), wsp.data_ptr(),
-                 grads[2 * layer].data_ptr(), grads[2 * layer + 1].data_ptr(), n, hout, s)
-            call("drq_conv3x3_dgrad_f32", d[layer].data_ptr(), ws[layer].data_ptr(), acts[layer - 1].data_ptr(),
-                 d[layer - 1].data_ptr(), n, hout, s)
-        call("drq_conv1_wgrad_f32", u8.data_ptr(), None, d[0].data_ptr(), wsp.data_ptr(), grads[0].data_ptr(),
-             grads[1].data_ptr(), n, cin, 4, s)
-        return (None,) + tuple(g if nd else None for g, nd in zip(grads, need))
+            if need[2 * layer] or need[2 * layer + 1]:
+                call("drq_conv3x3_wgrad_f32", acts[layer - 1].data_ptr(), d[layer].data_ptr(), wsp.data_ptr(),
+                     grads[2 * layer].data_ptr(), grads[2 * layer + 1].data_ptr(), n, hout, s)
+            if need_x or any(need[:2 * layer]):
+                call("drq_conv3x3_dgrad_f32", d[layer].data_ptr(), ws[layer].data_ptr(), acts[layer - 1].data_ptr(),
+                     d[layer - 1].data_ptr(), n, hout, s)
+        if need[0] or need[1]:
+            if px.dtype == torch.uint8:
+                call("drq_conv1_wgrad_f32", px.data_ptr(), None, d[0].data_ptr(), wsp.data_ptr(), grads[0].data_ptr(),
+                     grads[1].data_ptr(), n, cin, 4, s)
+            else:
+                call("drq_conv1_wgrad_f32_from_f32", px.data_ptr(), d[0].data_ptr(), wsp.data_ptr(),
+                     grads[0].data_ptr(), grads[1].data_ptr(), n, cin, s)
+        dx = None
+        if need_x:
+            dx = torch.empty(px.shape, device=dev)
+            call("drq_conv1_dgrad_f32", d[0].data_ptr(), w1.data_ptr(), dx.data_ptr(), n, cin, s)
+        return (dx,) + tuple(g if nd else None for g, nd in zip(grads, need))
 
 
 class _ActorFn(torch.autograd.Function):
@@ -325,6 +350,12 @@ def _flag(differentiable, what):
     return bool(differentiable)
 
 
+def _pixels_flag(pixels, what):
+    if not isinstance(pixels, str) or pixels not in ("u8", "float"):
+        raise ValueError(f"{what}: pixels must be 'u8' or 'float', got {pixels!r}")
+    return pixels
+
+
 def _check_bf16_dims(A, H, Fd, dev=None):
     """Refuse at construction the head shapes the tensor-core kernels refuse (csrc/heads.cu), which would otherwise
     fail at the first act(), update() or forward.  dev None: the current device, when there is one (the shared-memory
@@ -364,11 +395,38 @@ def _wants_graph(module, *inputs):
 
 
 # ----------------------------------------------------------------------------- modules
+class _ShiftFn(torch.autograd.Function):
+    """RandomShiftsAug's integer shift with its transpose as the backward (drq_random_shift_bwd_f32).  Inputs: the fp32
+    pixels, the int32 shifts [N, 2], pad."""
+
+    @staticmethod
+    def forward(ctx, x, shift, pad):
+        n, c, h, w = x.shape
+        out = torch.empty_like(x)
+        call("drq_random_shift_f32", x.data_ptr(), shift.data_ptr(), out.data_ptr(), n, c, h, w, pad, _stream())
+        ctx.save_for_backward(shift)
+        ctx.pad = pad
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dout):
+        shift, = ctx.saved_tensors
+        dout = dout.float().contiguous()
+        n, c, h, w = dout.shape
+        dx = torch.empty_like(dout)
+        call("drq_random_shift_bwd_f32", dout.data_ptr(), shift.data_ptr(), dx.data_ptr(), n, c, h, w, ctx.pad,
+             _stream())
+        return dx, None, None
+
+
 class RandomShiftsAug(nn.Module):
     """Random translation by up to ±pad pixels after replicate padding, as the exact
     integer shift (the reference's bilinear grid_sample equals it to 3.6e-3 on the 0..255
     scale, SURVEY §8a R3).  The draw is the reference's own ``torch.randint`` call, so
-    the same patch injects shifts into either implementation."""
+    the same patch injects shifts into either implementation.  When autograd records and
+    ``x`` requires grad, the output carries the shift's transpose as its backward (the
+    gradient w.r.t. ``x``, drq_random_shift_bwd_f32)."""
 
     def __init__(self, pad):
         super().__init__()
@@ -381,6 +439,8 @@ class RandomShiftsAug(nn.Module):
         shift = torch.randint(0, 2 * self.pad + 1, size=(n, 1, 1, 2), device=x.device, dtype=x.dtype)
         shift = shift.view(n, 2).to(torch.int32).contiguous()
         x = x.float().contiguous()
+        if torch.is_grad_enabled() and x.requires_grad:
+            return _ShiftFn.apply(x, shift, self.pad)
         out = torch.empty_like(x)
         call("drq_random_shift_f32", x.data_ptr(), shift.data_ptr(), out.data_ptr(), n, c, h, w, self.pad,
              _stream())
@@ -399,16 +459,21 @@ def _as_u8_pixels(obs):
 
 class Encoder(nn.Module):
     differentiable = False      # class default: instances pickled before the flag existed read it too
+    pixels = "u8"               # likewise
     refresh = _refresh_bf16
 
-    def __init__(self, obs_shape, *, differentiable=False):
+    def __init__(self, obs_shape, *, differentiable=False, pixels="u8"):
         """differentiable=True: forward records an autograd node (_EncoderFn) whenever autograd records and a parameter
         requires grad, so that a loss on the features trains the convs; off (the default), outputs are plain tensors.
         differentiable="bf16": the same on the tensor-core kernels (bf16 operands, fp32 accumulation; _bf16.EncoderFn),
-        under no_grad too; up to 10 input channels."""
+        under no_grad too; up to 10 input channels.
+        pixels="u8" (the default): integer-valued pixels in 0..255, which may not require grad.  pixels="float": any
+        real-valued pixels on the 0..255 scale, cast to fp32 - with no integrality and no finiteness check - and, when
+        the module is differentiable, autograd records and they require grad, obs.grad = dL/dpixels on that scale."""
         super().__init__()
         assert len(obs_shape) == 3
         self.differentiable = _flag(differentiable, "Encoder")
+        self.pixels = _pixels_flag(pixels, "Encoder")
         if self.differentiable == "bf16" and int(obs_shape[0]) * 9 + 1 > 96:
             raise ValueError(f"Encoder(differentiable='bf16'): {int(obs_shape[0])} input channels; the tensor-core conv1 "
                              "takes cin * 9 + 1 <= 96, at most 10 channels (differentiable=True takes up to 16)")
@@ -426,9 +491,11 @@ class Encoder(nn.Module):
 
     def forward(self, obs):
         """obs: [N, C, 84, 84] pixels on the 0..255 scale (uint8, or integer-valued float as
-        produced by RandomShiftsAug).  Returns features [N, 39200]."""
+        produced by RandomShiftsAug; any real values with pixels="float").  Returns features [N, 39200]."""
         _need_cuda(obs, "Encoder")
         _need_cuda(self.convnet[0].weight, "Encoder parameters")
+        if self.pixels == "float":
+            return self._forward_float(obs)
         if self.differentiable and torch.is_grad_enabled() and obs.requires_grad:
             raise ValueError("Encoder(differentiable=True): the pixels require grad, but the integer-shift encoder has no "
                              "gradient w.r.t. its input pixels; pass them detached")
@@ -446,6 +513,31 @@ class Encoder(nn.Module):
         feat = torch.empty(n, self.repr_dim, device=u8.device)
         w, b = self.conv_ptrs()
         _encoder_fwd(u8.data_ptr(), 0, w, b, [a.data_ptr() for a in acts], feat.data_ptr(), n, cin)
+        return feat
+
+    def _forward_float(self, obs):
+        x = obs.float().contiguous()
+        cin = self.convnet[0].in_channels
+        if obs.dim() != 4 or tuple(x.shape[1:]) != (cin, 84, 84):
+            raise ValueError(f"Encoder: pixels of shape {tuple(obs.shape)}, expected [N, {cin}, 84, 84]")
+        params = list(self.parameters())
+        if torch.is_grad_enabled() and x.requires_grad:
+            # non-leaf edges: _bf16.needed can tell which the backward reaches, so that torch.autograd.grad(q, obs) runs
+            # no weight-gradient kernel (tests/test_gpu_pixel_grad.py::test_saliency_runs_no_encoder_weight_gradient)
+            params = [p.view_as(p) for p in params]
+        if self.differentiable == "bf16":
+            _bf16.check_batch(x.shape[0], "Encoder")
+            ops = _bf16.operands(self, "encoder")
+            if _wants_graph(self, x):
+                return _bf16.EncoderFn.apply(ops, x, *params)
+            return _bf16.encoder_forward(ops, x, [self.convnet[i].bias.data_ptr() for i in (2, 4, 6)])[0]
+        if _wants_graph(self, x):
+            return _EncoderFn.apply(x, *params)
+        n, cin = x.shape[0], x.shape[1]
+        acts = [torch.empty(n * 32 * PLANE, device=x.device) for _ in range(3)]
+        feat = torch.empty(n, self.repr_dim, device=x.device)
+        w, b = self.conv_ptrs()
+        _encoder_fwd_f32_pixels(x.data_ptr(), w, b, [a.data_ptr() for a in acts], feat.data_ptr(), n, cin)
         return feat
 
 
@@ -746,7 +838,8 @@ METRIC_KEYS = ("batch_reward", "critic_target_q", "critic_q1", "critic_q2", "cri
 class DrQV2Agent:
     def __init__(self, obs_shape, action_shape, device, lr, feature_dim, hidden_dim, critic_target_tau,
                  num_expl_steps, update_every_steps, stddev_schedule, stddev_clip, use_tb,
-                 use_cuda_graph=True, seed=None, mode=None, data_parallel=False, prefetch=False, differentiable=False):
+                 use_cuda_graph=True, seed=None, mode=None, data_parallel=False, prefetch=False, differentiable=False,
+                 pixels="u8"):
         """Reference signature (drqv2.py:125-127) plus three keyword-only extras: use_cuda_graph,
         seed (device RNG key) and mode — "fp32" (parity mode, CUDA-core kernels, <= 1e-4 vs the
         reference on pre-optimiser quantities) or "bf16" (tcgen05 tensor-core kernels, bf16
@@ -761,8 +854,11 @@ class DrQV2Agent:
         differentiable=True: encoder, actor and critic record autograd nodes (Encoder / Actor / Critic above) and their
         parameters require grad, so the reference's own update_critic / update_actor bodies (loss.backward();
         opt.step()) train this agent: gradients land in the arena that encoder_opt / critic_opt / actor_opt.step() read
-        (INTEGRATION.md).  The fused update() is unaffected.  Not with data_parallel (those steps do not all-reduce)."""
+        (INTEGRATION.md).  The fused update() is unaffected.  Not with data_parallel (those steps do not all-reduce).
+        pixels="float": agent.encoder takes real-valued pixels, and gives gradients w.r.t. them (Encoder above); act(),
+        update() and the stage API read uint8 frames as before."""
         differentiable = _flag(differentiable, "DrQV2Agent")
+        pixels = _pixels_flag(pixels, "DrQV2Agent")
         if differentiable and data_parallel:
             raise ValueError(f"DrQV2Agent: differentiable={differentiable!r} with data_parallel=True is not supported - "
                              "the optimisers' step() does not average gradients over ranks")
@@ -826,7 +922,7 @@ class DrQV2Agent:
 
         # models: built on the host in the reference's order (so a seed reproduces its init)
         self.differentiable = differentiable
-        self.encoder = Encoder(self.obs_shape, differentiable=self.differentiable)
+        self.encoder = Encoder(self.obs_shape, differentiable=self.differentiable, pixels=pixels)
         self.actor = Actor(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim, differentiable=self.differentiable)
         self.critic = Critic(self.encoder.repr_dim, action_shape, feature_dim, hidden_dim,
                              differentiable=self.differentiable)

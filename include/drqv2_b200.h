@@ -210,6 +210,15 @@ int drq_update_prologue(const float* scal_ring, int slots, uint64_t* cursor, flo
 int drq_random_shift_f32(const float* in, const int32_t* shift, float* out, int N, int C, int H,
                          int W, int pad, void* stream);
 
+/* Its transpose, the backward of the RandomShiftsAug module w.r.t. its input: dx[n,c,i,j] = sum of dout[n,c,r,col]
+ * over every (r, col) with clamp(r+sy-pad,0,H-1) = i and clamp(col+sx-pad,0,W-1) = j, summed in fp32 in ascending
+ * (r, col) order (deterministic, no atomics).  A pixel takes none, one or several: the first / last rows and columns
+ * take the whole clamped run, and on the side the image moves away from there are pixels that take none - those are
+ * written as +0.  Reads dout [N][C][H][W] and shift [N][2] (x, y), and nothing else; writes every element of dx
+ * [N][C][H][W] exactly once and nothing else. */
+int drq_random_shift_bwd_f32(const float* dout, const int32_t* shift, float* dx, int N, int C, int H, int W, int pad,
+                             void* stream);
+
 /* ------------------------------------------------------------------ encoder, fp32 */
 
 /* conv1 of drqv2.py:55 (Cin->32, k3, stride 2) + ReLU, with RandomShiftsAug
@@ -226,6 +235,23 @@ int drq_conv1_fwd_f32(const uint8_t* obs, const int32_t* shift, const float* w, 
 int drq_conv1_wgrad_f32(const uint8_t* obs, const int32_t* shift, const float* dpre,
                         float* partial, float* dw, float* db, int N, int cin, int pad,
                         void* stream);
+
+/* The same two from real-valued pixels: obs fp32 [N][cin][84][84] on the 0..255 scale, already augmented (no shift),
+ * any value (no range, integrality or finiteness check).  The loader computes x/255 - 0.5 exactly as the u8 loader
+ * does, so integer-valued pixels give the bits of drq_conv1_{fwd,wgrad}_f32 with shift = NULL.  Same outputs, same
+ * write sets; the wgrad reads dpre on [0, 1681) of each plane only. */
+int drq_conv1_fwd_f32_from_f32(const float* obs, const float* w, const float* b, float* out, int N, int cin,
+                               void* stream);
+int drq_conv1_wgrad_f32_from_f32(const float* obs, const float* dpre, float* partial, float* dw, float* db, int N,
+                                 int cin, void* stream);
+
+/* conv1's data gradient w.r.t. the pixels (the backward of drqv2.py:64-65 through conv1, 1/255 included):
+ * dx[n][c][iy][ix] = (sum over taps (ky, kx) with iy = 2oy+ky, ix = 2ox+kx, oy, ox < 41, and over co, of
+ * w[co][c][ky][kx] * dpre[n][co][oy*41 + ox]) / 255 - at most 2 x 2 taps x 32 channels per pixel; row and column 83
+ * take no tap.  dpre: wide, gradient w.r.t. conv1's pre-ReLU output, read on [0, 1681) of each plane only; w fp32
+ * [32][cin][3][3].  Writes every element of dx fp32 [N][cin][84][84] exactly once (+0 at row 83) and nothing else.
+ * CUDA cores, fixed summation order (taps ascending, co ascending within a tap), then one division by 255. */
+int drq_conv1_dgrad_f32(const float* dpre, const float* w, float* dx, int N, int cin, void* stream);
 
 /* conv2..4 of drqv2.py:56-59 (32->32, k3, stride 1) + ReLU.
  * in: wide plane; hout = valid output rows = cols (39, 37 or 35).
@@ -331,6 +357,33 @@ int drq_conv1_wgrad_bf16_ring(const drq_ring_src* src, int B, const int32_t* shi
                               float* partial, float* dw, float* db, int N, int pad, void* stream);
 
 int64_t drq_conv1_wgrad_bf16_ws_floats(void);
+
+/* The same two from real-valued pixels: obs fp32 [N][cin][84][84] on the 0..255 scale, already augmented (no shift),
+ * any value (no range, integrality or finiteness check), through the im2col kernel at every batch size.  The im2col
+ * entries are RN-bf16(RN-fp32(x - 128)) - the pixel's rounding point: exact for integers in 0..255 (so integer-valued
+ * pixels give the bits of the im2col selection of drq_conv1_{fwd,wgrad}_bf16, drq_set_conv1_planes(0), with shift =
+ * NULL), 8 significant bits otherwise - and the epilogues are those of the u8 kernels.  Same outputs and write sets.
+ * The wgrad's partial holds drq_conv1_wgrad_bf16_ws_floats() floats; dw and db are required. */
+int drq_conv1_fwd_bf16_from_f32(const float* obs, const uint16_t* w_packed, uint16_t* out, int N, int cin,
+                                void* stream);
+int drq_conv1_wgrad_bf16_from_f32(const float* obs, const uint16_t* dpre, float* partial, float* dw, float* db, int N,
+                                  int cin, void* stream);
+
+/* conv1's data gradient w.r.t. the pixels on tcgen05 tensor cores: per tile of three output rows, col[p][9c + tap] =
+ * sum_co dpre[p][co] * W[co][9c + tap] (M = 128 positions, N = 96, K = 32; bf16 operands, fp32 accumulation in TMEM),
+ * then col2im in the epilogue: dx[n][c][iy][ix] = (sum of the <= 4 col entries of the pixel) / 255, fp32, summed from
+ * +0 with taps (ky, kx) ascending - except input rows 6t (t = 1..13), which two tiles share: their sum starts with the
+ * ky = 2 taps of tile t-1 (kx ascending), carried in shared memory, and adds the ky = 0 taps of tile t (kx
+ * ascending).  Row 83 and column 83 take no tap (+0).  A CTA walks whole images, tiles in order (deterministic, no
+ * atomics, no global scratch).
+ *   dpre: WB bf16 buffer of N images, conv1's pre-ReLU gradient.  Read: pixel rows n*DRQ_PLB + DRQ_GUARD + [0, 1727)
+ *     of every channel block (positions 1681.. reach only accumulator rows that are never stored: they may hold
+ *     anything, NaN included; the last image's reads end inside the buffer's slack).
+ *   w_packed: the packed conv1 operand of drq_pack_conv1_w_bf16; its bf16 weights [12][32][8] are read (entries of
+ *     k >= cin*9 reach only unused columns: anything), the fused biases behind them are not.
+ *   dx: fp32 [N][cin][84][84]; every element written exactly once, nothing else.
+ * Grid min(N, 2 x the SM budget) CTAs of 128 threads. */
+int drq_conv1_dgrad_bf16(const uint16_t* dpre, const uint16_t* w_packed, float* dx, int N, int cin, void* stream);
 
 /* ------------------------------------------------------------------ dense, bf16 tensor cores */
 
