@@ -789,10 +789,20 @@ def _param_key(module):
 def _own_operands(module, kind):
     """Copies owned by a standalone module (drq_pack_multi of its parameters: the pack kinds the agent's copies use),
     re-derived on first use, when a parameter was replaced or changed in place (its version counter moved), or after
-    refresh() / utils.soft_update_params marked them stale."""
+    refresh() / utils.soft_update_params marked them stale.
+    Once a forward of the module has been captured in a CUDA graph, every forward re-derives them, captured or eager:
+    a replay of an optimiser step captured with it (torch.optim.Adam(capturable=True)) changes the parameters without
+    moving a version counter, so neither the version counters read at capture time nor those read between replays
+    tell whether the copies are current.  Two cases they would get wrong: an eager forward between the warm-up and the
+    capture matches the counters, and the captured forwards would then read copies frozen at that eager forward on
+    every replay; and inside the graph the actor's and the encoder's last forward runs before their optimiser step
+    (the target's before the soft update), so an eager forward after a replay would read copies one step behind."""
     key = _param_key(module)
     ops = module.__dict__.get("_bf16_ops")
-    if ops is not None and ops.key == key and not module.__dict__.get("_bf16_stale", False):
+    if torch.cuda.is_current_stream_capturing():
+        module.__dict__["_bf16_captured"] = True
+    elif (ops is not None and ops.key == key and not module.__dict__.get("_bf16_stale", False)
+          and not module.__dict__.get("_bf16_captured", False)):
         return ops
     dev = next(module.parameters()).device
     zb = lambda n: torch.zeros(n, dtype=torch.bfloat16, device=dev)

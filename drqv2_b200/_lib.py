@@ -18,6 +18,7 @@ I = C.c_int
 L = C.c_int64
 U = C.c_uint64
 F = C.c_float
+D = C.c_double
 
 # name -> argument ctypes, in header order.  All return int status unless noted.
 SIGNATURES = {
@@ -88,6 +89,7 @@ SIGNATURES = {
     "drq_actor_loss": [P, P, P, P, P, I, P],
     "drq_copy2d_f32": [P, L, P, L, I, I, P],
     "drq_adam_step": [P, P, P, P, L, P, P],
+    "drq_adam_scalars_advance": [P, D, D, D, D, P, P],
     "drq_soft_update": [P, P, L, F, F, P],
     "drq_adam_ema_step": [P, P, P, P, L, P, P, P, L, F, F, P],
     "drq_adam_pack_step": [P, P, P, P, P, P, P, F, F, P, I, P],

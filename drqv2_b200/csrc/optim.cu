@@ -344,6 +344,25 @@ __global__ void __launch_bounds__(256, 4) adam_pack_kernel(const OptArgs a) {
     }
 }
 
+// One thread: the Adam scalars of the next step from a device step count, so that a captured optimiser step advances
+// its own count on every replay.  fp64 term by term as utils.adam_scalars (1 - beta1 ** t, bc2 ** 0.5, -(lr / bc1)),
+// each value rounded once to fp32.
+__global__ void __launch_bounds__(32) adam_scalars_advance_kernel(long long* step, double lr, double beta1, double beta2,
+                                                                  double eps, float* out) {
+    const long long t = *step + 1;
+    *step = t;
+    const double bc1 = 1.0 - pow(beta1, (double)t);
+    const double bc2 = 1.0 - pow(beta2, (double)t);
+    out[0] = (float)(1.0 - beta1);
+    out[1] = (float)beta2;
+    out[2] = (float)(1.0 - beta2);
+    out[3] = (float)pow(bc2, 0.5);
+    out[4] = (float)eps;
+    out[5] = (float)(-(lr / bc1));
+    out[6] = 0.f;
+    out[7] = 0.f;
+}
+
 static inline bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 
 static int blocks_for(long long n) {
@@ -435,6 +454,13 @@ int drq_adam_pack_step(float* p, const float* g, float* m, float* v, const float
 int drq_adam_step(float* p, const float* g, float* m, float* v, int64_t n, const float* scalars,
                   void* stream) {
     return drq_adam_ema_step(p, g, m, v, n, scalars, nullptr, nullptr, 0, 0.f, 0.f, stream);
+}
+
+int drq_adam_scalars_advance(int64_t* step, double lr, double beta1, double beta2, double eps, float* scalars,
+                             void* stream) {
+    DRQ_REQUIRE(step && scalars, "adam_scalars_advance: null pointer");
+    adam_scalars_advance_kernel<<<1, 1, 0, as_stream(stream)>>>((long long*)step, lr, beta1, beta2, eps, scalars);
+    return check_launch("adam_scalars_advance_kernel");
 }
 
 int drq_soft_update(const float* p, float* tp, int64_t n, float tau, float one_minus_tau, void* stream) {

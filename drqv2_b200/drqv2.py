@@ -30,6 +30,8 @@ F32 = 4
 # of critic_opt at [0, 8), stddev(step) at [8], encoder_opt at [16, 24), actor_opt at [24, 32).
 SCAL_SLOT = 32
 SCAL_OFF = dict(critic=0, stddev=8, encoder=16, actor=24)
+# slots of a capturable agent's device step counts (DrQV2Agent(capturable=True), one int64 per optimiser)
+_STEP_IDX = dict(encoder=0, critic=1, actor=2)
 
 
 def _stream():
@@ -499,6 +501,11 @@ class Encoder(nn.Module):
         if self.differentiable and torch.is_grad_enabled() and obs.requires_grad:
             raise ValueError("Encoder(differentiable=True): the pixels require grad, but the integer-shift encoder has no "
                              "gradient w.r.t. its input pixels; pass them detached")
+        if obs.dtype != torch.uint8 and torch.cuda.is_current_stream_capturing():
+            raise ValueError("Encoder(pixels='u8'): non-uint8 pixels under CUDA graph capture - their integrality check "
+                             "synchronises with the host and cannot run in a graph.  Build the Encoder (or the agent) "
+                             "with pixels='float', which captures and gives the u8 path's bits on integer-valued pixels, "
+                             "or pass uint8 pixels")
         u8 = _as_u8_pixels(obs)
         if self.differentiable == "bf16":
             _bf16.check_batch(u8.shape[0], "Encoder")
@@ -794,7 +801,7 @@ class _Opt:
 
     def state_dict(self):
         a = self._agent._arena
-        return dict(step=self._agent._opt_steps[self.net], exp_avg=self._flat(a.exp_avg), exp_avg_sq=self._flat(a.exp_avg_sq),
+        return dict(step=self._agent._step_counts()[self.net], exp_avg=self._flat(a.exp_avg), exp_avg_sq=self._flat(a.exp_avg_sq),
                     **self.defaults)
 
     def zero_grad(self, set_to_none=True):
@@ -808,13 +815,24 @@ class _Opt:
         .grad is None, this steps every parameter of the network: the arena's gradients are never None (zero_grad
         zeroes them).  The reference's update_critic / update_actor give every parameter they step a gradient, so
         they see no difference.  In the tensor-core mode the bf16 operand copies are re-derived before the next
-        act() / update()."""
+        act() / update().
+        On an agent built with capturable=True the step count lives on the device: one drq_adam_scalars_advance launch
+        derives the Adam scalars there, then the step - in the tensor-core mode Adam and the refresh of this network's
+        bf16 copies in one launch - so that a captured step() is correct on every replay.  Any other agent refuses a
+        step() while the current stream captures: a replay would reuse the scalars of the captured step."""
+        ag = self._agent
+        if not ag.capturable and torch.cuda.is_current_stream_capturing():
+            raise ValueError(f"{self.net}_opt.step() under CUDA graph capture: this agent computes its Adam scalars on "
+                             "the host, and every replay would reuse the captured step's; build the agent with "
+                             "capturable=True to capture its optimiser steps")
         loss = None
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
-        ag = self._agent
         with torch.cuda.device(ag._dev):
+            if ag.capturable:
+                self._step_on_device()
+                return loss
             ag._host_scalars(None, (self.net,))
             ag._fetch_scalars()
             ag._scalars_enqueued()
@@ -830,16 +848,31 @@ class _Opt:
             ag._opt_steps[self.net] += 1
         return loss
 
+    def _step_on_device(self):
+        ag = self._agent
+        beta1, beta2 = self.defaults["betas"]
+        call("drq_adam_scalars_advance", ag._steps_dev.data_ptr() + 8 * _STEP_IDX[self.net], float(self.defaults["lr"]),
+             float(beta1), float(beta2), float(self.defaults["eps"]), ag._sc(self.net), _stream())
+        if ag._bf16 is not None:
+            getattr(ag._bf16, f"step_{self.net}")()      # = drq_adam_step + the pack of this network's copies, bit for bit
+            return
+        a = ag._arena
+        off, n = a.seg[self.net][0], a.seg[self.net][2]
+        call("drq_adam_step", a.params.data_ptr() + F32 * off, a.grads.data_ptr() + F32 * off,
+             a.exp_avg.data_ptr() + F32 * off, a.exp_avg_sq.data_ptr() + F32 * off, n, ag._sc(self.net), _stream())
+
 
 METRIC_KEYS = ("batch_reward", "critic_target_q", "critic_q1", "critic_q2", "critic_loss",
                "actor_loss", "actor_logprob", "actor_ent")
 
 
 class DrQV2Agent:
+    capturable = False          # class default: agents pickled before the flag existed read it too
+
     def __init__(self, obs_shape, action_shape, device, lr, feature_dim, hidden_dim, critic_target_tau,
                  num_expl_steps, update_every_steps, stddev_schedule, stddev_clip, use_tb,
                  use_cuda_graph=True, seed=None, mode=None, data_parallel=False, prefetch=False, differentiable=False,
-                 pixels="u8"):
+                 pixels="u8", *, capturable=False):
         """Reference signature (drqv2.py:125-127) plus three keyword-only extras: use_cuda_graph,
         seed (device RNG key) and mode — "fp32" (parity mode, CUDA-core kernels, <= 1e-4 vs the
         reference on pre-optimiser quantities) or "bf16" (tcgen05 tensor-core kernels, bf16
@@ -856,9 +889,21 @@ class DrQV2Agent:
         opt.step()) train this agent: gradients land in the arena that encoder_opt / critic_opt / actor_opt.step() read
         (INTEGRATION.md).  The fused update() is unaffected.  Not with data_parallel (those steps do not all-reduce).
         pixels="float": agent.encoder takes real-valued pixels, and gives gradients w.r.t. them (Encoder above); act(),
-        update() and the stage API read uint8 frames as before."""
+        update() and the stage API read uint8 frames as before.
+        capturable=True (with differentiable): the reference's update body, optimiser steps included, may be captured
+        in a CUDA graph and replayed.  The three optimisers' step counts live on the device and every step() derives
+        its Adam scalars there (drq_adam_scalars_advance); update(), update_async() and the stage API, which take
+        theirs from host counts, are refused (INTEGRATION.md, "Capturing the update body")."""
         differentiable = _flag(differentiable, "DrQV2Agent")
         pixels = _pixels_flag(pixels, "DrQV2Agent")
+        if capturable not in (False, True):
+            raise ValueError(f"DrQV2Agent: capturable must be False or True, got {capturable!r}")
+        if capturable and not differentiable:
+            raise ValueError("DrQV2Agent: capturable=True captures the optimisers' step() of the reference's update "
+                             "body and needs differentiable=True or 'bf16'; the fused update() captures itself")
+        if capturable and data_parallel:
+            raise ValueError("DrQV2Agent: capturable=True with data_parallel=True is not supported - the optimisers' "
+                             "step() does not average gradients over ranks")
         if differentiable and data_parallel:
             raise ValueError(f"DrQV2Agent: differentiable={differentiable!r} with data_parallel=True is not supported - "
                              "the optimisers' step() does not average gradients over ranks")
@@ -946,6 +991,9 @@ class DrQV2Agent:
         self.critic_opt = _Opt(self, "critic", lr)
         self.aug = RandomShiftsAug(pad=4)
         self._opt_steps = dict(encoder=0, critic=0, actor=0)   # torch.optim.Adam keeps one step count per optimiser
+        self.capturable = bool(capturable)
+        # capturable: the step counts on the device instead, [encoder, critic, actor] (_STEP_IDX), advanced by step()
+        self._steps_dev = torch.zeros(3, dtype=torch.int64, device=dev) if self.capturable else None
         self._seed = int(seed) if seed is not None else int(torch.initial_seed() & 0x7FFFFFFFFFFFFFFF)
         self.data_parallel = bool(data_parallel) and _dist.world() > 1
         # SMs a data-parallel update leaves to NCCL (bf16 mode overlaps its all-reduces with the encoder backward).  Off:
@@ -1048,7 +1096,10 @@ class DrQV2Agent:
                     else:
                         a.exp_avg[off:off + n].zero_()
                         a.exp_avg_sq[off:off + n].zero_()
-                self._opt_steps[net] = step
+                if self.capturable:
+                    self._steps_dev[_STEP_IDX[net]] = step
+                else:
+                    self._opt_steps[net] = step
         self._bf16_dirty = True
         return self
 
@@ -1060,12 +1111,14 @@ class DrQV2Agent:
         out = {net: {k: v.detach().clone() for k, v in getattr(self, net).state_dict().items()}
                for net in self._NETS + ("critic_target",)}
         a = self._arena
+        counts = self._step_counts()
         for net in self._NETS:
             state = {}
+            steps = counts[net]
             for i, (pname, p) in enumerate(getattr(self, net).named_parameters()):
                 off, n = a.offsets[net][pname], p.numel()
-                if self._opt_steps[net] > 0:
-                    state[i] = dict(step=torch.tensor(float(self._opt_steps[net])),
+                if steps > 0:
+                    state[i] = dict(step=torch.tensor(float(steps)),
                                     exp_avg=a.exp_avg[off:off + n].view(p.shape).clone(),
                                     exp_avg_sq=a.exp_avg_sq[off:off + n].view(p.shape).clone())
             group = dict(lr=self.lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0, amsgrad=False, maximize=False,
@@ -1073,6 +1126,20 @@ class DrQV2Agent:
                          params=list(range(len(state) if state else len(list(getattr(self, net).parameters())))))
             out[f"{net}_opt"] = dict(state=state, param_groups=[group])
         return out
+
+    def _step_counts(self):
+        """{net: optimiser step count}: on a capturable agent read from the device in one copy (graph replays advance
+        the counts there)"""
+        if self.capturable:
+            return dict(zip(_STEP_IDX, self._steps_dev.tolist()))
+        return dict(self._opt_steps)
+
+    def _refuse_capturable(self, what):
+        if self.capturable:
+            raise ValueError(f"DrQV2Agent.{what}: not on an agent built with capturable=True - it computes its Adam "
+                             "scalars on the host from host step counts, while this agent keeps its counts on the "
+                             "device.  Train it through the reference's update body (INTEGRATION.md, 'Capturing the "
+                             "update body'), or build it with capturable=False")
 
     def train(self, training=True):
         self.training = training
@@ -1210,6 +1277,7 @@ class DrQV2Agent:
     def update(self, replay_iter, step):
         """drqv2.py:230-262.  Returns {} (and does not advance the iterator) when
         step % update_every_steps != 0."""
+        self._refuse_capturable("update()")
         ws = self.update_async(replay_iter, step)
         if ws is None or not self.use_tb:
             return dict()
@@ -1228,6 +1296,7 @@ class DrQV2Agent:
         """update() without the metrics read-back: enqueues the whole update on the current stream and
         returns its workspace (None when step % update_every_steps != 0) - no host synchronisation, so
         several agents can be driven from one thread (ensemble.AgentEnsemble)."""
+        self._refuse_capturable("update_async()")
         if step % self.update_every_steps != 0:
             return None
         ring = None
@@ -1703,6 +1772,7 @@ class DrQV2Agent:
         and leaves the encoder untouched (a reference encoder whose gradients are None is skipped by Adam in the
         same way).  bf16 mode: features are always external (the tensor-core encoder keeps its output in its own
         bf16 layout), so only the critic is updated."""
+        self._refuse_capturable("update_critic()")
         with torch.cuda.device(self._dev):
             B = obs.shape[0]
             ws = self.workspace(B)
@@ -1728,6 +1798,7 @@ class DrQV2Agent:
     def update_actor(self, obs, step):
         """drqv2.py:206-228 on (detached) features: actor loss, backward, actor_opt.step().  The target critic is
         not touched (its soft update belongs to update(), drqv2.py:259-260)."""
+        self._refuse_capturable("update_actor()")
         with torch.cuda.device(self._dev):
             B = obs.shape[0]
             ws = self.workspace(B)
